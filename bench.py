@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR     (+ the last timed step's outputs)
 
 Workload (BASELINE.json): the 10-minute mono 44.1 kHz synthetic harmonic tone + noise of
 configs[1], analysed with the parameters the metric is quoted on (nfft=2048, hop=512,
@@ -48,6 +49,7 @@ CFG4 = dict(sr=44100, seconds=8 * 3600, nfft=2048, hop=256, npks=100, pkthresh=0
             f0=200.0, nharm=100, p=0.4, sigma=0.01, seed=4000)
 CFG3 = dict(sr=16000, seconds=3, nclips=4096, nfft=512, hop=128, npks=20, pkthresh=0.005)
 E2E_TABLES = ("f", "mag", "ph", "totalmag")      # what the end-to-end step downloads (the arrays north_star names)
+DUMP_BYTES = 60 << 20                            # --dump-outputs: data bytes of all files, under 64 MB with headers
 METRIC = "STFT frames/sec (nfft=2048,hop=512,npks=50) + resynth partial-samples/sec"
 WORKLOAD = ("10 min mono 44.1 kHz synthetic harmonic tone+noise (configs[1] length; 220 Hz, 90 harmonics, "
             "sigma 0.01), metric parameters nfft=2048 hop=512 npks=50, analysis + tracking + full resynthesis")
@@ -485,6 +487,13 @@ def gpu_main(args):
     launches = int(_lib.lib().pvk_launch_count()) - launches0     # libpvk kernels launched by the timed steps
     clocks = sampler.stop()
     gc.enable()
+    if args.dump_outputs:
+        own = slice(plan["own0"], plan["own0"] + plan["nown"]) if world > 1 else slice(None)
+        outs = {k: state["a"][k][0][own] for k in ("f", "mag", "ph", "realph", "binno", "totalmag")}
+        outs["track_ids"] = state["table"][plan["j0"]:plan["j1"]] if world > 1 else state["table"]
+        outs["partial_start"], outs["partial_length"] = state["spans"]
+        outs["synth"] = state["w"]
+        dump_outputs(args.dump_outputs, outs, DUMP_BYTES // world, "_rank%d" % rank if world > 1 else "")
     st = np.array([[e[i].elapsed_time(e[i + 1]) for i in range(4)] for e in timed])   # ms per stage
     ms_step_local = float(st.sum(axis=1).mean())
     sys.stderr.write("rank %d per-step stage ms [analysis, tracking, pack, resynth]:\n%s\n" % (rank, np.round(st, 3)))
@@ -528,7 +537,7 @@ def gpu_main(args):
             return time.perf_counter() - t0, nb
         for _ in range(4):
             e2e_step()
-        for _ in range(max(2, min(args.steps, 5))):
+        for _ in range(args.steps):
             flush.fill_(1)
             barrier()
             dt, nb = e2e_step()
@@ -609,6 +618,23 @@ def gpu_main(args):
     os.write(real_stdout, (json.dumps(line) + "\n").encode())
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(outdir, arrays, budget, suffix=""):
+    """Write device arrays as float64 `outdir/<name><suffix>.npy`.  An array larger than its equal share
+    of `budget` bytes keeps a fixed, seeded sample of its rows (sorted; the same rows for arrays of the
+    same length), so two builds run with the same arguments can be compared output for output."""
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    cap = budget // len(arrays)
+    for name, t in arrays.items():
+        t = t.to(torch.float64)
+        n = t.shape[0]
+        rows = max(1, cap // max(1, t[:1].numel() * 8))
+        if n > rows:
+            idx = np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+            t = t.index_select(0, torch.from_numpy(idx).to(t.device))
+        np.save(os.path.join(outdir, name + suffix + ".npy"), t.cpu().numpy())
 
 
 def _traffic(which):
@@ -745,7 +771,14 @@ def main():
     ap.add_argument("--workload", default="metric", choices=["metric", "cfg3", "cfg4"])
     ap.add_argument("--cfg4-hours", type=float, default=8.0)
     ap.add_argument("--cfg3-clips", type=int, default=4096)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's outputs (analysis tables, track ids, partial "
+                         "spans, resynthesis) as float64 DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload == "cfg3"):
+        ap.error("--dump-outputs covers the GPU path of the metric and cfg4 workloads")
     if args.impl == "reference":
         reference_main(args)
     else:

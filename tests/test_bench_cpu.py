@@ -35,3 +35,34 @@ def test_reference_arm_line():
 
 def test_reference_arm_other_ranks_are_silent():
     assert _run({"RANK": "1", "WORLD_SIZE": "2"}) == ""
+
+
+def test_dump_outputs_sampled_within_budget(tmp_path):
+    """--dump-outputs: float64 files, a fixed seeded row sample of arrays over their share of the budget,
+    identical from call to call."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    tab = torch.arange(5000 * 4, dtype=torch.float64).reshape(5000, 4)
+    arrays = {"tab": tab, "ids": tab.to(torch.int32), "small": torch.arange(10, dtype=torch.float32)}
+    budget = 3 * 8 * 4 * 1000                            # 1000 rows of [*, 4] per array
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, budget)
+    a = {k: np.load(str(tmp_path / "a" / (k + ".npy"))) for k in arrays}
+    assert all(v.dtype == np.float64 for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= budget
+    assert a["tab"].shape == (1000, 4) and np.array_equal(a["tab"], a["ids"])
+    rows = a["tab"][:, 0] / 4
+    assert np.all(np.diff(rows) > 0) and np.array_equal(a["tab"], tab.numpy()[rows.astype(int)])
+    assert np.array_equal(a["small"], np.arange(10))
+    for k in arrays:
+        assert np.array_equal(np.load(str(tmp_path / "b" / (k + ".npy"))), a[k])
+
+
+def test_bench_rejects_zero_steps_and_unsupported_dumps(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)],
+                  ["--workload", "cfg3", "--dump-outputs", str(tmp_path)]):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, stdout=subprocess.PIPE,
+                             stderr=subprocess.PIPE, text=True, timeout=120)
+        assert res.returncode == 2 and res.stdout == "", (extra, res.stderr)
