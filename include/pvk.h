@@ -300,7 +300,7 @@ int pvk_segment_rename_mcast(const int32_t *tid_own, int64_t n, const int32_t *g
 
 /* ------------------------------------------------------------------ resynthesis
  * Replaces SinSum.synth -> RegPartial.synth (PVAnalysis.py:1053-1070,684-756),
- * phase_preserve=True path, for ONE clip.
+ * phase_preserve=True path, for ONE clip (pvk_resynth_ex below: phase_preserve=False).
  *
  *   tid [nframes, npks]                  track id per frame slot (pvk_track)
  *   ntracks, tstart/tlen/toff, pf/pmag/prealph   the packed partials (pvk_track_pack); partials
@@ -342,6 +342,28 @@ int pvk_resynth_dev(const int32_t *tid, int64_t nframes, int npks, int64_t ntrac
                     double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
                     int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
                     int64_t workspace_bytes, int reuse_tracks, void *stream);
+
+/* pvk_resynth_dev with a choice of phase model (pvk_resynth_dev = pvk_resynth_ex(..., 1, 1.0, NULL, 0)).
+ *   phase_preserve  1: the reference's phase-preserving model above (every block re-anchored at the
+ *                   analysed realph); fscale must be 1.
+ *                   0: integrated phase -- theta(s) = realph[0] + 2 pi fscale / sr * sum_{m<s} fsig[m]
+ *                   over the whole body of a partial, heads / tails at the scaled first / last frequency
+ *                   (DESIGN.md 4.3).  A synthesis hop other than the analysis hop stretches time, fscale
+ *                   shifts pitch; partials with fscale * max(f) >= sr / 2 are not rendered.
+ *   fscale       frequency ratio, finite and > 0
+ *   phase_ws     integrated phase only: scratch of one double per packed point (phase_ws_len >=
+ *                toff[ntracks]; an upper bound such as nframes * npks when the count is on the device).
+ *                Written when reuse_tracks = 0 and read by every call, so calls rendering one signal in
+ *                block ranges pass the same buffer.  A length below min(ntracks, nframes * npks) is
+ *                rejected; partials whose points lie beyond phase_ws_len are not rendered.
+ */
+int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                   const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                   const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                   double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                   int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                   int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                   double *phase_ws, int64_t phase_ws_len, void *stream);
 
 #ifdef __cplusplus
 }

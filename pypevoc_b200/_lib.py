@@ -50,6 +50,8 @@ SIGNATURES = {
                          _i64, _p, _i64, _i, _p]),
     "pvk_resynth_dev": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _i, _p, _i64, _i64,
                              _i64, _p, _i64, _i, _p]),
+    "pvk_resynth_ex": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _i, _p, _i64, _i64,
+                            _i64, _p, _i64, _i, _i, _d, _p, _i64, _p]),
 }
 
 

@@ -13,6 +13,10 @@
 // hold the first / last frame of a rendered partial, the others are never touched.
 // Not HBM bound (8 bytes written per output sample, ~0.03-0.1 B per partial-sample): the
 // binding resources are MUFU and instruction issue; see DESIGN.md.
+// Integrated-phase mode (phase_preserve = 0, pvk_resynth_ex): the phase runs on over the whole
+// partial instead of being re-anchored at realph every block, so the start phase of each block is
+// computed first by a segmented scan over the packed points (phase_scan_*); the render kernels are
+// the same, instantiated with FREE = true (DESIGN.md 4.3).
 #include "pvk_common.cuh"
 
 namespace pvk {
@@ -45,6 +49,11 @@ struct RParams {
   double qaf, qam;          // fractional knot offsets times h (qk = ceil(qaf), qkm = ceil(qam))
   double inv_sr, inv_h, hpc;   // 1/sr, 1/h, pi / (2 fstep) (:715)
   int nchp, G;              // chunk threads per item group, number of item groups
+  // integrated-phase mode (phase_preserve = 0) only
+  unsigned long long *phase;   // [phcap] start phase of every packed point's body block, fixed point (PHASE_ONE)
+  int64_t phcap;            // capacity of phase: partials with points at or beyond it are not rendered
+  double fscale;            // frequency ratio
+  int free_phase;           // 1: integrated phase (launch-uniform; the render kernels take it as a template)
 };
 
 // np.interp at knot coordinate kf (sample position / h - knot offset) of values v[0..nfr),
@@ -124,7 +133,25 @@ __device__ __forceinline__ float frac_angle(double th) {
   return fmaf(x, 7.4901405e-7f, -6.2831855f);                    // (x - 2^23) * 2 pi / 2^23
 }
 
-// body of partial v (nfr frames) inside block b (PVAnalysis.py:701-736), in cycles
+// Integrated phase is kept as a 63-bit fixed-point fraction of a cycle: adding two of them modulo
+// PHASE_ONE is exact, hence associative, so the segmented scan of the block increments gives the
+// same bits whatever the grouping of its sums (batch = per clip, chunked = one shot).
+typedef unsigned long long phase_t;
+constexpr phase_t PHASE_MASK = 0x7fffffffffffffffull;        // PHASE_ONE - 1, PHASE_ONE = 2^63
+constexpr phase_t PHASE_HEAD = 0x8000000000000000ull;        // flag bit of the scan's group aggregates
+
+__device__ __forceinline__ phase_t phase_fix(double cyc) {
+  const double fr = cyc - floor(cyc);                           // [0, 1]
+  return (phase_t)(fr * 9.223372036854775808e18) & PHASE_MASK;   // * 2^63
+}
+__device__ __forceinline__ double phase_cycles(phase_t u) {
+  return (double)(u & PHASE_MASK) * 1.0842021724855044e-19;    // * 2^-63
+}
+
+// body of partial v (nfr frames) inside block b, in cycles.  FREE = false: phase-preserving
+// (PVAnalysis.py:701-736); FREE = true: integrated phase, starting at the scanned P of the block,
+// frequency scaled by fscale, no per-block correction (DESIGN.md 4.3)
+template <bool FREE>
 __device__ __forceinline__ void make_body(const RParams &p, int64_t b, int v, int nfr, BodyItem &it) {
   const double h = (double)p.h;
   const int ii = (int)(b - p.tstart[v]);
@@ -133,6 +160,23 @@ __device__ __forceinline__ void make_body(const RParams &p, int64_t b, int v, in
   const int k0 = ii - p.Af;
   const Lin2 Lf = interp_block(tf, nfr, k0, p.qaf, h, p.inv_h);
   const double qk = (double)p.qk;
+  if (FREE) {
+    const double fs = p.fscale * p.inv_sr;
+    const double th0 = phase_cycles(p.phase[o + ii]);
+    const Lin2 Lm = interp_block(tm, nfr, ii - p.Am, p.qam, h, p.inv_h);
+    PhaseSeg &s0 = it.s[0], &s1 = it.s[1];
+    s0.A = th0;
+    s0.B = (Lf.c0 - 0.5 * Lf.s0) * fs;
+    s0.C = 0.5 * Lf.s0 * fs;
+    s1.A = th0 + ((Lf.c0 - Lf.c1) * qk + 0.5 * (Lf.s0 - Lf.s1) * (qk * (qk - 1.0))) * fs;
+    s1.B = (Lf.c1 - 0.5 * Lf.s1) * fs;
+    s1.C = 0.5 * Lf.s1 * fs;
+    s0.tB = (float)(TWO_PI * s0.B); s0.tC2 = (float)(2.0 * TWO_PI * s0.C);
+    s1.tB = (float)(TWO_PI * s1.B); s1.tC2 = (float)(2.0 * TWO_PI * s1.C);
+    it.mc0 = (float)Lm.c0; it.ms0 = (float)Lm.s0;
+    it.mc1 = (float)Lm.c1; it.ms1 = (float)Lm.s1;
+    return;
+  }
   const double fb0 = p.qk > 0 ? Lf.c0 : Lf.c1;                      // fsig[hop*ii]
   const double fb1 = fma(Lf.s1, h, Lf.c1);                          // fsig[hop*(ii+1)]
   const double ph0 = tr[ii] + (fb1 - fb0) * p.hpc;                  // realph[ii] + phcor  :715,721
@@ -178,6 +222,14 @@ __global__ void __launch_bounds__(256) resynth_tracks_kernel(RParams p, int64_t 
     if (nfr < p.minframes || nfr <= 0) continue;
     const int64_t s = p.tstart[v], e = s + nfr - 1;
     if (s < 0 || e >= p.F) continue;
+    if (p.free_phase) {
+      // Nyquist rule (flag set by the scan) or points beyond the phase buffer: not rendered; the flag
+      // (tfade[v].pad0 != 0) takes the partial out of the render kernels' `on` predicate
+      if (tfade[v].pad0 != 0 || p.toff[v] + nfr > p.phcap) {
+        if (lane == 0) tfade[v].pad0 = 1;
+        continue;
+      }
+    }
     for (int c0 = 0; c0 < p.K; c0 += 32) {
       const int c = c0 + lane;
       const bool hs = c < p.K && p.tid[s * p.K + c] == (int)v;
@@ -197,8 +249,16 @@ __global__ void __launch_bounds__(256) resynth_tracks_kernel(RParams p, int64_t 
       const Lin2 Lf = interp_block(tf, nfr, il - p.Af, p.qaf, hd, p.inv_h);
       const double fb0 = p.qk > 0 ? Lf.c0 : Lf.c1;
       const double fb1 = fma(Lf.s1, hd, Lf.c1);
-      t.thl = (tr[il] + (fb1 - fb0) * p.hpc) * INV_2PI + cum_sum(Lf, (double)p.qk, hd - 1.0) * p.inv_sr;   // ph[-1] :750
-      t.fct = tf[il] * p.inv_sr;
+      if (p.free_phase) {
+        // integrated phase: theta(h*nfr - 1) = P of the last block + the scaled in-block sum
+        const double fs = p.fscale * p.inv_sr;
+        t.fch *= p.fscale;
+        t.thl = phase_cycles(p.phase[o + il]) + cum_sum(Lf, (double)p.qk, hd - 1.0) * fs;
+        t.fct = tf[il] * fs;
+      } else {
+        t.thl = (tr[il] + (fb1 - fb0) * p.hpc) * INV_2PI + cum_sum(Lf, (double)p.qk, hd - 1.0) * p.inv_sr;   // ph[-1] :750
+        t.fct = tf[il] * p.inv_sr;
+      }
       t.m0t = (float)lerp_knots(tm, nfr, (double)nfr - p.dfr);      // msig[hop*nfr] :748
       t.pad0 = t.pad1 = 0;
       tfade[v] = t;
@@ -206,9 +266,172 @@ __global__ void __launch_bounds__(256) resynth_tracks_kernel(RParams p, int64_t 
   }
 }
 
+// ------------------------------------------------------------------ integrated phase: block start phases
+// P[i] of packed point i = body block ii of partial v (i = toff[v] + ii): the phase, in cycles mod 1, of
+// the block's first sample, realph[0] / 2 pi + sum_{j < ii} fscale * cum_sum(Lf_j, qk, h) / sr.  A
+// segmented scan over the packed array (a segment per partial) in three passes, so that a partial of
+// millions of frames is spread over the whole GPU: groups of SCAN_GROUP consecutive points (group
+// sums + in-group scan), one CTA over the group sums, fix-up of the points before a group's first
+// partial start.  The sums are exact (phase_t), so P depends on nothing but the partial's own points.
+constexpr int SCAN_GROUP = 1024;                                  // points per group: 32 steps of one warp
+constexpr int SCAN_CARRY_THREADS = 1024;
+constexpr int SCAN_CARRY_SMEM = (SCAN_CARRY_THREADS / 32) * (int)(sizeof(unsigned long long) + sizeof(int));
+
+// number of real packed points: toff[ntracks] (ntracks from the device when given), at most phcap
+__device__ __forceinline__ int64_t scan_npoints(const RParams &p, int64_t &ntracks, const int32_t *ntracks_dev) {
+  if (ntracks_dev != nullptr) { const int64_t m = *ntracks_dev; ntracks = m < ntracks ? m : ntracks; }
+  if (ntracks <= 0) return 0;
+  const int64_t n = p.toff[ntracks];
+  return n < p.phcap ? n : p.phcap;
+}
+
+// partial holding packed point i: the largest v < ntracks with toff[v] <= i
+__device__ __forceinline__ int64_t scan_find(const RParams &p, int64_t ntracks, int64_t i) {
+  int64_t lo = 0, hi = ntracks - 1;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi + 1) >> 1;
+    if (p.toff[mid] <= i) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// fscale * (phase advance over body block j of partial v), cycles mod 1
+__device__ __forceinline__ phase_t block_advance(const RParams &p, int64_t v, int64_t j) {
+  const int64_t o = p.toff[v];
+  const Lin2 Lf = interp_block(p.pf + o, p.tlen[v], (int)j - p.Af, p.qaf, (double)p.h, p.inv_h);
+  return phase_fix(cum_sum(Lf, (double)p.qk, (double)p.h) * (p.fscale * p.inv_sr));
+}
+
+// pass 1: one warp per group, 32 consecutive points per step.  Element of point i: the head value
+// realph[0] / 2 pi (flagged) when i starts its partial, else the advance of block i - 1.  Writes the
+// in-group segmented inclusive scan; the group's last point also carries PHASE_HEAD when the group
+// holds a partial start.  Points of partials above the Nyquist limit flag them in tfade[v].pad0.
+__global__ void __launch_bounds__(256) phase_scan_groups_kernel(RParams p, int64_t ntracks,
+                                                                const int32_t *__restrict__ ntracks_dev,
+                                                                TrackFade *__restrict__ tfade) {
+  const int lane = threadIdx.x & 31;
+  const int64_t npts = scan_npoints(p, ntracks, ntracks_dev);
+  const int64_t ngroups = (npts + SCAN_GROUP - 1) / SCAN_GROUP;
+  const int64_t nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  const double nyq = 0.5 * p.sr;
+  for (int64_t c = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; c < ngroups; c += nw) {
+    const int64_t base = c * SCAN_GROUP;
+    const int64_t last = (base + SCAN_GROUP < npts ? base + SCAN_GROUP : npts) - 1;
+    // advance of the block before the group's first point (lane 31 of "step -1"); every lane then
+    // walks forward from the partial of the group's first point (one search per group)
+    int64_t v = scan_find(p, ntracks, base);
+    phase_t dprev = base > p.toff[v] ? block_advance(p, v, base - 1 - p.toff[v]) : 0;
+    int64_t vflag = -1;                                            // last partial this lane flagged
+    phase_t carry = 0;
+    bool seen = false;                                             // a partial start in the group so far
+    for (int64_t s0 = base; s0 <= last; s0 += 32) {
+      const int64_t i = s0 + lane;
+      const bool valid = i <= last;
+      phase_t d = 0, e = 0;
+      bool head = false;
+      if (valid) {
+        while (p.toff[v + 1] <= i) ++v;
+        const int64_t j = i - p.toff[v];
+        head = j == 0;
+        d = block_advance(p, v, j);
+        if (p.fscale * p.pf[i] >= nyq && v != vflag) {             // one flag per lane and partial: the
+          vflag = v;                                               // points of a skipped partial would
+          if (tfade[v].pad0 == 0) atomicOr(&tfade[v].pad0, 1);     // otherwise all hit one word
+        }
+      }
+      phase_t dup = __shfl_up_sync(FULL, d, 1);
+      if (lane == 0) dup = dprev;
+      dprev = __shfl_sync(FULL, d, 31);
+      if (valid) e = head ? phase_fix(p.prealph[i] * INV_2PI) : dup;
+      if (lane == 0 && !head) e = (e + carry) & PHASE_MASK;
+      bool f = head;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {                           // segmented inclusive scan
+        const phase_t eu = __shfl_up_sync(FULL, e, o);
+        const bool fu = __shfl_up_sync(FULL, (int)f, o) != 0;
+        if (lane >= o) {
+          if (!f) e = (e + eu) & PHASE_MASK;
+          f = f || fu;
+        }
+      }
+      if (valid) p.phase[i] = (i == last && (seen || f)) ? (e | PHASE_HEAD) : e;
+      carry = __shfl_sync(FULL, e, 31);
+      seen = seen || __shfl_sync(FULL, (int)f, 31) != 0;
+    }
+  }
+}
+
+// pass 2: one CTA; thread t owns a contiguous run of groups.  Turns every group's last point into
+// its final P (the carry of all earlier groups added up to the group's first partial start).
+__global__ void __launch_bounds__(SCAN_CARRY_THREADS) phase_scan_carry_kernel(RParams p, int64_t ntracks,
+                                                                              const int32_t *__restrict__ ntracks_dev) {
+  PVK_SMEM(smem);                                                  // warp totals: SCAN_CARRY_SMEM bytes
+  phase_t *s_val = reinterpret_cast<phase_t *>(smem);
+  int *s_flag = reinterpret_cast<int *>(smem + (SCAN_CARRY_THREADS / 32) * sizeof(phase_t));
+  const int t = threadIdx.x, lane = t & 31, w = t >> 5;
+  const int64_t npts = scan_npoints(p, ntracks, ntracks_dev);
+  const int64_t ngroups = (npts + SCAN_GROUP - 1) / SCAN_GROUP;
+  const int64_t per = (ngroups + SCAN_CARRY_THREADS - 1) / SCAN_CARRY_THREADS;
+  const int64_t g0 = t * per, g1 = g0 + per < ngroups ? g0 + per : ngroups;
+  auto last_of = [&](int64_t c) { const int64_t e = (c + 1) * SCAN_GROUP; return (e < npts ? e : npts) - 1; };
+  // this thread's aggregate
+  phase_t a = 0;
+  bool fa = false;
+  for (int64_t c = g0; c < g1; ++c) {
+    const phase_t x = p.phase[last_of(c)];
+    if (x & PHASE_HEAD) { a = x & PHASE_MASK; fa = true; } else a = (a + x) & PHASE_MASK;
+  }
+  // exclusive segmented scan of the thread aggregates: warp, then the warp totals
+  phase_t e = a;
+  bool f = fa;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const phase_t eu = __shfl_up_sync(FULL, e, o);
+    const bool fu = __shfl_up_sync(FULL, (int)f, o) != 0;
+    if (lane >= o) {
+      if (!f) e = (e + eu) & PHASE_MASK;
+      f = f || fu;
+    }
+  }
+  if (lane == 31) { s_val[w] = e; s_flag[w] = f ? 1 : 0; }
+  __syncthreads();
+  phase_t wcarry = 0;                                             // inclusive total of the warps before w
+  for (int k = 0; k < w; ++k) wcarry = s_flag[k] ? s_val[k] : (wcarry + s_val[k]) & PHASE_MASK;
+  phase_t ex = __shfl_up_sync(FULL, e, 1);                        // inclusive total of the lanes before
+  bool fex = __shfl_up_sync(FULL, (int)f, 1) != 0;
+  if (lane == 0) { ex = 0; fex = false; }
+  phase_t run = fex ? ex : (wcarry + ex) & PHASE_MASK;
+  for (int64_t c = g0; c < g1; ++c) {
+    const int64_t l = last_of(c);
+    const phase_t x = p.phase[l];
+    run = (x & PHASE_HEAD) ? (x & PHASE_MASK) : (run + x) & PHASE_MASK;
+    p.phase[l] = run;
+  }
+}
+
+// pass 3: one warp per group c > 0: the points before the group's first partial start (all but the
+// last point, final since pass 2) get the final P of the previous group's last point added.
+__global__ void __launch_bounds__(256) phase_scan_fixup_kernel(RParams p, int64_t ntracks,
+                                                               const int32_t *__restrict__ ntracks_dev) {
+  const int lane = threadIdx.x & 31;
+  const int64_t npts = scan_npoints(p, ntracks, ntracks_dev);
+  const int64_t ngroups = (npts + SCAN_GROUP - 1) / SCAN_GROUP;
+  const int64_t nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t c = 1 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); c < ngroups; c += nw) {
+    const int64_t base = c * SCAN_GROUP;
+    const int64_t last = (base + SCAN_GROUP < npts ? base + SCAN_GROUP : npts) - 1;
+    const int64_t v0 = scan_find(p, ntracks, base);
+    if (p.toff[v0] == base) continue;                              // the group starts a partial
+    const int64_t stop = p.toff[v0 + 1] < last ? p.toff[v0 + 1] : last;
+    const phase_t carry = p.phase[base - 1];
+    for (int64_t i = base + lane; i < stop; i += 32) p.phase[i] = (p.phase[i] + carry) & PHASE_MASK;
+  }
+}
+
 // ------------------------------------------------------------------ kernel 2: per frame row
 // One warp per row of the chunk: the bodies of the rendered partials of the row, as closed-form
 // coefficients, compacted in slot order (deterministic sum order) into gitems.
+template <bool FREE>
 __global__ void __launch_bounds__(128) resynth_prepare_kernel(RParams p, int64_t nrows, BodyItem *__restrict__ gitems,
                                                               int32_t *__restrict__ gcount) {
   const int lane = threadIdx.x & 31;
@@ -224,9 +447,9 @@ __global__ void __launch_bounds__(128) resynth_prepare_kernel(RParams p, int64_t
         v = p.tid[b * p.K + c];
         if (v >= 0 && v < p.ntcap) nfr = p.tlen[v];
       }
-      const bool on = v >= 0 && nfr >= p.minframes;                 // :1061
+      const bool on = v >= 0 && nfr >= p.minframes && (!FREE || p.tfade[v].pad0 == 0);   // :1061; Nyquist rule
       const unsigned mk = __ballot_sync(FULL, on);
-      if (on) make_body(p, b, v, nfr, gitems[row * p.K + n + __popc(mk & lanemask_lt())]);
+      if (on) make_body<FREE>(p, b, v, nfr, gitems[row * p.K + n + __popc(mk & lanemask_lt())]);
       n += __popc(mk);
     }
   }
@@ -441,7 +664,7 @@ constexpr int TILE_BATCH = 32;
 constexpr int TILE_WARP_BYTES = TILE_BATCH * (int)sizeof(BodyItem);   // 2560 >= RS * 33 * 4 for RS <= 16
 constexpr int TILE_WARPS = 4;
 
-template <int RS>
+template <int RS, bool FREE>
 __global__ void __launch_bounds__(TILE_WARPS * 32, 8) resynth_tile_kernel(RParams p, int64_t ntiles, int tpb) {
   PVK_SMEM(smem);
   constexpr int TILE = 32 * RS;
@@ -468,10 +691,10 @@ __global__ void __launch_bounds__(TILE_WARPS * 32, 8) resynth_tile_kernel(RParam
       const int cn = c0 + 32 + lane;
       vnext = cn < K ? trow[cn] : -1;
       const int nfr = (v >= 0 && v < p.ntcap) ? p.tlen[v] : 0;
-      const bool on = v >= 0 && nfr >= p.minframes;               // :1061
+      const bool on = v >= 0 && nfr >= p.minframes && (!FREE || p.tfade[v].pad0 == 0);   // :1061; Nyquist rule
       const unsigned mk = __ballot_sync(FULL, on);
       if (mk == 0u) continue;                                      // warp uniform
-      if (on) make_body(p, b, v, nfr, items[__popc(mk & lanemask_lt())]);
+      if (on) make_body<FREE>(p, b, v, nfr, items[__popc(mk & lanemask_lt())]);
       __syncwarp();
       render_bodies<RS>(p, items, __popc(mk), 0, 1, qs, fast, acc);
       __syncwarp();
@@ -529,8 +752,11 @@ template <int RS>
 static int launch_resynth_tile(const RParams &p, int64_t nblocks, void *stream) {
   const int tpb = p.h / (32 * RS);
   const int64_t ntiles = nblocks * tpb;
-  PVK_LAUNCH(resynth_tile_kernel<RS>, dim3((unsigned)((ntiles + TILE_WARPS - 1) / TILE_WARPS)), dim3(TILE_WARPS * 32),
-             TILE_WARPS * TILE_WARP_BYTES, stream, p, ntiles, tpb);
+  const dim3 grid((unsigned)((ntiles + TILE_WARPS - 1) / TILE_WARPS)), block(TILE_WARPS * 32);
+  if (p.free_phase)
+    PVK_LAUNCH((resynth_tile_kernel<RS, true>), grid, block, TILE_WARPS * TILE_WARP_BYTES, stream, p, ntiles, tpb);
+  else
+    PVK_LAUNCH((resynth_tile_kernel<RS, false>), grid, block, TILE_WARPS * TILE_WARP_BYTES, stream, p, ntiles, tpb);
   PVK_CHECK_LAUNCH("pvk_resynth(render tiles)");
   return PVK_OK;
 }
@@ -550,6 +776,30 @@ extern "C" int pvk_resynth_dev(const int32_t *tid, int64_t nframes, int npks, in
                                double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
                                int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
                                int64_t workspace_bytes, int reuse_tracks, void *stream) {
+  return pvk_resynth_ex(tid, nframes, npks, ntracks, ntracks_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop, nfft,
+                        hop_an, edge, minframes, out, nout, block0, nblocks, workspace, workspace_bytes, reuse_tracks,
+                        1, 1.0, nullptr, 0, stream);
+}
+
+extern "C" int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                              const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                              const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                              double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                              int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                              int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                              double *phase_ws, int64_t phase_ws_len, void *stream) {
+  PVK_REQUIRE(isfinite(fscale) && fscale > 0.0, "pvk_resynth: fscale=%g must be finite and > 0", fscale);
+  PVK_REQUIRE(!phase_preserve || fscale == 1.0,
+              "pvk_resynth: fscale=%g needs phase_preserve=0 (the analysed phases do not fit a scaled frequency)",
+              fscale);
+  if (!phase_preserve) {
+    // every partial has at least one point and there are at most nframes * npks points
+    const int64_t need = ntracks < nframes * (int64_t)npks ? ntracks : nframes * (int64_t)npks;
+    PVK_REQUIRE(phase_ws != nullptr, "pvk_resynth: phase_ws is NULL (phase_preserve=0 needs one double per packed point)");
+    PVK_REQUIRE(phase_ws_len >= need,
+                "pvk_resynth: phase_ws_len=%lld is short (one double per packed point, at least %lld)",
+                (long long)phase_ws_len, (long long)need);
+  }
   PVK_REQUIRE(hop >= 1 && nfft >= 1 && hop_an >= 1, "pvk_resynth: hop=%d nfft=%d hop_an=%d must be >= 1", hop, nfft, hop_an);
   PVK_REQUIRE(npks >= 1 && npks <= PVK_MAX_NPKS, "pvk_resynth: npks=%d must be in [1, %d]", npks, PVK_MAX_NPKS);
   PVK_REQUIRE(sr > 0.0 && edge >= 0.0, "pvk_resynth: sr and edge must be positive");
@@ -588,6 +838,10 @@ extern "C" int pvk_resynth_dev(const int32_t *tid, int64_t nframes, int npks, in
   p.inv_sr = 1.0 / sr; p.inv_h = 1.0 / (double)hop;
   p.hpc = 3.141592653589793 / (2.0 * p.fstep);
   p.mwk = (npks + 31) / 32;
+  p.phase = reinterpret_cast<unsigned long long *>(phase_ws);
+  p.phcap = phase_preserve ? 0 : phase_ws_len;
+  p.fscale = fscale;
+  p.free_phase = phase_preserve ? 0 : 1;
 
   // workspace: masks | fade parameters | staged bodies + counts of one chunk of blocks
   unsigned char *ws = reinterpret_cast<unsigned char *>(workspace);
@@ -603,9 +857,23 @@ extern "C" int pvk_resynth_dev(const int32_t *tid, int64_t nframes, int npks, in
 
   if (nframes > 0 && !reuse_tracks) cudaMemsetAsync(mask, 0, (size_t)(nframes * 2 * p.mwk * 4), (cudaStream_t)stream);
   if (ntracks > 0 && nframes > 0 && !reuse_tracks) {
+    p.chunk0 = 0;
+    if (p.free_phase) {
+      // block start phases + Nyquist flags (tfade[v].pad0), read by the tracks kernel below
+      cudaMemsetAsync(tfade, 0, (size_t)(ntracks * (int64_t)sizeof(TrackFade)), (cudaStream_t)stream);
+      const int64_t pcap = phase_ws_len < nframes * (int64_t)npks ? phase_ws_len : nframes * (int64_t)npks;
+      int64_t sg = ((pcap + SCAN_GROUP - 1) / SCAN_GROUP * 32 + 255) / 256;
+      if (sg > 148 * 16) sg = 148 * 16;
+      if (sg < 1) sg = 1;
+      PVK_LAUNCH(phase_scan_groups_kernel, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev, tfade);
+      PVK_CHECK_LAUNCH("pvk_resynth(phase scan)");
+      PVK_LAUNCH(phase_scan_carry_kernel, dim3(1), dim3(SCAN_CARRY_THREADS), SCAN_CARRY_SMEM, stream, p, ntracks, ntracks_dev);
+      PVK_CHECK_LAUNCH("pvk_resynth(phase carry)");
+      PVK_LAUNCH(phase_scan_fixup_kernel, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev);
+      PVK_CHECK_LAUNCH("pvk_resynth(phase fix-up)");
+    }
     int64_t gsz = (ntracks * 32 + 255) / 256;
     if (gsz > 148 * 16) gsz = 148 * 16;
-    p.chunk0 = 0;
     PVK_LAUNCH(resynth_tracks_kernel, dim3((unsigned)gsz), dim3(256), 0, stream, p, ntracks, ntracks_dev, mask, tfade);
     PVK_CHECK_LAUNCH("pvk_resynth(tracks)");
   }
@@ -629,7 +897,10 @@ extern "C" int pvk_resynth_dev(const int32_t *tid, int64_t nframes, int npks, in
     p.chunk0 = c0;
     p.block0 = c0;
     p.out = out + (c0 - block0) * (int64_t)hop;
-    PVK_LAUNCH(resynth_prepare_kernel, dim3((unsigned)((n + 3) / 4)), dim3(128), 0, stream, p, n, gitems, gcount);
+    if (p.free_phase)
+      PVK_LAUNCH(resynth_prepare_kernel<true>, dim3((unsigned)((n + 3) / 4)), dim3(128), 0, stream, p, n, gitems, gcount);
+    else
+      PVK_LAUNCH(resynth_prepare_kernel<false>, dim3((unsigned)((n + 3) / 4)), dim3(128), 0, stream, p, n, gitems, gcount);
     PVK_CHECK_LAUNCH("pvk_resynth(prepare)");
     const int rc = RS == 16 ? launch_resynth<16>(p, n, bd, stream) : launch_resynth<8>(p, n, bd, stream);
     if (rc != PVK_OK) return rc;

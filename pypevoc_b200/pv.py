@@ -375,8 +375,42 @@ def track_pack_device(fd, magd, phd, realphd, maxpitchjmp=0.5, after_link=None):
     return tr, pk
 
 
+def synth_mode(phase_preserve=True, fscale=1.0):
+    """Checked (phase_preserve, fscale) of a resynthesis call.  ``phase_preserve=False`` integrates the
+    phase from the frequency track (pitch shift by ``fscale``, time stretch by a synthesis hop other
+    than the analysis hop); the phase-preserving model honours the analysed phases and so takes no
+    ``fscale`` other than 1."""
+    if isinstance(fscale, bool) or not isinstance(fscale, (int, float, np.integer, np.floating)):
+        raise TypeError("fscale must be a real number, not %s" % type(fscale).__name__)
+    fscale = float(fscale)
+    if not np.isfinite(fscale) or fscale <= 0.0:
+        raise ValueError("fscale=%r must be finite and > 0" % fscale)
+    phase_preserve = bool(phase_preserve)
+    if phase_preserve and fscale != 1.0:
+        raise ValueError("fscale=%r needs phase_preserve=False: the analysed phases cannot be honoured at a "
+                         "scaled frequency" % fscale)
+    return phase_preserve, fscale
+
+
+def _phase_ws(phase_preserve, npts, dev):
+    """Scratch of the integrated-phase scan: one double per packed point (None when preserving phase)."""
+    if phase_preserve:
+        return None
+    return torch.empty((max(int(npts), 1),), dtype=torch.float64, device=dev)
+
+
+def _resynth_ex(L, tid, F, K, nt, nt_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop, nfft, hop_an, edge, minframes,
+                out, nout, block0, nblocks, ws, reuse_tracks, phase_preserve, fscale, phase_ws):
+    _lib.check(L.pvk_resynth_ex(_ptr(tid), F, K, nt, _ptr(nt_dev), _ptr(tstart), _ptr(tlen), _ptr(toff), _ptr(pf),
+                                _ptr(pmag), _ptr(prealph), float(sr), int(hop), int(nfft), int(hop_an), float(edge),
+                                int(minframes), _ptr(out), int(nout), int(block0), int(nblocks), _ptr(ws), int(ws.numel()),
+                                1 if reuse_tracks else 0, 1 if phase_preserve else 0, float(fscale), _ptr(phase_ws),
+                                0 if phase_ws is None else int(phase_ws.numel()), _stream()), "pvk_resynth")
+
+
 def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edge=1.0, minframes=3,
-                              maxpitchjmp=0.5, after_link=None, after_pack=None, block_range=None, before_sync=None):
+                              maxpitchjmp=0.5, after_link=None, after_pack=None, block_range=None, before_sync=None,
+                              phase_preserve=True, fscale=1.0):
     """The whole back half of the hot path of one clip -- link, id resolution, pack, resynthesis --
     queued back to back with ONE host read-back at the very end: pack and resynthesis are launched
     sized by upper bounds (capacity of the index arrays, (F + 1) * hop + edge output samples) and
@@ -386,7 +420,9 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
     nout): render only these output blocks of a signal of (at most) ``nout`` samples and return them
     uncut (segment-sharded runs: the caller knows its block range without any count and trims once the
     global last frame is known).  ``before_sync`` (optional) is called once everything is queued,
-    before the host waits: work launched there runs behind the rendering instead of after the wait."""
+    before the host waits: work launched there runs behind the rendering instead of after the wait.
+    ``phase_preserve`` / ``fscale``: see synth_mode()."""
+    phase_preserve, fscale = synth_mode(phase_preserve, fscale)
     L = _lib.lib()
     F, K = fd.shape
     if F * K == 0:
@@ -409,11 +445,10 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
     out = torch.empty((nsamp_out,), dtype=torch.float64, device=dev)
     if nsamp_out > 0:
         ws = resynth_workspace(F, K, nt_ub, nb, dev, hop=hop)
+        pws = _phase_ws(phase_preserve, F * K, dev)
         with torch.cuda.device(dev):
-            _lib.check(L.pvk_resynth_dev(_ptr(tr["tid"]), F, K, nt_ub, _ptr(tr["ntracks"]), _ptr(tstart), _ptr(tlen),
-                                         _ptr(toff), _ptr(packed[0]), _ptr(packed[1]), _ptr(packed[3]), float(sr), int(hop),
-                                         int(nfft), int(hop_an), float(edge), int(minframes), _ptr(out), int(nout_ub), b0, nb,
-                                         _ptr(ws), int(ws.numel()), 0, _stream()), "pvk_resynth")
+            _resynth_ex(L, tr["tid"], F, K, nt_ub, tr["ntracks"], tstart, tlen, toff, packed[0], packed[1], packed[3], sr,
+                        hop, nfft, hop_an, edge, minframes, out, nout_ub, b0, nb, ws, False, phase_preserve, fscale, pws)
     if before_sync is not None:
         before_sync(tr)
     nt, npts, last = track_counts(tr)                           # the hot path's one read-back
@@ -423,10 +458,12 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
         return tr, None, (None if block_range is None else out.zero_())
     if nt > nt_ub:                                              # more partials than the speculative cap: redo, sized exactly
         pk = pack_device(fd, magd, phd, realphd, tr["tid"], None, nt, npts=npts)
+        mode = dict(phase_preserve=phase_preserve, fscale=fscale)
         if block_range is None:
-            return tr, pk, resynth_device(tr["tid"], pk, sr, hop, nfft, hop_an, edge=edge, minframes=minframes, max_end=last)
+            return tr, pk, resynth_device(tr["tid"], pk, sr, hop, nfft, hop_an, edge=edge, minframes=minframes, max_end=last,
+                                          **mode)
         return tr, pk, resynth_device(tr["tid"], pk, sr, hop, nfft, hop_an, edge=edge, minframes=minframes, block0=b0,
-                                      nblocks=nb, nout=nout_ub, out=out)
+                                      nblocks=nb, nout=nout_ub, out=out, **mode)
     if block_range is not None:
         return tr, _pack_sliced(raw, nt, npts), out
     nout, _ = synth_geometry(last, hop, nfft, hop_an, edge)
@@ -454,10 +491,14 @@ def synth_geometry(max_end, hop, nfft, hop_an, edge=1.0):
 
 
 def resynth_device(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, max_end=None, block0=0,
-                   nblocks=-1, out=None, ws=None, reuse_tracks=False, nout=None):
-    """pvk_resynth for one clip; returns the float64 device signal (asynchronous).  ``ws``: a
-    workspace tensor to (re)use; ``reuse_tracks``: ``ws`` already holds the per-partial masks and
-    fade parameters of an earlier call with the same tracks and synthesis parameters."""
+                   nblocks=-1, out=None, ws=None, reuse_tracks=False, nout=None, phase_preserve=True, fscale=1.0,
+                   phase_ws=None):
+    """pvk_resynth_ex for one clip; returns the float64 device signal (asynchronous).  ``ws``: a
+    workspace tensor to (re)use; ``reuse_tracks``: ``ws`` (and ``phase_ws``) already hold the per-partial
+    masks, fade parameters (and block start phases) of an earlier call with the same tracks and
+    synthesis parameters.  ``phase_preserve`` / ``fscale``: see synth_mode(); ``phase_ws``: the
+    integrated-phase scratch to (re)use, one float64 per packed point."""
+    phase_preserve, fscale = synth_mode(phase_preserve, fscale)
     L = _lib.lib()
     dev = tid.device
     F, K = tid.shape
@@ -472,12 +513,14 @@ def resynth_device(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, max_en
     nt = int(pk["tstart"].shape[0])
     if ws is None:
         ws = resynth_workspace(F, K, nt, nb, dev)
+    if phase_ws is None and not phase_preserve:
+        if reuse_tracks:
+            raise ValueError("reuse_tracks with phase_preserve=False needs the phase_ws of the first call")
+        phase_ws = _phase_ws(False, pk["pf"].numel(), dev)
     with torch.cuda.device(dev):
-        _lib.check(L.pvk_resynth(_ptr(tid), F, K, nt, _ptr(pk["tstart"]), _ptr(pk["tlen"]),
-                                 _ptr(pk["toff"]), _ptr(pk["pf"]), _ptr(pk["pmag"]), _ptr(pk["prealph"]), float(sr),
-                                 int(hop), int(nfft), int(hop_an), float(edge), int(minframes), _ptr(out), int(nout),
-                                 int(block0), int(nblocks), _ptr(ws), int(ws.numel()), 1 if reuse_tracks else 0,
-                                 _stream()), "pvk_resynth")
+        _resynth_ex(L, tid, F, K, nt, None, pk["tstart"], pk["tlen"], pk["toff"], pk["pf"], pk["pmag"], pk["prealph"], sr,
+                    hop, nfft, hop_an, edge, minframes, out, nout, block0, nblocks, ws, reuse_tracks, phase_preserve,
+                    fscale, None if phase_preserve else phase_ws)
     return out
 
 
@@ -1170,10 +1213,12 @@ class SinSumBatch(object):
     def __len__(self):
         return self._pb.nclips
 
-    def synth_device(self, sr, hop, edge=1.0, minframes=3):
+    def synth_device(self, sr, hop, edge=1.0, minframes=3, phase_preserve=True, fscale=1.0):
         """Render all clips in one pvk_resynth: float64 CUDA tensor [nclips, rows_per_clip * hop]; row c
-        holds clip c's signal from its sample 0 (then the silence of the guard rows)."""
+        holds clip c's signal from its sample 0 (then the silence of the guard rows).  ``phase_preserve``
+        / ``fscale`` as in SinSum.synth (one phase scan over the flattened table, a segment per partial)."""
         pb = self._pb
+        phase_preserve, fscale = synth_mode(phase_preserve, fscale)
         if int(hop) != hop:
             raise TypeError("hop must be an integer number of samples")
         if edge > pb.max_edge:
@@ -1184,7 +1229,8 @@ class SinSumBatch(object):
         nout = pb.nclips * pb.rows_per_clip * hop
         if tr["ntracks"] == 0 or nout == 0:
             return torch.zeros((pb.nclips, pb.rows_per_clip * hop), dtype=torch.float64, device=pb._dev)
-        out = resynth_device(tr["tid"], pk, sr, hop, self.nfft, self.hop, edge=edge, minframes=minframes, nout=nout)
+        out = resynth_device(tr["tid"], pk, sr, hop, self.nfft, self.hop, edge=edge, minframes=minframes, nout=nout,
+                             phase_preserve=phase_preserve, fscale=fscale)
         return out.view(pb.nclips, pb.rows_per_clip * hop)
 
     def clip_lengths(self, hop, edge=1.0):
@@ -1194,10 +1240,10 @@ class SinSumBatch(object):
         n = np.array([synth_geometry(int(e), int(hop), self.nfft, self.hop, edge)[0] for e in last], dtype=np.int64)
         return np.where(last >= 0, n, 0)
 
-    def synth(self, sr, hop, edge=1.0, minframes=3, to_host=True):
+    def synth(self, sr, hop, edge=1.0, minframes=3, to_host=True, phase_preserve=True, fscale=1.0):
         """SinSum.synth of every clip (PVAnalysis.py:1053-1070): list of ``nclips`` float64 signals
         (numpy, or CUDA views with ``to_host=False``), each of its own length."""
-        w = self.synth_device(sr, hop, edge, minframes)
+        w = self.synth_device(sr, hop, edge, minframes, phase_preserve=phase_preserve, fscale=fscale)
         n = self.clip_lengths(hop, edge)
         if to_host:
             wh = w.cpu().numpy()
@@ -1515,22 +1561,26 @@ class SinSum(object):
         return d
 
     # -- resynthesis ---------------------------------------------------------------------
-    def synth(self, sr, hop, edge=1.0, minframes=3, phase_preserve=True, to_host=True, hostbuf=None, chunks=8):
+    def synth(self, sr, hop, edge=1.0, minframes=3, phase_preserve=True, to_host=True, hostbuf=None, chunks=8,
+              fscale=1.0):
         """Overlap-add resynthesis of all partials with >= minframes frames
         (PVAnalysis.py:1053-1070); float64 ``[(max(end)+2)*hop + edgsamp]``.
+        ``phase_preserve=False``: integrated phase instead of the analysed one -- the phase of a partial
+        is the running sum of its (interpolated) frequency times ``fscale``, so ``fscale`` shifts the
+        pitch and a ``hop`` other than the analysis hop stretches time (``synth(sr, round(hop_an * r),
+        phase_preserve=False)``); partials with ``fscale * max(f) >= sr / 2`` are left out.
         ``to_host=False`` returns the CUDA tensor instead of a numpy array.  ``hostbuf`` (a dict,
         reused across calls): render in ``chunks`` block ranges and download each finished range
         into the pinned tensor ``hostbuf['w']`` while the next one is rendered; returns a numpy view
         of it (valid until the next call with the same ``hostbuf``)."""
-        if not phase_preserve:
-            raise NotImplementedError("phase_preserve=False calls RegPartial.synth_no_phase, which is "
-                                      "broken in the reference (PVAnalysis.py:665); not provided")
+        phase_preserve, fscale = synth_mode(phase_preserve, fscale)
+        mode = dict(phase_preserve=phase_preserve, fscale=fscale)
         if int(hop) != hop:
             raise TypeError("hop must be an integer number of samples")
         if self._trk is None and hostbuf is not None:
             self._ensure_tables()
             if self._tables["f"].shape[0] * self._tables["f"].shape[1] > 0:
-                w = self._synth_streamed_fused(sr, int(hop), edge, minframes, hostbuf, int(chunks))
+                w = self._synth_streamed_fused(sr, int(hop), edge, minframes, hostbuf, int(chunks), **mode)
                 if w is not None:
                     return w
         if self._trk is None and hostbuf is None:
@@ -1541,7 +1591,8 @@ class SinSum(object):
             if t["f"].shape[0] * t["f"].shape[1] > 0:
                 tr, pk, out = track_pack_resynth_device(t["f"], t["mag"], t["ph"], t["realph"], sr, int(hop), self.nfft,
                                                         self.hop, edge=edge, minframes=minframes,
-                                                        maxpitchjmp=self._maxpitchjmp, after_link=self._after_link)
+                                                        maxpitchjmp=self._maxpitchjmp, after_link=self._after_link,
+                                                        **mode)
                 self._trk = tr
                 if pk is not None:
                     self._pk = pk
@@ -1553,12 +1604,12 @@ class SinSum(object):
         if tr["ntracks"] == 0:
             raise ValueError("max() arg is an empty sequence")     # what the reference raises (:1059)
         if hostbuf is not None:
-            return self._synth_streamed(pk, tr, sr, int(hop), edge, minframes, hostbuf, int(chunks))
+            return self._synth_streamed(pk, tr, sr, int(hop), edge, minframes, hostbuf, int(chunks), **mode)
         out = resynth_device(tr["tid"], pk, sr, int(hop), self.nfft, self.hop, edge=edge, minframes=minframes,
-                             max_end=tr.get("max_end"))
+                             max_end=tr.get("max_end"), **mode)
         return out.cpu().numpy() if to_host else out
 
-    def _synth_streamed_fused(self, sr, hop, edge, minframes, hostbuf, chunks):
+    def _synth_streamed_fused(self, sr, hop, edge, minframes, hostbuf, chunks, phase_preserve=True, fscale=1.0):
         """synth(hostbuf=...) on fresh partials: link, pack, the chunked rendering and the downloads of
         the finished chunks are all queued before the host reads any count (sizes are upper bounds,
         pvk_track_pack_dev / pvk_resynth_dev); the signal is cut to its real length at the end.  Returns
@@ -1584,15 +1635,14 @@ class SinSum(object):
             chunks = max(1, min(chunks, nblk // 64 if nblk >= 64 else 1))
             bounds = _chunk_bounds(nblk, chunks)
             ws = resynth_workspace(F, K, nt_ub, max(b - a for a, b in zip(bounds, bounds[1:])), dev, hop=hop)
+            pws = _phase_ws(phase_preserve, F * K, dev)        # the phase scan runs with the first chunk
             _mark("pack queued", cur)
             for i in range(chunks):
                 b0, b1 = bounds[i], bounds[i + 1]
                 n0, n1 = b0 * hop, min(b1 * hop, nout_ub)
-                _lib.check(L.pvk_resynth_dev(_ptr(tr["tid"]), F, K, nt_ub, _ptr(tr["ntracks"]), _ptr(tstart), _ptr(tlen),
-                                             _ptr(toff), _ptr(packed[0]), _ptr(packed[1]), _ptr(packed[3]), float(sr),
-                                             int(hop), int(self.nfft), int(self.hop), float(edge), int(minframes),
-                                             _ptr(out[n0:n1]), int(nout_ub), b0, b1 - b0, _ptr(ws), int(ws.numel()),
-                                             1 if i > 0 else 0, _stream()), "pvk_resynth")
+                _resynth_ex(L, tr["tid"], F, K, nt_ub, tr["ntracks"], tstart, tlen, toff, packed[0], packed[1], packed[3],
+                            sr, hop, self.nfft, self.hop, edge, minframes, out[n0:n1], nout_ub, b0, b1 - b0, ws, i > 0,
+                            phase_preserve, fscale, pws)
                 ev = torch.cuda.Event()
                 ev.record(cur)
                 _mark("resynth %d" % i, cur)
@@ -1615,7 +1665,7 @@ class SinSum(object):
         self._last_out = out
         return hw[:nout].numpy()
 
-    def _synth_streamed(self, pk, tr, sr, hop, edge, minframes, hostbuf, chunks):
+    def _synth_streamed(self, pk, tr, sr, hop, edge, minframes, hostbuf, chunks, phase_preserve=True, fscale=1.0):
         dev = self._dev
         F, K = tr["tid"].shape
         max_end = tr.get("max_end")
@@ -1633,12 +1683,14 @@ class SinSum(object):
             bounds = _chunk_bounds(nblk, chunks)
             ws = resynth_workspace(F, K, int(pk["tstart"].shape[0]), max(b - a for a, b in zip(bounds, bounds[1:])), dev,
                                    hop=hop)
+            pws = _phase_ws(phase_preserve, pk["pf"].numel(), dev)  # the phase scan runs with the first chunk
             _mark("pack done", cur)
             for i in range(chunks):
                 b0, b1 = bounds[i], bounds[i + 1]
                 n0, n1 = b0 * hop, min(b1 * hop, nout)
                 resynth_device(tr["tid"], pk, sr, hop, self.nfft, self.hop, edge=edge, minframes=minframes,
-                               max_end=max_end, block0=b0, nblocks=b1 - b0, out=out[n0:n1], ws=ws, reuse_tracks=i > 0)
+                               max_end=max_end, block0=b0, nblocks=b1 - b0, out=out[n0:n1], ws=ws, reuse_tracks=i > 0,
+                               phase_preserve=phase_preserve, fscale=fscale, phase_ws=pws)
                 ev = torch.cuda.Event()
                 ev.record(cur)
                 _mark("resynth %d" % i, cur)
