@@ -365,6 +365,53 @@ int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int64_t ntrack
                    int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
                    double *phase_ws, int64_t phase_ws_len, void *stream);
 
+/* pvk_resynth_ex with phase_preserve = 0, minus the phase scan: the block start phases in phase_ws and
+ * the Nyquist flags in the workspace were written by pvk_resynth_scan (+ pvk_resynth_handover /
+ * pvk_resynth_import_flags).  reuse_tracks = 0 computes the masks and fades from them; later block
+ * ranges of the same signal go through pvk_resynth_ex(reuse_tracks = 1).  phase_preserve must be 0. */
+int pvk_resynth_render(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                       const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                       const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                       double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                       int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                       int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                       double *phase_ws, int64_t phase_ws_len, void *stream);
+
+/* ------------------------------------------------------------------ integrated phase of a sharded signal
+ * One long signal split over ranks (dist.py): each rank scans the partials of its window rows only.
+ * The three calls below carry the true phases and the Nyquist rule across the ranks (DESIGN.md 4.3):
+ *
+ * pvk_resynth_scan -- the phase scan of pvk_resynth_ex (block start phases into phase_ws, local Nyquist
+ *   flags into the workspace), plus, when rec != NULL, this rank's hand-over record for local row h_hi
+ *   (the next rank's hand-over row; < 0: none): int64 rec[2 * npks], rec[k] = the column in local row
+ *   h_lo of the partial in column k of row h_hi (-1: born after h_lo or h_lo < 0, value absolute; -2: no
+ *   partial), rec[npks + k] = P(h_hi) - P(h_lo) or P(h_hi), 63-bit fixed point.  h_lo < 0: the window
+ *   starts at frame 0 (nothing cut).
+ * pvk_resynth_handover -- composes the records of ranks [0, rank) (recs [world][2 * npks], all ranks'
+ *   records as an all_gather leaves them) into the true P at local row h_lo and shifts the partials
+ *   alive there.  No-op for h_lo < 0 or rank 0.
+ * pvk_nyquist_flags -- flags[gid[i]] = 1 where fscale * f[i] >= sr / 2, over n points (this rank's own
+ *   rows and their global ids); the flags of all ranks are then OR-ed (all_reduce MAX).
+ * pvk_resynth_import_flags -- the global flags into the workspace: local partial v takes the flag of the
+ *   global id table[row0 + tstart[v]] holds in its slot (table [table_rows, npks]: the global track
+ *   table, row0: the global row of local row 0).
+ * All four check their arguments before any CUDA call.  Workspace: as pvk_resynth_ex's.
+ */
+int pvk_resynth_scan(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                     const int32_t *tlen, const int64_t *toff, const double *pf, const double *prealph, double sr,
+                     int hop, int nfft, int hop_an, double fscale, void *workspace, int64_t workspace_bytes,
+                     double *phase_ws, int64_t phase_ws_len, int64_t h_lo, int64_t h_hi, int64_t *rec,
+                     int64_t rec_len, void *stream);
+int pvk_resynth_handover(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                         const int32_t *tlen, const int64_t *toff, double *phase_ws, int64_t phase_ws_len,
+                         const int64_t *recs, int64_t recs_len, int world, int rank, int64_t h_lo, void *workspace,
+                         int64_t workspace_bytes, void *stream);
+int pvk_nyquist_flags(const double *f, const int32_t *gid, int64_t n, double sr, double fscale, uint8_t *flags,
+                      int64_t nflags, void *stream);
+int pvk_resynth_import_flags(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                             const int32_t *table, int64_t table_rows, int64_t row0, const uint8_t *flags,
+                             int64_t nflags, void *workspace, int64_t workspace_bytes, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -52,6 +52,13 @@ SIGNATURES = {
                              _i64, _p, _i64, _i, _p]),
     "pvk_resynth_ex": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _i, _p, _i64, _i64,
                             _i64, _p, _i64, _i, _i, _d, _p, _i64, _p]),
+    "pvk_resynth_render": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _i, _p, _i64,
+                                _i64, _i64, _p, _i64, _i, _i, _d, _p, _i64, _p]),
+    "pvk_resynth_scan": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _p, _i64, _p, _i64, _i64,
+                              _i64, _p, _i64, _p]),
+    "pvk_resynth_handover": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _i64, _p, _i64, _i, _i, _i64, _p, _i64, _p]),
+    "pvk_nyquist_flags": (_i, [_p, _p, _i64, _d, _d, _p, _i64, _p]),
+    "pvk_resynth_import_flags": (_i, [_p, _i64, _i, _i64, _p, _p, _i64, _i64, _p, _i64, _p, _i64, _p]),
 }
 
 

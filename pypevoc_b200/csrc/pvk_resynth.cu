@@ -781,13 +781,51 @@ extern "C" int pvk_resynth_dev(const int32_t *tid, int64_t nframes, int npks, in
                         1, 1.0, nullptr, 0, stream);
 }
 
-extern "C" int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
-                              const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
-                              const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
-                              double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
-                              int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
-                              int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
-                              double *phase_ws, int64_t phase_ws_len, void *stream) {
+// sample rate, hops and knots of a launch (everything but the tables and the output)
+static void synth_params(RParams &p, double sr, int hop, int nfft, int hop_an, int npks, double fscale) {
+  p.K = npks; p.sr = sr;
+  p.fstep = sr / (double)nfft;                               // :825
+  const double overlap = (double)hop_an / (double)nfft;      // :824
+  p.dfr = 1.0 / overlap / 2.0;                               // :687
+  p.h = hop;
+  {  // knots of the interpolated frequency (:701) / amplitude (:702) inside a block
+    const double af = p.dfr + 0.5, am = p.dfr;
+    p.Af = (int)floor(af); p.Am = (int)floor(am);
+    p.qaf = (af - floor(af)) * (double)hop; p.qam = (am - floor(am)) * (double)hop;
+    p.qk = (int)ceil(p.qaf); p.qkm = (int)ceil(p.qam);
+  }
+  p.inv_sr = 1.0 / sr; p.inv_h = 1.0 / (double)hop;
+  p.hpc = 3.141592653589793 / (2.0 * p.fstep);
+  p.mwk = (npks + 31) / 32;
+  p.fscale = fscale;
+}
+
+// block start phases + Nyquist flags (tfade[v].pad0) of every partial: the three scan passes
+static int launch_phase_scan(const RParams &p, int64_t ntracks, const int32_t *ntracks_dev, TrackFade *tfade,
+                             void *stream) {
+  cudaMemsetAsync(tfade, 0, (size_t)(ntracks * (int64_t)sizeof(TrackFade)), (cudaStream_t)stream);
+  const int64_t pcap = p.phcap < p.F * (int64_t)p.K ? p.phcap : p.F * (int64_t)p.K;
+  int64_t sg = ((pcap + SCAN_GROUP - 1) / SCAN_GROUP * 32 + 255) / 256;
+  if (sg > 148 * 16) sg = 148 * 16;
+  if (sg < 1) sg = 1;
+  PVK_LAUNCH(phase_scan_groups_kernel, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev, tfade);
+  PVK_CHECK_LAUNCH("pvk_resynth(phase scan)");
+  PVK_LAUNCH(phase_scan_carry_kernel, dim3(1), dim3(SCAN_CARRY_THREADS), SCAN_CARRY_SMEM, stream, p, ntracks, ntracks_dev);
+  PVK_CHECK_LAUNCH("pvk_resynth(phase carry)");
+  PVK_LAUNCH(phase_scan_fixup_kernel, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev);
+  PVK_CHECK_LAUNCH("pvk_resynth(phase fix-up)");
+  return PVK_OK;
+}
+
+// pvk_resynth_ex (scan = true) and pvk_resynth_render (scan = false: the block start phases and the
+// Nyquist flags are already in the workspace / phase_ws)
+static int resynth_run(bool scan, const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                       const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                       const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                       double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                       int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                       int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                       double *phase_ws, int64_t phase_ws_len, void *stream) {
   PVK_REQUIRE(isfinite(fscale) && fscale > 0.0, "pvk_resynth: fscale=%g must be finite and > 0", fscale);
   PVK_REQUIRE(!phase_preserve || fscale == 1.0,
               "pvk_resynth: fscale=%g needs phase_preserve=0 (the analysed phases do not fit a scaled frequency)",
@@ -817,30 +855,17 @@ extern "C" int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int
               "pvk_resynth: workspace too small (%lld bytes; pvk_resynth_workspace_bytes gives the size)",
               (long long)workspace_bytes);
   RParams p;
+  synth_params(p, sr, hop, nfft, hop_an, npks, fscale);
   p.tid = tid; p.tstart = tstart; p.tlen = tlen; p.toff = toff;
   p.pf = pf; p.pmag = pmag; p.prealph = prealph;
-  p.F = nframes; p.K = npks; p.sr = sr; p.ntcap = ntracks;
-  p.fstep = sr / (double)nfft;                               // :825
-  const double overlap = (double)hop_an / (double)nfft;      // :824
-  p.dfr = 1.0 / overlap / 2.0;                               // :687
-  p.h = hop;
+  p.F = nframes; p.ntcap = ntracks;
   p.E = (int)(p.dfr * (double)hop * edge);                   // :740
   p.dE = (p.E + hop - 1) / hop;
   p.einv = p.E > 0 ? (float)(1.0 / (double)p.E) : 0.f;
   p.minframes = minframes;
   p.out = out; p.nout = nout; p.block0 = block0;
-  {  // knots of the interpolated frequency (:701) / amplitude (:702) inside a block
-    const double af = p.dfr + 0.5, am = p.dfr;
-    p.Af = (int)floor(af); p.Am = (int)floor(am);
-    p.qaf = (af - floor(af)) * (double)hop; p.qam = (am - floor(am)) * (double)hop;
-    p.qk = (int)ceil(p.qaf); p.qkm = (int)ceil(p.qam);
-  }
-  p.inv_sr = 1.0 / sr; p.inv_h = 1.0 / (double)hop;
-  p.hpc = 3.141592653589793 / (2.0 * p.fstep);
-  p.mwk = (npks + 31) / 32;
   p.phase = reinterpret_cast<unsigned long long *>(phase_ws);
   p.phcap = phase_preserve ? 0 : phase_ws_len;
-  p.fscale = fscale;
   p.free_phase = phase_preserve ? 0 : 1;
 
   // workspace: masks | fade parameters | staged bodies + counts of one chunk of blocks
@@ -858,19 +883,10 @@ extern "C" int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int
   if (nframes > 0 && !reuse_tracks) cudaMemsetAsync(mask, 0, (size_t)(nframes * 2 * p.mwk * 4), (cudaStream_t)stream);
   if (ntracks > 0 && nframes > 0 && !reuse_tracks) {
     p.chunk0 = 0;
-    if (p.free_phase) {
+    if (p.free_phase && scan) {
       // block start phases + Nyquist flags (tfade[v].pad0), read by the tracks kernel below
-      cudaMemsetAsync(tfade, 0, (size_t)(ntracks * (int64_t)sizeof(TrackFade)), (cudaStream_t)stream);
-      const int64_t pcap = phase_ws_len < nframes * (int64_t)npks ? phase_ws_len : nframes * (int64_t)npks;
-      int64_t sg = ((pcap + SCAN_GROUP - 1) / SCAN_GROUP * 32 + 255) / 256;
-      if (sg > 148 * 16) sg = 148 * 16;
-      if (sg < 1) sg = 1;
-      PVK_LAUNCH(phase_scan_groups_kernel, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev, tfade);
-      PVK_CHECK_LAUNCH("pvk_resynth(phase scan)");
-      PVK_LAUNCH(phase_scan_carry_kernel, dim3(1), dim3(SCAN_CARRY_THREADS), SCAN_CARRY_SMEM, stream, p, ntracks, ntracks_dev);
-      PVK_CHECK_LAUNCH("pvk_resynth(phase carry)");
-      PVK_LAUNCH(phase_scan_fixup_kernel, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev);
-      PVK_CHECK_LAUNCH("pvk_resynth(phase fix-up)");
+      const int rc = launch_phase_scan(p, ntracks, ntracks_dev, tfade, stream);
+      if (rc != PVK_OK) return rc;
     }
     int64_t gsz = (ntracks * 32 + 255) / 256;
     if (gsz > 148 * 16) gsz = 148 * 16;
@@ -905,5 +921,278 @@ extern "C" int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int
     const int rc = RS == 16 ? launch_resynth<16>(p, n, bd, stream) : launch_resynth<8>(p, n, bd, stream);
     if (rc != PVK_OK) return rc;
   }
+  return PVK_OK;
+}
+
+extern "C" int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                              const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                              const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                              double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                              int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                              int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                              double *phase_ws, int64_t phase_ws_len, void *stream) {
+  return resynth_run(true, tid, nframes, npks, ntracks, ntracks_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop,
+                     nfft, hop_an, edge, minframes, out, nout, block0, nblocks, workspace, workspace_bytes,
+                     reuse_tracks, phase_preserve, fscale, phase_ws, phase_ws_len, stream);
+}
+
+extern "C" int pvk_resynth_render(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                                  const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                                  const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                                  double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                                  int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                                  int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                                  double *phase_ws, int64_t phase_ws_len, void *stream) {
+  PVK_REQUIRE(!phase_preserve, "pvk_resynth_render: phase_preserve=1 has no scan to leave out (use pvk_resynth_ex)");
+  return resynth_run(false, tid, nframes, npks, ntracks, ntracks_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop,
+                     nfft, hop_an, edge, minframes, out, nout, block0, nblocks, workspace, workspace_bytes,
+                     reuse_tracks, phase_preserve, fscale, phase_ws, phase_ws_len, stream);
+}
+
+// ------------------------------------------------------------------ integrated phase across segments
+// A rank of a segment-sharded run (dist.py) scans the partials of its window rows [w0, w1) only, so a
+// partial alive at w0 starts there with the wrong phase, and its first Af + 1 advances read frames
+// clamped at the cut.  From the hand-over row h = w0 + max(Af + 2, minframes) = j0 - dE on, the local
+// advances are the true ones: P_local(r) - P_local(h) is exact for every r in [h, j1 + Lf - Af - 1)
+// (fixed point, so the difference of two scanned values is the exact sum of the advances between them).
+// Each rank records, for every column of the NEXT rank's hand-over row, either that difference and the
+// partial's column in its own hand-over row or, for a partial born after its own hand-over row, the
+// absolute P.  Composing the records of the ranks before g column by column gives the true P at row
+// h(g); the partials alive there are shifted by seed - P_local(h(g)).  A rank whose window starts at
+// frame 0 cuts nothing and records absolute values only, which ends every chain.
+namespace pvk {
+
+// record of column k of local row h_hi: rec[k] = column of the same partial in row h_lo (-1: absolute
+// value, -2: no partial), rec[K + k] = P(h_hi) - P(h_lo) or P(h_hi), mod PHASE_ONE
+__global__ void __launch_bounds__(128) handover_record_kernel(RParams p, int64_t ntracks, int64_t h_lo, int64_t h_hi,
+                                                              int64_t *__restrict__ rec) {
+  const int K = p.K;
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < K; k += gridDim.x * blockDim.x) {
+    int64_t col = -2;
+    phase_t val = 0;
+    const int v = h_hi >= 0 ? p.tid[h_hi * K + k] : -1;
+    if (v >= 0 && v < ntracks) {
+      const int64_t s = p.tstart[v], o = p.toff[v];
+      if (o + (h_hi - s) < p.phcap) {
+        val = p.phase[o + (h_hi - s)] & PHASE_MASK;
+        col = -1;
+        if (h_lo >= s) {                                           // alive at h_lo: relative to it
+          for (int c = 0; c < K; ++c)
+            if (p.tid[h_lo * K + c] == v) { col = c; break; }
+          val = (val - p.phase[o + (h_lo - s)]) & PHASE_MASK;
+        }
+      }
+    }
+    rec[k] = col;
+    rec[K + k] = (int64_t)val;
+  }
+}
+
+// seed of column k of row h_lo from the records of ranks [0, rank) (recs [world][2K]), walked back from
+// rank - 1 until an absolute value; delta[k] = seed - P_local(h_lo), dv[k] = the partial (-1: none)
+__global__ void __launch_bounds__(128) handover_seed_kernel(RParams p, int64_t ntracks, const int64_t *__restrict__ recs,
+                                                            int rank, int64_t h_lo, int64_t *__restrict__ delta,
+                                                            int32_t *__restrict__ dv) {
+  const int K = p.K;
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < K; k += gridDim.x * blockDim.x) {
+    const int v = p.tid[h_lo * K + k];
+    int vv = -1;
+    phase_t d = 0;
+    if (v >= 0 && v < ntracks && p.toff[v] + (h_lo - p.tstart[v]) < p.phcap) {
+      phase_t acc = 0;
+      int c = k;
+      for (int g = rank - 1; g >= 0; --g) {
+        const int64_t col = recs[(int64_t)g * 2 * K + c];
+        if (col < -1 || col >= K) break;                           // no partial there: records inconsistent
+        acc = (acc + (phase_t)recs[(int64_t)g * 2 * K + K + c]) & PHASE_MASK;
+        if (col == -1) {
+          vv = v;
+          d = (acc - p.phase[p.toff[v] + (h_lo - p.tstart[v])]) & PHASE_MASK;
+          break;
+        }
+        c = (int)col;
+      }
+    }
+    delta[k] = (int64_t)d;
+    dv[k] = vv;
+  }
+}
+
+// every point from row h_lo on of the partials alive at h_lo gets its column's delta added.  Points
+// before h_lo keep a wrong P: nothing of an own block reads them (bodies start at j0 > h_lo, a tail reads
+// the P of its partial's last row, and partials ending before h_lo = j0 - dE have no tail in an own block).
+__global__ void __launch_bounds__(256) handover_fixup_kernel(RParams p, int64_t h_lo, const int64_t *__restrict__ delta,
+                                                             const int32_t *__restrict__ dv, int nx) {
+  const int k = blockIdx.x / nx, x = blockIdx.x % nx;
+  const int v = dv[k];
+  if (v < 0) return;
+  const phase_t d = (phase_t)delta[k];
+  const int64_t o = p.toff[v];
+  int64_t n = p.tlen[v];
+  if (o + n > p.phcap) n = p.phcap - o;
+  for (int64_t i = (h_lo - p.tstart[v]) + (int64_t)x * blockDim.x + threadIdx.x; i < n; i += (int64_t)nx * blockDim.x)
+    p.phase[o + i] = (p.phase[o + i] + d) & PHASE_MASK;
+}
+
+// global Nyquist flags: flags[gid[i]] = 1 for every point with fscale * f >= sr / 2 (the scan's test)
+__global__ void __launch_bounds__(256) nyquist_scatter_kernel(const double *__restrict__ f, const int32_t *__restrict__ gid,
+                                                              int64_t n, double sr, double fscale, uint8_t *flags,
+                                                              int64_t nflags) {
+  const double nyq = 0.5 * sr;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int g = gid[i];
+    if (g >= 0 && g < nflags && fscale * f[i] >= nyq && flags[g] == 0) flags[g] = 1;
+  }
+}
+
+// one warp per local partial: its global id from the row of its first point, its flag into tfade[v].pad0
+__global__ void __launch_bounds__(256) nyquist_import_kernel(RParams p, int64_t ntracks, const int32_t *__restrict__ table,
+                                                             int64_t row0, const uint8_t *__restrict__ flags,
+                                                             int64_t nflags, TrackFade *__restrict__ tfade) {
+  const int lane = threadIdx.x & 31;
+  const int64_t nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t v = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; v < ntracks; v += nw) {
+    const int64_t s = p.tstart[v];
+    int g = -1;
+    if (s >= 0 && s < p.F) {
+      for (int c0 = 0; c0 < p.K; c0 += 32) {
+        const int c = c0 + lane;
+        const bool hit = c < p.K && p.tid[s * p.K + c] == (int)v;
+        const unsigned m = __ballot_sync(FULL, hit);
+        if (m) { g = table[(row0 + s) * p.K + c0 + __ffs((int)m) - 1]; break; }
+      }
+    }
+    if (lane == 0) tfade[v].pad0 = (g >= 0 && g < nflags && flags[g]) ? 1 : 0;
+  }
+}
+
+}  // namespace pvk
+
+static TrackFade *resynth_tfade(void *workspace, int64_t nframes, int npks) {
+  const int64_t mwk = (npks + 31) / 32;
+  return reinterpret_cast<TrackFade *>(reinterpret_cast<unsigned char *>(workspace) + align_up(nframes * 2 * mwk * 4, 256));
+}
+
+#define PVK_REQUIRE_WS(fn)                                                                                          \
+  PVK_REQUIRE(workspace != nullptr && workspace_bytes >= resynth_fixed_ws(nframes, npks, ntracks) +                 \
+                                                             align_up(resynth_row_ws(npks), 256) + 512,             \
+              fn ": workspace too small (%lld bytes; pvk_resynth_workspace_bytes gives the size)",                 \
+              (long long)workspace_bytes)
+
+extern "C" int pvk_resynth_scan(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                                const int32_t *tlen, const int64_t *toff, const double *pf, const double *prealph,
+                                double sr, int hop, int nfft, int hop_an, double fscale, void *workspace,
+                                int64_t workspace_bytes, double *phase_ws, int64_t phase_ws_len, int64_t h_lo,
+                                int64_t h_hi, int64_t *rec, int64_t rec_len, void *stream) {
+  PVK_REQUIRE(isfinite(fscale) && fscale > 0.0, "pvk_resynth_scan: fscale=%g must be finite and > 0", fscale);
+  PVK_REQUIRE(hop >= 1 && nfft >= 1 && hop_an >= 1, "pvk_resynth_scan: hop=%d nfft=%d hop_an=%d must be >= 1", hop,
+              nfft, hop_an);
+  PVK_REQUIRE(npks >= 1 && npks <= PVK_MAX_NPKS, "pvk_resynth_scan: npks=%d must be in [1, %d]", npks, PVK_MAX_NPKS);
+  PVK_REQUIRE(sr > 0.0, "pvk_resynth_scan: sr must be positive");
+  PVK_REQUIRE(nframes >= 0 && ntracks >= 0, "pvk_resynth_scan: negative sizes");
+  PVK_REQUIRE(nframes == 0 || ntracks == 0 || (tid && tstart && tlen && toff && pf && prealph),
+              "pvk_resynth_scan: NULL pointer argument");
+  PVK_REQUIRE(h_lo < nframes && h_hi < nframes, "pvk_resynth_scan: hand-over rows %lld / %lld outside the %lld rows",
+              (long long)h_lo, (long long)h_hi, (long long)nframes);
+  PVK_REQUIRE(h_hi < 0 || h_lo <= h_hi, "pvk_resynth_scan: h_lo=%lld after h_hi=%lld", (long long)h_lo, (long long)h_hi);
+  PVK_REQUIRE(rec == nullptr || rec_len >= 2 * (int64_t)npks, "pvk_resynth_scan: rec_len=%lld is short (2 * npks = %d)",
+              (long long)rec_len, 2 * npks);
+  const int64_t need = ntracks < nframes * (int64_t)npks ? ntracks : nframes * (int64_t)npks;
+  PVK_REQUIRE(phase_ws != nullptr && phase_ws_len >= need,
+              "pvk_resynth_scan: phase_ws_len=%lld is short (one double per packed point, at least %lld)",
+              (long long)phase_ws_len, (long long)need);
+  PVK_REQUIRE_WS("pvk_resynth_scan");
+  RParams p;
+  synth_params(p, sr, hop, nfft, hop_an, npks, fscale);
+  p.tid = tid; p.tstart = tstart; p.tlen = tlen; p.toff = toff; p.pf = pf; p.prealph = prealph;
+  p.F = nframes; p.ntcap = ntracks;
+  p.phase = reinterpret_cast<unsigned long long *>(phase_ws);
+  p.phcap = phase_ws_len;
+  p.free_phase = 1;
+  if (ntracks > 0 && nframes > 0) {
+    const int rc = launch_phase_scan(p, ntracks, nullptr, resynth_tfade(workspace, nframes, npks), stream);
+    if (rc != PVK_OK) return rc;
+  }
+  if (rec != nullptr) {
+    PVK_LAUNCH(handover_record_kernel, dim3((unsigned)((npks + 127) / 128)), dim3(128), 0, stream, p,
+               nframes > 0 ? ntracks : 0, h_lo, nframes > 0 ? h_hi : -1, rec);
+    PVK_CHECK_LAUNCH("pvk_resynth_scan(record)");
+  }
+  return PVK_OK;
+}
+
+extern "C" int pvk_resynth_handover(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                                    const int32_t *tstart, const int32_t *tlen, const int64_t *toff, double *phase_ws,
+                                    int64_t phase_ws_len, const int64_t *recs, int64_t recs_len, int world, int rank,
+                                    int64_t h_lo, void *workspace, int64_t workspace_bytes, void *stream) {
+  PVK_REQUIRE(npks >= 1 && npks <= PVK_MAX_NPKS, "pvk_resynth_handover: npks=%d must be in [1, %d]", npks,
+              PVK_MAX_NPKS);
+  PVK_REQUIRE(nframes >= 0 && ntracks >= 0, "pvk_resynth_handover: negative sizes");
+  PVK_REQUIRE(world >= 1 && rank >= 0 && rank < world, "pvk_resynth_handover: rank=%d outside world=%d", rank, world);
+  PVK_REQUIRE(h_lo < nframes, "pvk_resynth_handover: h_lo=%lld outside the %lld rows", (long long)h_lo,
+              (long long)nframes);
+  PVK_REQUIRE(recs != nullptr && recs_len >= (int64_t)world * 2 * npks,
+              "pvk_resynth_handover: recs_len=%lld is short (world * 2 * npks = %lld)", (long long)recs_len,
+              (long long)world * 2 * npks);
+  PVK_REQUIRE(nframes == 0 || ntracks == 0 || (tid && tstart && tlen && toff && phase_ws),
+              "pvk_resynth_handover: NULL pointer argument");
+  PVK_REQUIRE(phase_ws_len >= 0, "pvk_resynth_handover: negative phase_ws_len");
+  PVK_REQUIRE_WS("pvk_resynth_handover");
+  if (h_lo < 0 || rank == 0 || nframes == 0 || ntracks == 0) return PVK_OK;     // nothing cut: the scan is exact
+  RParams p;
+  p.tid = tid; p.tstart = tstart; p.tlen = tlen; p.toff = toff;
+  p.F = nframes; p.K = npks; p.ntcap = ntracks;
+  p.phase = reinterpret_cast<unsigned long long *>(phase_ws);
+  p.phcap = phase_ws_len;
+  // delta / dv live in the chunk area of the workspace (the render stage rewrites it)
+  unsigned char *scratch = reinterpret_cast<unsigned char *>(workspace) + resynth_fixed_ws(nframes, npks, ntracks);
+  int64_t *delta = reinterpret_cast<int64_t *>(scratch);
+  int32_t *dv = reinterpret_cast<int32_t *>(scratch + 8 * (int64_t)npks);
+  PVK_LAUNCH(handover_seed_kernel, dim3((unsigned)((npks + 127) / 128)), dim3(128), 0, stream, p, ntracks, recs, rank,
+             h_lo, delta, dv);
+  PVK_CHECK_LAUNCH("pvk_resynth_handover(seed)");
+  const int nx = 32;
+  PVK_LAUNCH(handover_fixup_kernel, dim3((unsigned)(npks * nx)), dim3(256), 0, stream, p, h_lo, delta, dv, nx);
+  PVK_CHECK_LAUNCH("pvk_resynth_handover(fix-up)");
+  return PVK_OK;
+}
+
+extern "C" int pvk_nyquist_flags(const double *f, const int32_t *gid, int64_t n, double sr, double fscale,
+                                 uint8_t *flags, int64_t nflags, void *stream) {
+  PVK_REQUIRE(isfinite(fscale) && fscale > 0.0, "pvk_nyquist_flags: fscale=%g must be finite and > 0", fscale);
+  PVK_REQUIRE(sr > 0.0, "pvk_nyquist_flags: sr must be positive");
+  PVK_REQUIRE(n >= 0 && nflags >= 0, "pvk_nyquist_flags: negative sizes");
+  PVK_REQUIRE(n == 0 || (f && gid), "pvk_nyquist_flags: NULL pointer argument");
+  PVK_REQUIRE(nflags == 0 || flags, "pvk_nyquist_flags: flags is NULL");
+  if (n == 0 || nflags == 0) return PVK_OK;
+  int64_t g = (n + 255) / 256;
+  if (g > 148 * 8) g = 148 * 8;
+  PVK_LAUNCH(nyquist_scatter_kernel, dim3((unsigned)g), dim3(256), 0, stream, f, gid, n, sr, fscale, flags, nflags);
+  PVK_CHECK_LAUNCH("pvk_nyquist_flags");
+  return PVK_OK;
+}
+
+extern "C" int pvk_resynth_import_flags(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                                        const int32_t *tstart, const int32_t *table, int64_t table_rows, int64_t row0,
+                                        const uint8_t *flags, int64_t nflags, void *workspace, int64_t workspace_bytes,
+                                        void *stream) {
+  PVK_REQUIRE(npks >= 1 && npks <= PVK_MAX_NPKS, "pvk_resynth_import_flags: npks=%d must be in [1, %d]", npks,
+              PVK_MAX_NPKS);
+  PVK_REQUIRE(nframes >= 0 && ntracks >= 0 && nflags >= 0 && table_rows >= 0, "pvk_resynth_import_flags: negative sizes");
+  PVK_REQUIRE(row0 >= 0 && row0 + nframes <= table_rows,
+              "pvk_resynth_import_flags: rows [%lld, %lld) outside the table's %lld rows", (long long)row0,
+              (long long)(row0 + nframes), (long long)table_rows);
+  PVK_REQUIRE(nframes == 0 || ntracks == 0 || (tid && tstart && table), "pvk_resynth_import_flags: NULL pointer argument");
+  PVK_REQUIRE(nflags == 0 || flags, "pvk_resynth_import_flags: flags is NULL");
+  PVK_REQUIRE_WS("pvk_resynth_import_flags");
+  if (nframes == 0 || ntracks == 0) return PVK_OK;
+  RParams p;
+  p.tid = tid; p.tstart = tstart;
+  p.F = nframes; p.K = npks;
+  int64_t g = (ntracks * 32 + 255) / 256;
+  if (g > 148 * 16) g = 148 * 16;
+  PVK_LAUNCH(nyquist_import_kernel, dim3((unsigned)g), dim3(256), 0, stream, p, ntracks, table, row0, flags, nflags,
+             resynth_tfade(workspace, nframes, npks));
+  PVK_CHECK_LAUNCH("pvk_resynth_import_flags");
   return PVK_OK;
 }

@@ -549,11 +549,13 @@ def render_range(plan, plans, max_end, hop, nfft, hop_an, edge=1.0):
 
 
 def resynth_local(tid_local, pk_local, plan, plans, max_end, sr, hop, nfft, hop_an, edge=1.0, minframes=3,
-                  out=None, ws=None, block_range=None, reuse_tracks=False, local_last=None):
+                  out=None, ws=None, block_range=None, reuse_tracks=False, local_last=None, **mode):
     """Render this rank's block range (or the sub-range ``block_range`` of it, global block
     indices) from its LOCAL tables: float64 device tensor holding global samples
     [b0*hop, min(b1*hop, nout)).  ``local_last`` (instead of the global ``max_end``): the range
-    of render_range_local(), to be cut with trim_local() once ``max_end`` is known."""
+    of render_range_local(), to be cut with trim_local() once ``max_end`` is known.  ``mode``:
+    phase_preserve / fscale / phase_ws / scanned of resynth_device (integrated phase: after
+    integrated_phase_local)."""
     if local_last is not None:
         b0, b1, nout = render_range_local(plan, plans, local_last, hop, nfft, hop_an, edge)
     else:
@@ -566,7 +568,7 @@ def resynth_local(tid_local, pk_local, plan, plans, max_end, sr, hop, nfft, hop_
     nout_local = nout - w0 * hop                       # same signal, local sample origin w0*hop
     return P.resynth_device(tid_local, pk_local, sr, hop, nfft, hop_an, edge=edge, minframes=minframes,
                             block0=b0 - w0, nblocks=b1 - b0, nout=nout_local, out=out, ws=ws,
-                            reuse_tracks=reuse_tracks)
+                            reuse_tracks=reuse_tracks, **mode)
 
 
 def track_pack_resynth_local(tab, plan, plans, sr, hop, nfft, hop_an, edge=1.0, minframes=3, maxpitchjmp=0.5,
@@ -587,6 +589,114 @@ def track_pack_resynth_local(tab, plan, plans, sr, hop, nfft, hop_an, edge=1.0, 
     if w is None:
         w = torch.zeros((0,), dtype=torch.float64, device=tab["f"].device)
     return tr, pk, w, b0
+
+
+# --------------------------------------------------------------------------- integrated phase
+def handover_rows(plan, plans, nfft, hop, edge=1.0):
+    """(h_lo, h_hi): local rows of this rank's hand-over row h(g) = j0 - dE and of the next rank's,
+    h(g+1) (-1: none).  h(g) = w0 + max(Af + 2, minframes) is where the local advances stop reading
+    frames clamped at the cut w0 (the first Af + 1 advances of a cut partial do), and no P an own block
+    reads lies before it: bodies start at j0, tails read the last row of partials ending at or after
+    j0 - dE.  A window starting at frame 0 cuts nothing: h_lo = -1, the local scan is exact."""
+    if plan["nframes"] == 0:
+        return -1, -1
+    dE = int(np.ceil(nfft / float(hop) / 2. * edge))
+    w0, g = plan["w0"], plan["rank"]
+    lo = plan["j0"] - dE - w0 if w0 > 0 else -1
+    nxt = plans[g + 1] if g + 1 < len(plans) else None
+    hi = nxt["j0"] - dE - w0 if nxt is not None and nxt["nframes"] > 0 and nxt["w0"] > 0 else -1
+    return lo, hi
+
+
+def _pk_args(pk):
+    return pk["tstart"], pk["tlen"], pk["toff"], int(pk["tstart"].shape[0])
+
+
+def handover_scan_device(tid_local, pk, plan, plans, sr, hop, nfft, hop_an, fscale, ws, phase_ws, edge=1.0):
+    """pvk_resynth_scan of this rank's window partials (block start phases into ``phase_ws``, local
+    Nyquist flags into ``ws``) + its hand-over record, CUDA int64 [2K] -- gathered over the ranks by
+    the caller (all_gather, world x 2K)."""
+    import ctypes as C
+    from . import _lib
+    L = _lib.lib()
+    F, K = tid_local.shape
+    tstart, tlen, toff, nt = _pk_args(pk)
+    lo, hi = handover_rows(plan, plans, nfft, hop_an, edge)
+    dev = tid_local.device
+    with torch.cuda.device(dev):
+        rec = torch.empty((2 * K,), dtype=torch.int64, device=dev)
+        _lib.check(L.pvk_resynth_scan(P._ptr(tid_local), F, K, nt, P._ptr(tstart), P._ptr(tlen), P._ptr(toff),
+                                      P._ptr(pk["pf"]), P._ptr(pk["prealph"]), float(sr), int(hop), int(nfft),
+                                      int(hop_an), float(fscale), P._ptr(ws), int(ws.numel()), P._ptr(phase_ws),
+                                      int(phase_ws.numel()), lo, hi, P._ptr(rec), rec.numel(), P._stream()),
+                   "pvk_resynth_scan")
+    return rec
+
+
+def handover_apply_device(tid_local, pk, plan, plans, recs, nfft, hop_an, ws, phase_ws, edge=1.0):
+    """pvk_resynth_handover: the true block start phases of the partials alive at this rank's hand-over
+    row, from the records of all ranks ``recs`` (CUDA int64 [world * 2K])."""
+    from . import _lib
+    L = _lib.lib()
+    F, K = tid_local.shape
+    tstart, tlen, toff, nt = _pk_args(pk)
+    lo, _ = handover_rows(plan, plans, nfft, hop_an, edge)
+    with torch.cuda.device(tid_local.device):
+        _lib.check(L.pvk_resynth_handover(P._ptr(tid_local), F, K, nt, P._ptr(tstart), P._ptr(tlen), P._ptr(toff),
+                                          P._ptr(phase_ws), int(phase_ws.numel()), P._ptr(recs), recs.numel(),
+                                          len(plans), plan["rank"], lo, P._ptr(ws), int(ws.numel()), P._stream()),
+                   "pvk_resynth_handover")
+
+
+def nyquist_flags_device(f_own, tid_own, ntracks, sr, fscale):
+    """uint8 CUDA [ntracks]: 1 for the global partials with a point of this rank's own rows at
+    fscale * f >= sr / 2.  The own rows partition the frames, so the element-wise max over the ranks
+    (all_reduce MAX, by the caller) is the unsharded Nyquist rule."""
+    from . import _lib
+    L = _lib.lib()
+    dev = tid_own.device
+    flags = torch.zeros((max(int(ntracks), 1),), dtype=torch.uint8, device=dev)
+    f_own = f_own.contiguous()
+    tid_own = tid_own.contiguous()
+    with torch.cuda.device(dev):
+        _lib.check(L.pvk_nyquist_flags(P._ptr(f_own), P._ptr(tid_own), tid_own.numel(), float(sr), float(fscale),
+                                       P._ptr(flags), int(ntracks), P._stream()), "pvk_nyquist_flags")
+    return flags
+
+
+def nyquist_import_device(tid_local, pk, plan, table, flags, ntracks, ws):
+    """pvk_resynth_import_flags: the global flags of this rank's window partials into ``ws`` (where the
+    render reads them), through the global track table ``table`` (CUDA int32 [F, K])."""
+    from . import _lib
+    L = _lib.lib()
+    F, K = tid_local.shape
+    tstart, _, _, nt = _pk_args(pk)
+    with torch.cuda.device(tid_local.device):
+        _lib.check(L.pvk_resynth_import_flags(P._ptr(tid_local), F, K, nt, P._ptr(tstart), P._ptr(table),
+                                              int(table.shape[0]), plan["w0"], P._ptr(flags), int(ntracks), P._ptr(ws),
+                                              int(ws.numel()), P._stream()), "pvk_resynth_import_flags")
+
+
+def integrated_phase_local(tid_local, pk, f_local, plan, plans, tid_own, table, ntracks, sr, hop, nfft, hop_an, fscale,
+                           ws, phase_ws, edge=1.0, group=None):
+    """Scan, hand-over and Nyquist flags of one rank (phase_preserve=False): afterwards ``ws`` and
+    ``phase_ws`` hold what the unsharded scan would give for every partial point an own block reads, and
+    resynth_device(..., scanned=True) renders the own blocks.  COLLECTIVE: one all_gather of world x 2K
+    int64 records and one all_reduce(MAX) of ntracks bytes."""
+    import torch.distributed as dist
+    world = len(plans)
+    rec = handover_scan_device(tid_local, pk, plan, plans, sr, hop, nfft, hop_an, fscale, ws, phase_ws, edge)
+    if world > 1:
+        recs = torch.empty((world * rec.numel(),), dtype=torch.int64, device=rec.device)
+        dist.all_gather_into_tensor(recs, rec, group=group)
+    else:
+        recs = rec
+    handover_apply_device(tid_local, pk, plan, plans, recs, nfft, hop_an, ws, phase_ws, edge)
+    o0, n = plan["own0"], plan["nown"]
+    flags = nyquist_flags_device(f_local[o0:o0 + n], tid_own, ntracks, sr, fscale)
+    if world > 1:
+        dist.all_reduce(flags, op=dist.ReduceOp.MAX, group=group)
+    nyquist_import_device(tid_local, pk, plan, table, flags, ntracks, ws)
 
 
 # --------------------------------------------------------------------------- host API
@@ -671,16 +781,24 @@ class ShardedSinSum(object):
         ss._set_device_tracks(self.device_track_table, None, self.ntracks)
         return ss
 
-    def synth_local(self, sr=None, hop=None, edge=1.0, minframes=3, hostbuf=None, chunks=8, to_host=False):
+    def synth_local(self, sr=None, hop=None, edge=1.0, minframes=3, hostbuf=None, chunks=8, to_host=False,
+                    phase_preserve=True, fscale=1.0):
         """Render this rank's own block range of the resynthesised signal (the last rank also renders
         the tail): global samples [b0*hop, ...).  Returns (signal, first global sample).  ``hostbuf``:
-        render in ``chunks`` ranges and download each into pinned ``hostbuf['w']`` meanwhile."""
+        render in ``chunks`` ranges and download each into pinned ``hostbuf['w']`` meanwhile.
+        ``phase_preserve`` / ``fscale`` as in SinSum.synth: with ``phase_preserve=False`` the ranks hand
+        the integrated phases of the partials crossing their boundaries on to each other and agree on the
+        Nyquist rule (integrated_phase_local: one all_gather of world x 2K int64 and one all_reduce of
+        ntracks bytes), so the concatenated own signals equal the unsharded render bit for bit.
+        COLLECTIVE in that mode: every rank makes the same call."""
+        phase_preserve, fscale = P.synth_mode(phase_preserve, fscale)
         spv = self._spv
         sr = spv.sr if sr is None else sr
         hop = spv.hop if hop is None else int(hop)
         if (edge, minframes) != (spv.edge, spv.minframes):
             raise ValueError("the segment halos were planned for edge=%r, minframes=%r" % (spv.edge, spv.minframes))
-        if self._handle is None and hostbuf is None and self.local._trk is None and spv.plan["nframes"] > 0:
+        if (phase_preserve and self._handle is None and hostbuf is None and self.local._trk is None
+                and spv.plan["nframes"] > 0):
             # first use: link, numbering + gather (side stream), pack and rendering are queued back to back;
             # the counts are read once at the end
             t = self.local._tables
@@ -704,8 +822,22 @@ class ShardedSinSum(object):
         b0, b1, bound = render_range_local(spv.plan, spv.plans, ll, hop, self.nfft, self.hop, edge)
         n_local = max(min(b1 * hop, bound) - b0 * hop, 0)
         dev = tidl.device
+        nblk = b1 - b0
+        chunks = max(1, min(chunks, nblk // 64 if nblk >= 64 else 1)) if hostbuf is not None else 1
+        F, K = tidl.shape
+        ws, mode = None, {}
+        if not phase_preserve:
+            # scan -> hand-over -> flags -> render: the hand-over needs the gathered track table and the
+            # global partial count, so the integrated-phase render starts behind them
+            ws = P.resynth_workspace(F, K, int(pk["tstart"].shape[0]), max(-(-nblk // chunks), 1), dev, hop=hop)
+            pws = P._phase_ws(False, pk["pf"].numel(), dev)
+            integrated_phase_local(tidl, pk, self.local._tables["f"], spv.plan, spv.plans, self.tid_own,
+                                   self.device_track_table, self.ntracks, sr, hop, self.nfft, self.hop, fscale, ws, pws,
+                                   edge, spv.group)
+            mode = dict(phase_preserve=False, fscale=fscale, phase_ws=pws, scanned=True)
         if hostbuf is None:
-            w = resynth_local(tidl, pk, *args, None, sr, hop, self.nfft, self.hop, edge, minframes, local_last=ll)
+            w = resynth_local(tidl, pk, *args, None, sr, hop, self.nfft, self.hop, edge, minframes, ws=ws,
+                              local_last=ll, **mode)
             n, s0 = trim_local(w.numel(), b0, *args, self.max_end, hop, self.nfft, self.hop, edge)
             w = w[:n]
             return (w.cpu().numpy() if to_host else w), s0
@@ -715,15 +847,13 @@ class ShardedSinSum(object):
             out = torch.empty((n_local,), dtype=torch.float64, device=dev)
             hw = P._pinned(hostbuf, "w", (n_local,), torch.float64)
             d2h.wait_stream(cur)
-            nblk = b1 - b0
-            chunks = max(1, min(chunks, nblk // 64 if nblk >= 64 else 1))
-            F, K = tidl.shape
-            ws = P.resynth_workspace(F, K, int(pk["tstart"].shape[0]), -(-nblk // chunks), dev) if nblk else None
+            if ws is None and nblk:
+                ws = P.resynth_workspace(F, K, int(pk["tstart"].shape[0]), -(-nblk // chunks), dev)
             for i in range(chunks if nblk else 0):
                 c0, c1 = b0 + (nblk * i) // chunks, b0 + (nblk * (i + 1)) // chunks
                 n0, n1 = (c0 - b0) * hop, min((c1 - b0) * hop, n_local)
                 resynth_local(tidl, pk, *args, None, sr, hop, self.nfft, self.hop, edge, minframes, out=out[n0:n1],
-                              ws=ws, block_range=(c0, c1), reuse_tracks=i > 0, local_last=ll)
+                              ws=ws, block_range=(c0, c1), reuse_tracks=i > 0, local_last=ll, **mode)
                 ev = torch.cuda.Event()
                 ev.record(cur)
                 with torch.cuda.stream(d2h):

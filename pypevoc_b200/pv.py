@@ -400,12 +400,14 @@ def _phase_ws(phase_preserve, npts, dev):
 
 
 def _resynth_ex(L, tid, F, K, nt, nt_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop, nfft, hop_an, edge, minframes,
-                out, nout, block0, nblocks, ws, reuse_tracks, phase_preserve, fscale, phase_ws):
-    _lib.check(L.pvk_resynth_ex(_ptr(tid), F, K, nt, _ptr(nt_dev), _ptr(tstart), _ptr(tlen), _ptr(toff), _ptr(pf),
-                                _ptr(pmag), _ptr(prealph), float(sr), int(hop), int(nfft), int(hop_an), float(edge),
-                                int(minframes), _ptr(out), int(nout), int(block0), int(nblocks), _ptr(ws), int(ws.numel()),
-                                1 if reuse_tracks else 0, 1 if phase_preserve else 0, float(fscale), _ptr(phase_ws),
-                                0 if phase_ws is None else int(phase_ws.numel()), _stream()), "pvk_resynth")
+                out, nout, block0, nblocks, ws, reuse_tracks, phase_preserve, fscale, phase_ws, scanned=False):
+    # scanned: the block start phases and Nyquist flags are in place already (pvk_resynth_render)
+    fn = L.pvk_resynth_render if scanned and not reuse_tracks else L.pvk_resynth_ex
+    _lib.check(fn(_ptr(tid), F, K, nt, _ptr(nt_dev), _ptr(tstart), _ptr(tlen), _ptr(toff), _ptr(pf),
+                  _ptr(pmag), _ptr(prealph), float(sr), int(hop), int(nfft), int(hop_an), float(edge),
+                  int(minframes), _ptr(out), int(nout), int(block0), int(nblocks), _ptr(ws), int(ws.numel()),
+                  1 if reuse_tracks else 0, 1 if phase_preserve else 0, float(fscale), _ptr(phase_ws),
+                  0 if phase_ws is None else int(phase_ws.numel()), _stream()), "pvk_resynth")
 
 
 def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edge=1.0, minframes=3,
@@ -492,13 +494,17 @@ def synth_geometry(max_end, hop, nfft, hop_an, edge=1.0):
 
 def resynth_device(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, max_end=None, block0=0,
                    nblocks=-1, out=None, ws=None, reuse_tracks=False, nout=None, phase_preserve=True, fscale=1.0,
-                   phase_ws=None):
+                   phase_ws=None, scanned=False):
     """pvk_resynth_ex for one clip; returns the float64 device signal (asynchronous).  ``ws``: a
     workspace tensor to (re)use; ``reuse_tracks``: ``ws`` (and ``phase_ws``) already hold the per-partial
     masks, fade parameters (and block start phases) of an earlier call with the same tracks and
     synthesis parameters.  ``phase_preserve`` / ``fscale``: see synth_mode(); ``phase_ws``: the
-    integrated-phase scratch to (re)use, one float64 per packed point."""
+    integrated-phase scratch to (re)use, one float64 per packed point.  ``scanned``: ``ws`` and
+    ``phase_ws`` already hold the block start phases and Nyquist flags (dist.py's hand-over), so the
+    scan is left out (pvk_resynth_render)."""
     phase_preserve, fscale = synth_mode(phase_preserve, fscale)
+    if scanned and (phase_preserve or phase_ws is None):
+        raise ValueError("scanned=True needs phase_preserve=False and the phase_ws of the scan")
     L = _lib.lib()
     dev = tid.device
     F, K = tid.shape
@@ -520,7 +526,7 @@ def resynth_device(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, max_en
     with torch.cuda.device(dev):
         _resynth_ex(L, tid, F, K, nt, None, pk["tstart"], pk["tlen"], pk["toff"], pk["pf"], pk["pmag"], pk["prealph"], sr,
                     hop, nfft, hop_an, edge, minframes, out, nout, block0, nblocks, ws, reuse_tracks, phase_preserve,
-                    fscale, None if phase_preserve else phase_ws)
+                    fscale, None if phase_preserve else phase_ws, scanned)
     return out
 
 
