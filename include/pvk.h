@@ -412,6 +412,45 @@ int pvk_resynth_import_flags(const int32_t *tid, int64_t nframes, int npks, int6
                              const int32_t *table, int64_t table_rows, int64_t row0, const uint8_t *flags,
                              int64_t nflags, void *workspace, int64_t workspace_bytes, void *stream);
 
+/* ------------------------------------------------------------------ time-varying frequency ratio
+ * The _curve variants take, after fscale, a frequency-ratio curve: fcurve[row] (device, fcurve_len
+ * doubles) is the ratio of every partial in frame row `row` of the table, i.e. of output block `row`,
+ * in place of fscale (DESIGN.md 4.3).  The block advances, the in-block phase polynomial and the Nyquist
+ * test of a point use the ratio of its own row; a head runs at the ratio of its partial's first row, a
+ * tail at that of its last row.  The phase stays continuous at every block edge; the frequency steps by
+ * fcurve[b + 1] / fcurve[b] there.  fcurve = NULL: exactly the variant without _curve.  A non-NULL
+ * fcurve needs fcurve_len >= the number of rows (nframes; n / npks for pvk_nyquist_flags_curve, whose
+ * f / gid are whole rows of npks slots), fscale == 1 and phase_preserve == 0; these are checked before
+ * any CUDA call.  The values (finite, > 0) are the caller's to check.  A constant curve c renders the
+ * same bits as fscale = c.  A sharded rank passes the rows of its window (pvk_nyquist_flags_curve: of
+ * its own rows); pvk_resynth_handover needs no curve.
+ */
+int pvk_resynth_ex_curve(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                         const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                         const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                         double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                         int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                         int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                         const double *fcurve, int64_t fcurve_len, double *phase_ws, int64_t phase_ws_len,
+                         void *stream);
+int pvk_resynth_render_curve(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                             const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                             const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                             double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                             int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                             int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                             const double *fcurve, int64_t fcurve_len, double *phase_ws, int64_t phase_ws_len,
+                             void *stream);
+int pvk_resynth_scan_curve(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                           const int32_t *tlen, const int64_t *toff, const double *pf, const double *prealph,
+                           double sr, int hop, int nfft, int hop_an, double fscale, const double *fcurve,
+                           int64_t fcurve_len, void *workspace, int64_t workspace_bytes, double *phase_ws,
+                           int64_t phase_ws_len, int64_t h_lo, int64_t h_hi, int64_t *rec, int64_t rec_len,
+                           void *stream);
+int pvk_nyquist_flags_curve(const double *f, const int32_t *gid, int64_t n, double sr, double fscale,
+                            const double *fcurve, int64_t fcurve_len, int npks, uint8_t *flags, int64_t nflags,
+                            void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -59,6 +59,13 @@ SIGNATURES = {
     "pvk_resynth_handover": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _i64, _p, _i64, _i, _i, _i64, _p, _i64, _p]),
     "pvk_nyquist_flags": (_i, [_p, _p, _i64, _d, _d, _p, _i64, _p]),
     "pvk_resynth_import_flags": (_i, [_p, _i64, _i, _i64, _p, _p, _i64, _i64, _p, _i64, _p, _i64, _p]),
+    "pvk_resynth_ex_curve": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _i, _p, _i64,
+                                  _i64, _i64, _p, _i64, _i, _i, _d, _p, _i64, _p, _i64, _p]),
+    "pvk_resynth_render_curve": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _i, _p, _i64,
+                                      _i64, _i64, _p, _i64, _i, _i, _d, _p, _i64, _p, _i64, _p]),
+    "pvk_resynth_scan_curve": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _p, _i64, _p, _i64, _p,
+                                    _i64, _i64, _i64, _p, _i64, _p]),
+    "pvk_nyquist_flags_curve": (_i, [_p, _p, _i64, _d, _d, _p, _i64, _i, _p, _i64, _p]),
 }
 
 

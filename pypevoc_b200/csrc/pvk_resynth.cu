@@ -54,6 +54,11 @@ struct RParams {
   int64_t phcap;            // capacity of phase: partials with points at or beyond it are not rendered
   double fscale;            // frequency ratio
   int free_phase;           // 1: integrated phase (launch-uniform; the render kernels take it as a template)
+  const double *fcurve;     // [F] frequency ratio of every table row, in place of fscale (NULL: fscale;
+                            // launch-uniform, the kernels take it as the template flag CURVE)
+  int64_t fcurve_len;       // rows fcurve covers (checked >= F on the host).  With it RParams grows by 16
+                            // bytes, so the kernel arguments after it keep their 16-byte alignment and the
+                            // scalar-ratio kernels compile to the same instructions as without a curve
 };
 
 // np.interp at knot coordinate kf (sample position / h - knot offset) of values v[0..nfr),
@@ -148,10 +153,16 @@ __device__ __forceinline__ double phase_cycles(phase_t u) {
   return (double)(u & PHASE_MASK) * 1.0842021724855044e-19;    // * 2^-63
 }
 
+// frequency ratio of table row `row`: the launch's fscale, or the curve's value of that row (CURVE)
+template <bool CURVE>
+__device__ __forceinline__ double row_ratio(const RParams &p, int64_t row) {
+  return CURVE ? p.fcurve[row] : p.fscale;
+}
+
 // body of partial v (nfr frames) inside block b, in cycles.  FREE = false: phase-preserving
 // (PVAnalysis.py:701-736); FREE = true: integrated phase, starting at the scanned P of the block,
-// frequency scaled by fscale, no per-block correction (DESIGN.md 4.3)
-template <bool FREE>
+// frequency scaled by fscale (CURVE: by the curve's ratio of row b), no per-block correction (DESIGN.md 4.3)
+template <bool FREE, bool CURVE>
 __device__ __forceinline__ void make_body(const RParams &p, int64_t b, int v, int nfr, BodyItem &it) {
   const double h = (double)p.h;
   const int ii = (int)(b - p.tstart[v]);
@@ -161,7 +172,7 @@ __device__ __forceinline__ void make_body(const RParams &p, int64_t b, int v, in
   const Lin2 Lf = interp_block(tf, nfr, k0, p.qaf, h, p.inv_h);
   const double qk = (double)p.qk;
   if (FREE) {
-    const double fs = p.fscale * p.inv_sr;
+    const double fs = row_ratio<CURVE>(p, b) * p.inv_sr;
     const double th0 = phase_cycles(p.phase[o + ii]);
     const Lin2 Lm = interp_block(tm, nfr, ii - p.Am, p.qam, h, p.inv_h);
     PhaseSeg &s0 = it.s[0], &s1 = it.s[1];
@@ -210,7 +221,9 @@ __device__ __forceinline__ void make_body(const RParams &p, int64_t b, int v, in
 // ------------------------------------------------------------------ kernel 1: per partial
 // One warp per partial.  For the rendered ones (tlen >= minframes, :1061): find the slots of the
 // first and the last frame in the frame table, set their bits in the start / end masks and store
-// the fade-in / fade-out parameters.
+// the fade-in / fade-out parameters.  CURVE: the head runs at the ratio of the first row, the tail at
+// the ratio of the last row.
+template <bool CURVE>
 __global__ void __launch_bounds__(256) resynth_tracks_kernel(RParams p, int64_t ntracks,
                                                              const int32_t *__restrict__ ntracks_dev,
                                                              uint32_t *__restrict__ mask, TrackFade *__restrict__ tfade) {
@@ -251,8 +264,8 @@ __global__ void __launch_bounds__(256) resynth_tracks_kernel(RParams p, int64_t 
       const double fb1 = fma(Lf.s1, hd, Lf.c1);
       if (p.free_phase) {
         // integrated phase: theta(h*nfr - 1) = P of the last block + the scaled in-block sum
-        const double fs = p.fscale * p.inv_sr;
-        t.fch *= p.fscale;
+        const double fs = row_ratio<CURVE>(p, e) * p.inv_sr;
+        t.fch *= row_ratio<CURVE>(p, s);
         t.thl = phase_cycles(p.phase[o + il]) + cum_sum(Lf, (double)p.qk, hd - 1.0) * fs;
         t.fct = tf[il] * fs;
       } else {
@@ -295,17 +308,22 @@ __device__ __forceinline__ int64_t scan_find(const RParams &p, int64_t ntracks, 
   return lo;
 }
 
-// fscale * (phase advance over body block j of partial v), cycles mod 1
+// fscale (CURVE: the ratio of row tstart[v] + j) * (phase advance over body block j of partial v),
+// cycles mod 1
+template <bool CURVE>
 __device__ __forceinline__ phase_t block_advance(const RParams &p, int64_t v, int64_t j) {
   const int64_t o = p.toff[v];
   const Lin2 Lf = interp_block(p.pf + o, p.tlen[v], (int)j - p.Af, p.qaf, (double)p.h, p.inv_h);
-  return phase_fix(cum_sum(Lf, (double)p.qk, (double)p.h) * (p.fscale * p.inv_sr));
+  const double r = row_ratio<CURVE>(p, p.tstart[v] + j);
+  return phase_fix(cum_sum(Lf, (double)p.qk, (double)p.h) * (r * p.inv_sr));
 }
 
 // pass 1: one warp per group, 32 consecutive points per step.  Element of point i: the head value
 // realph[0] / 2 pi (flagged) when i starts its partial, else the advance of block i - 1.  Writes the
 // in-group segmented inclusive scan; the group's last point also carries PHASE_HEAD when the group
-// holds a partial start.  Points of partials above the Nyquist limit flag them in tfade[v].pad0.
+// holds a partial start.  Points of partials above the Nyquist limit flag them in tfade[v].pad0 (CURVE:
+// each point tested at the ratio of its own row).
+template <bool CURVE>
 __global__ void __launch_bounds__(256) phase_scan_groups_kernel(RParams p, int64_t ntracks,
                                                                 const int32_t *__restrict__ ntracks_dev,
                                                                 TrackFade *__restrict__ tfade) {
@@ -320,7 +338,7 @@ __global__ void __launch_bounds__(256) phase_scan_groups_kernel(RParams p, int64
     // advance of the block before the group's first point (lane 31 of "step -1"); every lane then
     // walks forward from the partial of the group's first point (one search per group)
     int64_t v = scan_find(p, ntracks, base);
-    phase_t dprev = base > p.toff[v] ? block_advance(p, v, base - 1 - p.toff[v]) : 0;
+    phase_t dprev = base > p.toff[v] ? block_advance<CURVE>(p, v, base - 1 - p.toff[v]) : 0;
     int64_t vflag = -1;                                            // last partial this lane flagged
     phase_t carry = 0;
     bool seen = false;                                             // a partial start in the group so far
@@ -333,8 +351,9 @@ __global__ void __launch_bounds__(256) phase_scan_groups_kernel(RParams p, int64
         while (p.toff[v + 1] <= i) ++v;
         const int64_t j = i - p.toff[v];
         head = j == 0;
-        d = block_advance(p, v, j);
-        if (p.fscale * p.pf[i] >= nyq && v != vflag) {             // one flag per lane and partial: the
+        d = block_advance<CURVE>(p, v, j);
+        const double r = row_ratio<CURVE>(p, p.tstart[v] + j);
+        if (r * p.pf[i] >= nyq && v != vflag) {                    // one flag per lane and partial: the
           vflag = v;                                               // points of a skipped partial would
           if (tfade[v].pad0 == 0) atomicOr(&tfade[v].pad0, 1);     // otherwise all hit one word
         }
@@ -431,7 +450,7 @@ __global__ void __launch_bounds__(256) phase_scan_fixup_kernel(RParams p, int64_
 // ------------------------------------------------------------------ kernel 2: per frame row
 // One warp per row of the chunk: the bodies of the rendered partials of the row, as closed-form
 // coefficients, compacted in slot order (deterministic sum order) into gitems.
-template <bool FREE>
+template <bool FREE, bool CURVE>
 __global__ void __launch_bounds__(128) resynth_prepare_kernel(RParams p, int64_t nrows, BodyItem *__restrict__ gitems,
                                                               int32_t *__restrict__ gcount) {
   const int lane = threadIdx.x & 31;
@@ -449,7 +468,7 @@ __global__ void __launch_bounds__(128) resynth_prepare_kernel(RParams p, int64_t
       }
       const bool on = v >= 0 && nfr >= p.minframes && (!FREE || p.tfade[v].pad0 == 0);   // :1061; Nyquist rule
       const unsigned mk = __ballot_sync(FULL, on);
-      if (on) make_body<FREE>(p, b, v, nfr, gitems[row * p.K + n + __popc(mk & lanemask_lt())]);
+      if (on) make_body<FREE, CURVE>(p, b, v, nfr, gitems[row * p.K + n + __popc(mk & lanemask_lt())]);
       n += __popc(mk);
     }
   }
@@ -664,7 +683,7 @@ constexpr int TILE_BATCH = 32;
 constexpr int TILE_WARP_BYTES = TILE_BATCH * (int)sizeof(BodyItem);   // 2560 >= RS * 33 * 4 for RS <= 16
 constexpr int TILE_WARPS = 4;
 
-template <int RS, bool FREE>
+template <int RS, bool FREE, bool CURVE>
 __global__ void __launch_bounds__(TILE_WARPS * 32, 8) resynth_tile_kernel(RParams p, int64_t ntiles, int tpb) {
   PVK_SMEM(smem);
   constexpr int TILE = 32 * RS;
@@ -694,7 +713,7 @@ __global__ void __launch_bounds__(TILE_WARPS * 32, 8) resynth_tile_kernel(RParam
       const bool on = v >= 0 && nfr >= p.minframes && (!FREE || p.tfade[v].pad0 == 0);   // :1061; Nyquist rule
       const unsigned mk = __ballot_sync(FULL, on);
       if (mk == 0u) continue;                                      // warp uniform
-      if (on) make_body<FREE>(p, b, v, nfr, items[__popc(mk & lanemask_lt())]);
+      if (on) make_body<FREE, CURVE>(p, b, v, nfr, items[__popc(mk & lanemask_lt())]);
       __syncwarp();
       render_bodies<RS>(p, items, __popc(mk), 0, 1, qs, fast, acc);
       __syncwarp();
@@ -753,10 +772,12 @@ static int launch_resynth_tile(const RParams &p, int64_t nblocks, void *stream) 
   const int tpb = p.h / (32 * RS);
   const int64_t ntiles = nblocks * tpb;
   const dim3 grid((unsigned)((ntiles + TILE_WARPS - 1) / TILE_WARPS)), block(TILE_WARPS * 32);
-  if (p.free_phase)
-    PVK_LAUNCH((resynth_tile_kernel<RS, true>), grid, block, TILE_WARPS * TILE_WARP_BYTES, stream, p, ntiles, tpb);
+  if (p.fcurve != nullptr)
+    PVK_LAUNCH((resynth_tile_kernel<RS, true, true>), grid, block, TILE_WARPS * TILE_WARP_BYTES, stream, p, ntiles, tpb);
+  else if (p.free_phase)
+    PVK_LAUNCH((resynth_tile_kernel<RS, true, false>), grid, block, TILE_WARPS * TILE_WARP_BYTES, stream, p, ntiles, tpb);
   else
-    PVK_LAUNCH((resynth_tile_kernel<RS, false>), grid, block, TILE_WARPS * TILE_WARP_BYTES, stream, p, ntiles, tpb);
+    PVK_LAUNCH((resynth_tile_kernel<RS, false, false>), grid, block, TILE_WARPS * TILE_WARP_BYTES, stream, p, ntiles, tpb);
   PVK_CHECK_LAUNCH("pvk_resynth(render tiles)");
   return PVK_OK;
 }
@@ -798,7 +819,22 @@ static void synth_params(RParams &p, double sr, int hop, int nfft, int hop_an, i
   p.hpc = 3.141592653589793 / (2.0 * p.fstep);
   p.mwk = (npks + 31) / 32;
   p.fscale = fscale;
+  p.fcurve = nullptr;
+  p.fcurve_len = 0;
 }
+
+// the argument checks of a frequency-ratio curve (the _curve exports): one ratio per table row, none
+// together with a scalar ratio or the phase-preserving model; the values are the caller's to check
+#define PVK_REQUIRE_CURVE(fn, nrows, phase_preserve)                                                            \
+  do {                                                                                                       \
+    if (fcurve != nullptr) {                                                                                 \
+      PVK_REQUIRE(fcurve_len >= (nrows), fn ": fcurve_len=%lld is short (one ratio per frame row, %lld rows)", \
+                  (long long)fcurve_len, (long long)(nrows));                                                \
+      PVK_REQUIRE(fscale == 1.0, fn ": fscale=%g with an fcurve (the curve carries the ratio; pass 1)", fscale); \
+      PVK_REQUIRE(!(phase_preserve), fn ": an fcurve needs phase_preserve=0 (the analysed phases do not fit a " \
+                  "scaled frequency)");                                                                      \
+    }                                                                                                        \
+  } while (0)
 
 // block start phases + Nyquist flags (tfade[v].pad0) of every partial: the three scan passes
 static int launch_phase_scan(const RParams &p, int64_t ntracks, const int32_t *ntracks_dev, TrackFade *tfade,
@@ -808,7 +844,10 @@ static int launch_phase_scan(const RParams &p, int64_t ntracks, const int32_t *n
   int64_t sg = ((pcap + SCAN_GROUP - 1) / SCAN_GROUP * 32 + 255) / 256;
   if (sg > 148 * 16) sg = 148 * 16;
   if (sg < 1) sg = 1;
-  PVK_LAUNCH(phase_scan_groups_kernel, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev, tfade);
+  if (p.fcurve != nullptr)
+    PVK_LAUNCH(phase_scan_groups_kernel<true>, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev, tfade);
+  else
+    PVK_LAUNCH(phase_scan_groups_kernel<false>, dim3((unsigned)sg), dim3(256), 0, stream, p, ntracks, ntracks_dev, tfade);
   PVK_CHECK_LAUNCH("pvk_resynth(phase scan)");
   PVK_LAUNCH(phase_scan_carry_kernel, dim3(1), dim3(SCAN_CARRY_THREADS), SCAN_CARRY_SMEM, stream, p, ntracks, ntracks_dev);
   PVK_CHECK_LAUNCH("pvk_resynth(phase carry)");
@@ -825,7 +864,8 @@ static int resynth_run(bool scan, const int32_t *tid, int64_t nframes, int npks,
                        double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
                        int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
                        int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
-                       double *phase_ws, int64_t phase_ws_len, void *stream) {
+                       const double *fcurve, int64_t fcurve_len, double *phase_ws, int64_t phase_ws_len,
+                       void *stream) {
   PVK_REQUIRE(isfinite(fscale) && fscale > 0.0, "pvk_resynth: fscale=%g must be finite and > 0", fscale);
   PVK_REQUIRE(!phase_preserve || fscale == 1.0,
               "pvk_resynth: fscale=%g needs phase_preserve=0 (the analysed phases do not fit a scaled frequency)",
@@ -867,6 +907,8 @@ static int resynth_run(bool scan, const int32_t *tid, int64_t nframes, int npks,
   p.phase = reinterpret_cast<unsigned long long *>(phase_ws);
   p.phcap = phase_preserve ? 0 : phase_ws_len;
   p.free_phase = phase_preserve ? 0 : 1;
+  p.fcurve = fcurve;
+  p.fcurve_len = fcurve_len;
 
   // workspace: masks | fade parameters | staged bodies + counts of one chunk of blocks
   unsigned char *ws = reinterpret_cast<unsigned char *>(workspace);
@@ -890,7 +932,10 @@ static int resynth_run(bool scan, const int32_t *tid, int64_t nframes, int npks,
     }
     int64_t gsz = (ntracks * 32 + 255) / 256;
     if (gsz > 148 * 16) gsz = 148 * 16;
-    PVK_LAUNCH(resynth_tracks_kernel, dim3((unsigned)gsz), dim3(256), 0, stream, p, ntracks, ntracks_dev, mask, tfade);
+    if (p.fcurve != nullptr)
+      PVK_LAUNCH(resynth_tracks_kernel<true>, dim3((unsigned)gsz), dim3(256), 0, stream, p, ntracks, ntracks_dev, mask, tfade);
+    else
+      PVK_LAUNCH(resynth_tracks_kernel<false>, dim3((unsigned)gsz), dim3(256), 0, stream, p, ntracks, ntracks_dev, mask, tfade);
     PVK_CHECK_LAUNCH("pvk_resynth(tracks)");
   }
   // thread layout of the render kernel: RS samples per thread, nchp chunk threads per item
@@ -913,10 +958,13 @@ static int resynth_run(bool scan, const int32_t *tid, int64_t nframes, int npks,
     p.chunk0 = c0;
     p.block0 = c0;
     p.out = out + (c0 - block0) * (int64_t)hop;
-    if (p.free_phase)
-      PVK_LAUNCH(resynth_prepare_kernel<true>, dim3((unsigned)((n + 3) / 4)), dim3(128), 0, stream, p, n, gitems, gcount);
+    const dim3 pgrid((unsigned)((n + 3) / 4));
+    if (p.fcurve != nullptr)
+      PVK_LAUNCH((resynth_prepare_kernel<true, true>), pgrid, dim3(128), 0, stream, p, n, gitems, gcount);
+    else if (p.free_phase)
+      PVK_LAUNCH((resynth_prepare_kernel<true, false>), pgrid, dim3(128), 0, stream, p, n, gitems, gcount);
     else
-      PVK_LAUNCH(resynth_prepare_kernel<false>, dim3((unsigned)((n + 3) / 4)), dim3(128), 0, stream, p, n, gitems, gcount);
+      PVK_LAUNCH((resynth_prepare_kernel<false, false>), pgrid, dim3(128), 0, stream, p, n, gitems, gcount);
     PVK_CHECK_LAUNCH("pvk_resynth(prepare)");
     const int rc = RS == 16 ? launch_resynth<16>(p, n, bd, stream) : launch_resynth<8>(p, n, bd, stream);
     if (rc != PVK_OK) return rc;
@@ -933,7 +981,21 @@ extern "C" int pvk_resynth_ex(const int32_t *tid, int64_t nframes, int npks, int
                               double *phase_ws, int64_t phase_ws_len, void *stream) {
   return resynth_run(true, tid, nframes, npks, ntracks, ntracks_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop,
                      nfft, hop_an, edge, minframes, out, nout, block0, nblocks, workspace, workspace_bytes,
-                     reuse_tracks, phase_preserve, fscale, phase_ws, phase_ws_len, stream);
+                     reuse_tracks, phase_preserve, fscale, nullptr, 0, phase_ws, phase_ws_len, stream);
+}
+
+extern "C" int pvk_resynth_ex_curve(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                                    const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                                    const int64_t *toff, const double *pf, const double *pmag, const double *prealph,
+                                    double sr, int hop, int nfft, int hop_an, double edge, int minframes, double *out,
+                                    int64_t nout, int64_t block0, int64_t nblocks, void *workspace,
+                                    int64_t workspace_bytes, int reuse_tracks, int phase_preserve, double fscale,
+                                    const double *fcurve, int64_t fcurve_len, double *phase_ws, int64_t phase_ws_len,
+                                    void *stream) {
+  PVK_REQUIRE_CURVE("pvk_resynth_ex_curve", nframes, phase_preserve);
+  return resynth_run(true, tid, nframes, npks, ntracks, ntracks_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop,
+                     nfft, hop_an, edge, minframes, out, nout, block0, nblocks, workspace, workspace_bytes,
+                     reuse_tracks, phase_preserve, fscale, fcurve, fcurve_len, phase_ws, phase_ws_len, stream);
 }
 
 extern "C" int pvk_resynth_render(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
@@ -946,7 +1008,23 @@ extern "C" int pvk_resynth_render(const int32_t *tid, int64_t nframes, int npks,
   PVK_REQUIRE(!phase_preserve, "pvk_resynth_render: phase_preserve=1 has no scan to leave out (use pvk_resynth_ex)");
   return resynth_run(false, tid, nframes, npks, ntracks, ntracks_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop,
                      nfft, hop_an, edge, minframes, out, nout, block0, nblocks, workspace, workspace_bytes,
-                     reuse_tracks, phase_preserve, fscale, phase_ws, phase_ws_len, stream);
+                     reuse_tracks, phase_preserve, fscale, nullptr, 0, phase_ws, phase_ws_len, stream);
+}
+
+extern "C" int pvk_resynth_render_curve(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                                        const int32_t *ntracks_dev, const int32_t *tstart, const int32_t *tlen,
+                                        const int64_t *toff, const double *pf, const double *pmag,
+                                        const double *prealph, double sr, int hop, int nfft, int hop_an, double edge,
+                                        int minframes, double *out, int64_t nout, int64_t block0, int64_t nblocks,
+                                        void *workspace, int64_t workspace_bytes, int reuse_tracks, int phase_preserve,
+                                        double fscale, const double *fcurve, int64_t fcurve_len, double *phase_ws,
+                                        int64_t phase_ws_len, void *stream) {
+  PVK_REQUIRE_CURVE("pvk_resynth_render_curve", nframes, phase_preserve);
+  PVK_REQUIRE(!phase_preserve,
+              "pvk_resynth_render_curve: phase_preserve=1 has no scan to leave out (use pvk_resynth_ex)");
+  return resynth_run(false, tid, nframes, npks, ntracks, ntracks_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop,
+                     nfft, hop_an, edge, minframes, out, nout, block0, nblocks, workspace, workspace_bytes,
+                     reuse_tracks, phase_preserve, fscale, fcurve, fcurve_len, phase_ws, phase_ws_len, stream);
 }
 
 // ------------------------------------------------------------------ integrated phase across segments
@@ -1034,14 +1112,17 @@ __global__ void __launch_bounds__(256) handover_fixup_kernel(RParams p, int64_t 
     p.phase[o + i] = (p.phase[o + i] + d) & PHASE_MASK;
 }
 
-// global Nyquist flags: flags[gid[i]] = 1 for every point with fscale * f >= sr / 2 (the scan's test)
+// global Nyquist flags: flags[gid[i]] = 1 for every point with fscale * f >= sr / 2 (the scan's test;
+// CURVE: the ratio of the point's row i / K, fcurve[i / K], in place of fscale)
+template <bool CURVE>
 __global__ void __launch_bounds__(256) nyquist_scatter_kernel(const double *__restrict__ f, const int32_t *__restrict__ gid,
                                                               int64_t n, double sr, double fscale, uint8_t *flags,
-                                                              int64_t nflags) {
+                                                              int64_t nflags, const double *__restrict__ fcurve, int K) {
   const double nyq = 0.5 * sr;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const int g = gid[i];
-    if (g >= 0 && g < nflags && fscale * f[i] >= nyq && flags[g] == 0) flags[g] = 1;
+    const double r = CURVE ? fcurve[i / K] : fscale;
+    if (g >= 0 && g < nflags && r * f[i] >= nyq && flags[g] == 0) flags[g] = 1;
   }
 }
 
@@ -1079,11 +1160,11 @@ static TrackFade *resynth_tfade(void *workspace, int64_t nframes, int npks) {
               fn ": workspace too small (%lld bytes; pvk_resynth_workspace_bytes gives the size)",                 \
               (long long)workspace_bytes)
 
-extern "C" int pvk_resynth_scan(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
-                                const int32_t *tlen, const int64_t *toff, const double *pf, const double *prealph,
-                                double sr, int hop, int nfft, int hop_an, double fscale, void *workspace,
-                                int64_t workspace_bytes, double *phase_ws, int64_t phase_ws_len, int64_t h_lo,
-                                int64_t h_hi, int64_t *rec, int64_t rec_len, void *stream) {
+static int resynth_scan_run(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                            const int32_t *tlen, const int64_t *toff, const double *pf, const double *prealph,
+                            double sr, int hop, int nfft, int hop_an, double fscale, const double *fcurve,
+                            int64_t fcurve_len, void *workspace, int64_t workspace_bytes, double *phase_ws, int64_t phase_ws_len,
+                            int64_t h_lo, int64_t h_hi, int64_t *rec, int64_t rec_len, void *stream) {
   PVK_REQUIRE(isfinite(fscale) && fscale > 0.0, "pvk_resynth_scan: fscale=%g must be finite and > 0", fscale);
   PVK_REQUIRE(hop >= 1 && nfft >= 1 && hop_an >= 1, "pvk_resynth_scan: hop=%d nfft=%d hop_an=%d must be >= 1", hop,
               nfft, hop_an);
@@ -1109,6 +1190,8 @@ extern "C" int pvk_resynth_scan(const int32_t *tid, int64_t nframes, int npks, i
   p.phase = reinterpret_cast<unsigned long long *>(phase_ws);
   p.phcap = phase_ws_len;
   p.free_phase = 1;
+  p.fcurve = fcurve;
+  p.fcurve_len = fcurve_len;
   if (ntracks > 0 && nframes > 0) {
     const int rc = launch_phase_scan(p, ntracks, nullptr, resynth_tfade(workspace, nframes, npks), stream);
     if (rc != PVK_OK) return rc;
@@ -1119,6 +1202,26 @@ extern "C" int pvk_resynth_scan(const int32_t *tid, int64_t nframes, int npks, i
     PVK_CHECK_LAUNCH("pvk_resynth_scan(record)");
   }
   return PVK_OK;
+}
+
+extern "C" int pvk_resynth_scan(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                                const int32_t *tlen, const int64_t *toff, const double *pf, const double *prealph,
+                                double sr, int hop, int nfft, int hop_an, double fscale, void *workspace,
+                                int64_t workspace_bytes, double *phase_ws, int64_t phase_ws_len, int64_t h_lo,
+                                int64_t h_hi, int64_t *rec, int64_t rec_len, void *stream) {
+  return resynth_scan_run(tid, nframes, npks, ntracks, tstart, tlen, toff, pf, prealph, sr, hop, nfft, hop_an, fscale,
+                          nullptr, 0, workspace, workspace_bytes, phase_ws, phase_ws_len, h_lo, h_hi, rec, rec_len, stream);
+}
+
+extern "C" int pvk_resynth_scan_curve(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                                      const int32_t *tstart, const int32_t *tlen, const int64_t *toff, const double *pf,
+                                      const double *prealph, double sr, int hop, int nfft, int hop_an, double fscale,
+                                      const double *fcurve, int64_t fcurve_len, void *workspace,
+                                      int64_t workspace_bytes, double *phase_ws, int64_t phase_ws_len, int64_t h_lo,
+                                      int64_t h_hi, int64_t *rec, int64_t rec_len, void *stream) {
+  PVK_REQUIRE_CURVE("pvk_resynth_scan_curve", nframes, 0);
+  return resynth_scan_run(tid, nframes, npks, ntracks, tstart, tlen, toff, pf, prealph, sr, hop, nfft, hop_an, fscale,
+                          fcurve, fcurve_len, workspace, workspace_bytes, phase_ws, phase_ws_len, h_lo, h_hi, rec, rec_len, stream);
 }
 
 extern "C" int pvk_resynth_handover(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
@@ -1157,8 +1260,8 @@ extern "C" int pvk_resynth_handover(const int32_t *tid, int64_t nframes, int npk
   return PVK_OK;
 }
 
-extern "C" int pvk_nyquist_flags(const double *f, const int32_t *gid, int64_t n, double sr, double fscale,
-                                 uint8_t *flags, int64_t nflags, void *stream) {
+static int nyquist_flags_run(const double *f, const int32_t *gid, int64_t n, double sr, double fscale,
+                             const double *fcurve, int npks, uint8_t *flags, int64_t nflags, void *stream) {
   PVK_REQUIRE(isfinite(fscale) && fscale > 0.0, "pvk_nyquist_flags: fscale=%g must be finite and > 0", fscale);
   PVK_REQUIRE(sr > 0.0, "pvk_nyquist_flags: sr must be positive");
   PVK_REQUIRE(n >= 0 && nflags >= 0, "pvk_nyquist_flags: negative sizes");
@@ -1167,9 +1270,30 @@ extern "C" int pvk_nyquist_flags(const double *f, const int32_t *gid, int64_t n,
   if (n == 0 || nflags == 0) return PVK_OK;
   int64_t g = (n + 255) / 256;
   if (g > 148 * 8) g = 148 * 8;
-  PVK_LAUNCH(nyquist_scatter_kernel, dim3((unsigned)g), dim3(256), 0, stream, f, gid, n, sr, fscale, flags, nflags);
+  if (fcurve != nullptr)
+    PVK_LAUNCH(nyquist_scatter_kernel<true>, dim3((unsigned)g), dim3(256), 0, stream, f, gid, n, sr, fscale, flags, nflags,
+               fcurve, npks);
+  else
+    PVK_LAUNCH(nyquist_scatter_kernel<false>, dim3((unsigned)g), dim3(256), 0, stream, f, gid, n, sr, fscale, flags,
+               nflags, nullptr, 1);
   PVK_CHECK_LAUNCH("pvk_nyquist_flags");
   return PVK_OK;
+}
+
+extern "C" int pvk_nyquist_flags(const double *f, const int32_t *gid, int64_t n, double sr, double fscale,
+                                 uint8_t *flags, int64_t nflags, void *stream) {
+  return nyquist_flags_run(f, gid, n, sr, fscale, nullptr, 1, flags, nflags, stream);
+}
+
+extern "C" int pvk_nyquist_flags_curve(const double *f, const int32_t *gid, int64_t n, double sr, double fscale,
+                                       const double *fcurve, int64_t fcurve_len, int npks, uint8_t *flags,
+                                       int64_t nflags, void *stream) {
+  PVK_REQUIRE(npks >= 1 && npks <= PVK_MAX_NPKS, "pvk_nyquist_flags_curve: npks=%d must be in [1, %d]", npks,
+              PVK_MAX_NPKS);
+  PVK_REQUIRE(n >= 0 && n % npks == 0, "pvk_nyquist_flags_curve: n=%lld is not a whole number of rows of %d",
+              (long long)n, npks);
+  PVK_REQUIRE_CURVE("pvk_nyquist_flags_curve", n / npks, 0);
+  return nyquist_flags_run(f, gid, n, sr, fscale, fcurve, npks, flags, nflags, stream);
 }
 
 extern "C" int pvk_resynth_import_flags(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,

@@ -615,7 +615,8 @@ def _pk_args(pk):
 def handover_scan_device(tid_local, pk, plan, plans, sr, hop, nfft, hop_an, fscale, ws, phase_ws, edge=1.0):
     """pvk_resynth_scan of this rank's window partials (block start phases into ``phase_ws``, local
     Nyquist flags into ``ws``) + its hand-over record, CUDA int64 [2K] -- gathered over the ranks by
-    the caller (all_gather, world x 2K)."""
+    the caller (all_gather, world x 2K).  ``fscale``: a float, or a pv._DeviceCurve of the window rows
+    (pvk_resynth_scan_curve)."""
     import ctypes as C
     from . import _lib
     L = _lib.lib()
@@ -625,11 +626,14 @@ def handover_scan_device(tid_local, pk, plan, plans, sr, hop, nfft, hop_an, fsca
     dev = tid_local.device
     with torch.cuda.device(dev):
         rec = torch.empty((2 * K,), dtype=torch.int64, device=dev)
-        _lib.check(L.pvk_resynth_scan(P._ptr(tid_local), F, K, nt, P._ptr(tstart), P._ptr(tlen), P._ptr(toff),
-                                      P._ptr(pk["pf"]), P._ptr(pk["prealph"]), float(sr), int(hop), int(nfft),
-                                      int(hop_an), float(fscale), P._ptr(ws), int(ws.numel()), P._ptr(phase_ws),
-                                      int(phase_ws.numel()), lo, hi, P._ptr(rec), rec.numel(), P._stream()),
-                   "pvk_resynth_scan")
+        if isinstance(fscale, P._DeviceCurve):
+            fn, ratio = L.pvk_resynth_scan_curve, (1.0, P._ptr(fscale.t), int(fscale.t.numel()))
+        else:
+            fn, ratio = L.pvk_resynth_scan, (float(fscale),)
+        _lib.check(fn(P._ptr(tid_local), F, K, nt, P._ptr(tstart), P._ptr(tlen), P._ptr(toff), P._ptr(pk["pf"]),
+                      P._ptr(pk["prealph"]), float(sr), int(hop), int(nfft), int(hop_an), *ratio, P._ptr(ws),
+                      int(ws.numel()), P._ptr(phase_ws), int(phase_ws.numel()), lo, hi, P._ptr(rec), rec.numel(),
+                      P._stream()), "pvk_resynth_scan")
     return rec
 
 
@@ -651,7 +655,8 @@ def handover_apply_device(tid_local, pk, plan, plans, recs, nfft, hop_an, ws, ph
 def nyquist_flags_device(f_own, tid_own, ntracks, sr, fscale):
     """uint8 CUDA [ntracks]: 1 for the global partials with a point of this rank's own rows at
     fscale * f >= sr / 2.  The own rows partition the frames, so the element-wise max over the ranks
-    (all_reduce MAX, by the caller) is the unsharded Nyquist rule."""
+    (all_reduce MAX, by the caller) is the unsharded Nyquist rule.  ``fscale``: a float, or a
+    pv._DeviceCurve of the own rows (each point tested at its row's ratio)."""
     from . import _lib
     L = _lib.lib()
     dev = tid_own.device
@@ -659,8 +664,13 @@ def nyquist_flags_device(f_own, tid_own, ntracks, sr, fscale):
     f_own = f_own.contiguous()
     tid_own = tid_own.contiguous()
     with torch.cuda.device(dev):
-        _lib.check(L.pvk_nyquist_flags(P._ptr(f_own), P._ptr(tid_own), tid_own.numel(), float(sr), float(fscale),
-                                       P._ptr(flags), int(ntracks), P._stream()), "pvk_nyquist_flags")
+        if isinstance(fscale, P._DeviceCurve):
+            _lib.check(L.pvk_nyquist_flags_curve(P._ptr(f_own), P._ptr(tid_own), tid_own.numel(), float(sr), 1.0,
+                                                 P._ptr(fscale.t), int(fscale.t.numel()), int(tid_own.shape[1]),
+                                                 P._ptr(flags), int(ntracks), P._stream()), "pvk_nyquist_flags_curve")
+        else:
+            _lib.check(L.pvk_nyquist_flags(P._ptr(f_own), P._ptr(tid_own), tid_own.numel(), float(sr), float(fscale),
+                                           P._ptr(flags), int(ntracks), P._stream()), "pvk_nyquist_flags")
     return flags
 
 
@@ -682,7 +692,8 @@ def integrated_phase_local(tid_local, pk, f_local, plan, plans, tid_own, table, 
     """Scan, hand-over and Nyquist flags of one rank (phase_preserve=False): afterwards ``ws`` and
     ``phase_ws`` hold what the unsharded scan would give for every partial point an own block reads, and
     resynth_device(..., scanned=True) renders the own blocks.  COLLECTIVE: one all_gather of world x 2K
-    int64 records and one all_reduce(MAX) of ntracks bytes."""
+    int64 records and one all_reduce(MAX) of ntracks bytes.  ``fscale``: a float, or a pv._DeviceCurve
+    of the window rows [w0, w1) (the flags take its own-row part)."""
     import torch.distributed as dist
     world = len(plans)
     rec = handover_scan_device(tid_local, pk, plan, plans, sr, hop, nfft, hop_an, fscale, ws, phase_ws, edge)
@@ -693,7 +704,8 @@ def integrated_phase_local(tid_local, pk, f_local, plan, plans, tid_own, table, 
         recs = rec
     handover_apply_device(tid_local, pk, plan, plans, recs, nfft, hop_an, ws, phase_ws, edge)
     o0, n = plan["own0"], plan["nown"]
-    flags = nyquist_flags_device(f_local[o0:o0 + n], tid_own, ntracks, sr, fscale)
+    own = P._DeviceCurve(fscale.t[o0:o0 + n]) if isinstance(fscale, P._DeviceCurve) else fscale
+    flags = nyquist_flags_device(f_local[o0:o0 + n], tid_own, ntracks, sr, own)
     if world > 1:
         dist.all_reduce(flags, op=dist.ReduceOp.MAX, group=group)
     nyquist_import_device(tid_local, pk, plan, table, flags, ntracks, ws)
@@ -790,9 +802,13 @@ class ShardedSinSum(object):
         the integrated phases of the partials crossing their boundaries on to each other and agree on the
         Nyquist rule (integrated_phase_local: one all_gather of world x 2K int64 and one all_reduce of
         ntracks bytes), so the concatenated own signals equal the unsharded render bit for bit.
-        COLLECTIVE in that mode: every rank makes the same call."""
-        phase_preserve, fscale = P.synth_mode(phase_preserve, fscale)
+        COLLECTIVE in that mode: every rank makes the same call.  ``fscale`` may be a curve over the
+        GLOBAL frames, ``[frames_total]`` (see pv.synth_mode()); each rank uses its window's rows.  It is
+        checked on every rank before anything is launched."""
         spv = self._spv
+        phase_preserve, fscale = P.synth_mode(phase_preserve, fscale, nframes=spv.plans[0]["frames_total"])
+        if isinstance(fscale, np.ndarray):
+            fscale = P._on_device(np.ascontiguousarray(fscale[spv.plan["w0"]:spv.plan["w1"]]), spv.pv._dev)
         sr = spv.sr if sr is None else sr
         hop = spv.hop if hop is None else int(hop)
         if (edge, minframes) != (spv.edge, spv.minframes):

@@ -375,11 +375,60 @@ def track_pack_device(fd, magd, phd, realphd, maxpitchjmp=0.5, after_link=None):
     return tr, pk
 
 
-def synth_mode(phase_preserve=True, fscale=1.0):
+class _DeviceCurve(object):
+    """A frequency-ratio curve that synth_mode() has checked, uploaded once per call: ``t`` is a
+    float64 CUDA tensor with one ratio per frame row of the table it goes with."""
+    __slots__ = ("t",)
+
+    def __init__(self, t):
+        self.t = t
+
+
+def _curve_values(fscale):
+    """float64 numpy copy of a ratio curve of any shape, every value finite and > 0."""
+    if isinstance(fscale, torch.Tensor):
+        if fscale.dtype == torch.bool or fscale.is_complex():
+            raise TypeError("an fscale curve must hold real numbers, not %s" % fscale.dtype)
+        a = fscale.detach().cpu().numpy()
+    else:
+        a = np.asarray(fscale)
+    if a.dtype.kind not in "iuf":
+        raise TypeError("an fscale curve must hold real numbers, not %s" % a.dtype)
+    a = np.ascontiguousarray(a, dtype=np.float64)
+    if not np.all(np.isfinite(a)) or np.any(a <= 0.0):
+        raise ValueError("every value of an fscale curve must be finite and > 0")
+    return a
+
+
+def synth_mode(phase_preserve=True, fscale=1.0, nframes=None):
     """Checked (phase_preserve, fscale) of a resynthesis call.  ``phase_preserve=False`` integrates the
     phase from the frequency track (pitch shift by ``fscale``, time stretch by a synthesis hop other
     than the analysis hop); the phase-preserving model honours the analysed phases and so takes no
-    ``fscale`` other than 1."""
+    ``fscale`` other than 1.
+
+    ``fscale`` is one ratio for the whole signal, or a curve: a 1-D numpy array, sequence or torch
+    tensor of ``nframes`` real ratios, one per analysis frame (row of the frame table), returned as a
+    float64 numpy array.  Ratio ``r[b]`` applies to every partial in output block ``b`` (output samples
+    ``[b*hop, (b+1)*hop)``, input samples ``[b*hop_an, (b+1)*hop_an)``); the phase stays continuous
+    and the frequency steps by ``r[b+1] / r[b]`` between blocks (DESIGN.md 4.3).  To build one from
+    time, use the input time of the frame rows, ``r = ratio_of(np.arange(nframes) * hop_an / sr)``
+    (not ``PV.t``, which is offset by ``nfft / 2``).  A curve needs ``phase_preserve=False``."""
+    if isinstance(fscale, _DeviceCurve):
+        if phase_preserve:
+            raise ValueError("an fscale curve needs phase_preserve=False")
+        if nframes is not None and fscale.t.numel() != nframes:
+            raise ValueError("the fscale curve has %d ratios for %d frames" % (fscale.t.numel(), nframes))
+        return False, fscale
+    if isinstance(fscale, (np.ndarray, torch.Tensor, list, tuple)):
+        r = _curve_values(fscale)
+        if r.ndim != 1:
+            raise ValueError("an fscale curve must be 1-D (one ratio per frame), not of shape %s" % (r.shape,))
+        if nframes is not None and len(r) != nframes:
+            raise ValueError("the fscale curve has %d ratios for %d frames" % (len(r), nframes))
+        if phase_preserve:
+            raise ValueError("an fscale curve needs phase_preserve=False: the analysed phases cannot be honoured "
+                             "at a scaled frequency")
+        return False, r
     if isinstance(fscale, bool) or not isinstance(fscale, (int, float, np.integer, np.floating)):
         raise TypeError("fscale must be a real number, not %s" % type(fscale).__name__)
     fscale = float(fscale)
@@ -392,6 +441,13 @@ def synth_mode(phase_preserve=True, fscale=1.0):
     return phase_preserve, fscale
 
 
+def _on_device(fscale, dev):
+    """fscale as the kernels take it: a float, or a checked curve (numpy) uploaded as float64."""
+    if isinstance(fscale, np.ndarray):
+        return _DeviceCurve(torch.from_numpy(fscale).to(dev))
+    return fscale
+
+
 def _phase_ws(phase_preserve, npts, dev):
     """Scratch of the integrated-phase scan: one double per packed point (None when preserving phase)."""
     if phase_preserve:
@@ -402,11 +458,18 @@ def _phase_ws(phase_preserve, npts, dev):
 def _resynth_ex(L, tid, F, K, nt, nt_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop, nfft, hop_an, edge, minframes,
                 out, nout, block0, nblocks, ws, reuse_tracks, phase_preserve, fscale, phase_ws, scanned=False):
     # scanned: the block start phases and Nyquist flags are in place already (pvk_resynth_render)
-    fn = L.pvk_resynth_render if scanned and not reuse_tracks else L.pvk_resynth_ex
+    # fscale: a float, or a _DeviceCurve (the _curve exports, ratio 1 + the curve)
+    render = scanned and not reuse_tracks
+    if isinstance(fscale, _DeviceCurve):
+        fn = L.pvk_resynth_render_curve if render else L.pvk_resynth_ex_curve
+        ratio = (1.0, _ptr(fscale.t), int(fscale.t.numel()))
+    else:
+        fn = L.pvk_resynth_render if render else L.pvk_resynth_ex
+        ratio = (float(fscale),)
     _lib.check(fn(_ptr(tid), F, K, nt, _ptr(nt_dev), _ptr(tstart), _ptr(tlen), _ptr(toff), _ptr(pf),
                   _ptr(pmag), _ptr(prealph), float(sr), int(hop), int(nfft), int(hop_an), float(edge),
                   int(minframes), _ptr(out), int(nout), int(block0), int(nblocks), _ptr(ws), int(ws.numel()),
-                  1 if reuse_tracks else 0, 1 if phase_preserve else 0, float(fscale), _ptr(phase_ws),
+                  1 if reuse_tracks else 0, 1 if phase_preserve else 0, *ratio, _ptr(phase_ws),
                   0 if phase_ws is None else int(phase_ws.numel()), _stream()), "pvk_resynth")
 
 
@@ -423,8 +486,9 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
     uncut (segment-sharded runs: the caller knows its block range without any count and trims once the
     global last frame is known).  ``before_sync`` (optional) is called once everything is queued,
     before the host waits: work launched there runs behind the rendering instead of after the wait.
-    ``phase_preserve`` / ``fscale``: see synth_mode()."""
-    phase_preserve, fscale = synth_mode(phase_preserve, fscale)
+    ``phase_preserve`` / ``fscale``: see synth_mode() (a curve has one ratio per row of ``fd``)."""
+    phase_preserve, fscale = synth_mode(phase_preserve, fscale, nframes=fd.shape[0])
+    fscale = _on_device(fscale, fd.device)
     L = _lib.lib()
     F, K = fd.shape
     if F * K == 0:
@@ -501,8 +565,9 @@ def resynth_device(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, max_en
     synthesis parameters.  ``phase_preserve`` / ``fscale``: see synth_mode(); ``phase_ws``: the
     integrated-phase scratch to (re)use, one float64 per packed point.  ``scanned``: ``ws`` and
     ``phase_ws`` already hold the block start phases and Nyquist flags (dist.py's hand-over), so the
-    scan is left out (pvk_resynth_render)."""
-    phase_preserve, fscale = synth_mode(phase_preserve, fscale)
+    scan is left out (pvk_resynth_render).  A ``fscale`` curve has one ratio per row of ``tid``."""
+    phase_preserve, fscale = synth_mode(phase_preserve, fscale, nframes=tid.shape[0])
+    fscale = _on_device(fscale, tid.device)
     if scanned and (phase_preserve or phase_ws is None):
         raise ValueError("scanned=True needs phase_preserve=False and the phase_ws of the scan")
     L = _lib.lib()
@@ -1222,9 +1287,10 @@ class SinSumBatch(object):
     def synth_device(self, sr, hop, edge=1.0, minframes=3, phase_preserve=True, fscale=1.0):
         """Render all clips in one pvk_resynth: float64 CUDA tensor [nclips, rows_per_clip * hop]; row c
         holds clip c's signal from its sample 0 (then the silence of the guard rows).  ``phase_preserve``
-        / ``fscale`` as in SinSum.synth (one phase scan over the flattened table, a segment per partial)."""
+        / ``fscale`` as in SinSum.synth (one phase scan over the flattened table, a segment per partial);
+        a curve is ``[nclips, nframes]``, one ratio per clip and frame."""
         pb = self._pb
-        phase_preserve, fscale = synth_mode(phase_preserve, fscale)
+        phase_preserve, fscale = self._batch_mode(phase_preserve, fscale)
         if int(hop) != hop:
             raise TypeError("hop must be an integer number of samples")
         if edge > pb.max_edge:
@@ -1238,6 +1304,23 @@ class SinSumBatch(object):
         out = resynth_device(tr["tid"], pk, sr, hop, self.nfft, self.hop, edge=edge, minframes=minframes, nout=nout,
                              phase_preserve=phase_preserve, fscale=fscale)
         return out.view(pb.nclips, pb.rows_per_clip * hop)
+
+    def _batch_mode(self, phase_preserve, fscale):
+        """synth_mode() for a batch: a ``[nclips, nframes]`` curve becomes one ratio per row of the
+        flattened table (the guard rows, where no partial lives, at 1) on the device."""
+        pb = self._pb
+        if not isinstance(fscale, (np.ndarray, torch.Tensor, list, tuple)):
+            return synth_mode(phase_preserve, fscale)
+        r = _curve_values(fscale)
+        if r.shape != (pb.nclips, pb.nframes):
+            raise ValueError("a batch fscale curve must be [nclips, nframes] = [%d, %d], not of shape %s"
+                             % (pb.nclips, pb.nframes, r.shape))
+        if phase_preserve:
+            raise ValueError("an fscale curve needs phase_preserve=False: the analysed phases cannot be honoured "
+                             "at a scaled frequency")
+        rows = np.ones((pb.nclips, pb.rows_per_clip))
+        rows[:, :pb.nframes] = r
+        return False, _DeviceCurve(torch.from_numpy(rows.reshape(-1)).to(pb._dev))
 
     def clip_lengths(self, hop, edge=1.0):
         """Length of every clip's resynthesis, (max(end) + 2) * hop + edgsamp (PVAnalysis.py:1055-1059,
@@ -1575,12 +1658,21 @@ class SinSum(object):
         is the running sum of its (interpolated) frequency times ``fscale``, so ``fscale`` shifts the
         pitch and a ``hop`` other than the analysis hop stretches time (``synth(sr, round(hop_an * r),
         phase_preserve=False)``); partials with ``fscale * max(f) >= sr / 2`` are left out.
+        ``fscale`` may also be a curve of one ratio per analysis frame, ``r[b]`` applying in output
+        block ``b`` (glides, vibrato, intonation), e.g. ``r = ratio_of(np.arange(nframes) * hop_an /
+        sr)`` with the input time of each frame row; a partial is then left out when any of its points
+        has ``r[row] * f >= sr / 2`` (see synth_mode()).
         ``to_host=False`` returns the CUDA tensor instead of a numpy array.  ``hostbuf`` (a dict,
         reused across calls): render in ``chunks`` block ranges and download each finished range
         into the pinned tensor ``hostbuf['w']`` while the next one is rendered; returns a numpy view
         of it (valid until the next call with the same ``hostbuf``)."""
-        phase_preserve, fscale = synth_mode(phase_preserve, fscale)
-        mode = dict(phase_preserve=phase_preserve, fscale=fscale)
+        nframes = None
+        if isinstance(fscale, (np.ndarray, torch.Tensor, list, tuple)):
+            if self._trk is None:
+                self._ensure_tables()
+            nframes = int((self._trk["tid"] if self._trk is not None else self._tables["f"]).shape[0])
+        phase_preserve, fscale = synth_mode(phase_preserve, fscale, nframes)
+        mode = dict(phase_preserve=phase_preserve, fscale=_on_device(fscale, self._dev))
         if int(hop) != hop:
             raise TypeError("hop must be an integer number of samples")
         if self._trk is None and hostbuf is not None:

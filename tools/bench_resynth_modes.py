@@ -8,6 +8,8 @@ nfft 2048 / hop 512 / npks 50 and tracked once; then, alternating in every round
   free          phase_preserve=False, fscale 1
   free_shift    phase_preserve=False, fscale 2^(7/12)      (partials scaled to >= sr/2 are left out)
   free_stretch  phase_preserve=False, synthesis hop 1024   (2x time stretch)
+  free_curve    phase_preserve=False, a per-frame fscale curve: +-1 semitone vibrato at 5 Hz
+                (uploaded once before the timed passes; the upload is not part of the stage)
 
 The phase scan alone (its three kernels) is timed from a torch.profiler capture of its own.  A
 second leg does the same at the cfg4 length (one 8-hour signal, nfft 2048 / hop 256 / npks 100),
@@ -63,14 +65,25 @@ def tracked(c, dev):
     return tr, pk
 
 
+def vibrato_curve(F, hop_an, sr, rate=5.0, semitones=1.0):
+    """One ratio per frame row from its input time row * hop_an / sr."""
+    t = np.arange(F) * hop_an / float(sr)
+    return 2.0 ** (semitones * np.sin(2 * np.pi * rate * t) / 12.0)
+
+
 def partial_samples(pk, hop, nfft, hop_an, sr, fscale=None, edge=1.0, minframes=3):
-    """Work units: sum over rendered partials of hop * nfr + 2 * edge samples (fscale: Nyquist rule)."""
+    """Work units: sum over rendered partials of hop * nfr + 2 * edge samples (fscale: Nyquist rule;
+    a numpy curve: each point at the ratio of its row)."""
     tl = pk["tlen"].to(torch.int64)
     keep = tl >= minframes
     if fscale is not None:
         ids = torch.repeat_interleave(torch.arange(tl.numel(), device=tl.device), tl)
+        f = pk["pf"]
+        if isinstance(fscale, np.ndarray):
+            rows = pk["tstart"].to(torch.int64)[ids] + torch.arange(ids.numel(), device=tl.device) - pk["toff"][ids]
+            f, fscale = f * torch.from_numpy(fscale).to(tl.device)[rows], 1.0
         fmax = torch.full((tl.numel(),), -1.0, dtype=torch.float64, device=tl.device)
-        fmax.scatter_reduce_(0, ids, pk["pf"], reduce="amax")
+        fmax.scatter_reduce_(0, ids, f, reduce="amax")
         keep &= fscale * fmax < 0.5 * sr
     E = int(nfft / hop_an / 2. * hop * edge)
     return int((tl[keep] * hop + 2 * E).sum().item())
@@ -84,7 +97,9 @@ def run_leg(c, dev, rounds, label):
     tid, max_end = tr["tid"], tr["max_end"]
     F, K = tid.shape
     modes = [("preserve", hop_an, True, 1.0), ("free", hop_an, False, 1.0),
-             ("free_shift", hop_an, False, 2 ** (7 / 12.)), ("free_stretch", 2 * hop_an, False, 1.0)]
+             ("free_shift", hop_an, False, 2 ** (7 / 12.)), ("free_stretch", 2 * hop_an, False, 1.0),
+             ("free_curve", hop_an, False, vibrato_curve(F, hop_an, sr))]
+    dcurve = P._on_device(modes[-1][3], dev)
     bufs = {}
     for name, hop, pp, fs in modes:
         nout, _ = P.synth_geometry(max_end, hop, nfft, hop_an)
@@ -97,7 +112,7 @@ def run_leg(c, dev, rounds, label):
     def render(name, hop, pp, fs):
         b = bufs[name]
         P.resynth_device(tid, pk, sr, hop, nfft, hop_an, max_end=max_end, out=b["out"], ws=b["ws"],
-                         phase_preserve=pp, fscale=fs, phase_ws=b["pws"])
+                         phase_preserve=pp, fscale=dcurve if name == "free_curve" else fs, phase_ws=b["pws"])
 
     for m in modes:                                          # warm-up: module load, every shape once
         render(*m)
@@ -135,7 +150,8 @@ def run_leg(c, dev, rounds, label):
     for name, hop, pp, fs in modes:
         t = np.array(times[name])
         ps = partial_samples(pk, hop, nfft, hop_an, sr, None if pp else fs)
-        res["modes"][name] = dict(hop=hop, phase_preserve=pp, fscale=fs, median_ms=round(float(np.median(t)), 4),
+        fs_doc = "vibrato +-1 semitone, 5 Hz, per frame" if isinstance(fs, np.ndarray) else fs
+        res["modes"][name] = dict(hop=hop, phase_preserve=pp, fscale=fs_doc, median_ms=round(float(np.median(t)), 4),
                                   min_ms=round(float(t.min()), 4), max_ms=round(float(t.max()), 4),
                                   partial_samples=ps, partial_samples_per_s=float("%.4g" % (ps / (np.median(t) * 1e-3))))
     base = res["modes"]["preserve"]["median_ms"]
@@ -143,8 +159,9 @@ def run_leg(c, dev, rounds, label):
         res["modes"][name]["vs_preserve"] = round(res["modes"][name]["median_ms"] / base, 3)
     res["scan_only_ms"] = round(scan_us / 1e3, 4)
     res["scan_share_of_free"] = round(scan_us / 1e3 / res["modes"]["free"]["median_ms"], 3)
+    res["free_curve_vs_free"] = round(res["modes"]["free_curve"]["median_ms"] / res["modes"]["free"]["median_ms"], 3)
     res["profiled_kernels_us_per_pass"] = kern
-    del bufs, flush, tr, pk
+    del bufs, flush, tr, pk, dcurve
     torch.cuda.empty_cache()
     return res
 

@@ -15,6 +15,8 @@ a device synchronise, max over the ranks:
   free          phase_preserve=False, fscale 1
   free_shift    phase_preserve=False, fscale 2^(7/12)
   free_stretch  phase_preserve=False, synthesis hop 2x the analysis hop
+  free_curve    phase_preserve=False, a per-frame fscale curve over the global frames: +-1 semitone
+                vibrato at 5 Hz (checked and uploaded inside the timed call, as a user's call does)
 
 ``handover`` times dist.integrated_phase_local alone (scan + records + all_gather + seed / fix-up +
 flags + all_reduce + import) at fscale 2^(7/12).
@@ -37,7 +39,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tools"))
 
 from pypevoc_b200 import dist as D, pv as P, signals  # noqa: E402
-from bench_resynth_modes import card  # noqa: E402
+from bench_resynth_modes import card, vibrato_curve  # noqa: E402
 
 METRIC = dict(sr=44100, seconds=600, nfft=2048, hop=512, npks=50, f0=220.0, nharm=90, p=0.5, sigma=0.01, seed=1)
 CFG4 = dict(sr=44100, seconds=3600, nfft=2048, hop=256, npks=100, f0=200.0, nharm=100, p=0.4, sigma=0.01, seed=4000)
@@ -79,7 +81,9 @@ def timed(fn, world, flush):
 def run(c, rank, world, dev, group, rounds, flush):
     ss = sharded_sinsum(c, rank, world, dev, group)
     hop = c["hop"]
-    res = {m: [] for m, _, _ in MODES}
+    curve = vibrato_curve(ss._spv.plans[0]["frames_total"], hop, c["sr"])
+    modes = MODES + [("free_curve", 1, dict(phase_preserve=False, fscale=curve))]
+    res = {m: [] for m, _, _ in modes}
     res["handover"] = []
 
     def handover():
@@ -92,7 +96,7 @@ def run(c, rank, world, dev, group, rounds, flush):
                                  ss.device_track_table, ss.ntracks, c["sr"], hop, c["nfft"], hop, 2 ** (7 / 12.), ws, pws,
                                  group=group)
     for r in range(rounds + 1):                                    # round 0: warm-up
-        for name, hm, kw in MODES:
+        for name, hm, kw in modes:
             ms = timed(lambda: ss.synth_local(hop=hm * hop, **kw), world, flush)
             if r:
                 res[name].append(ms)
