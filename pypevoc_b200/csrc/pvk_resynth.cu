@@ -479,8 +479,9 @@ __global__ void __launch_bounds__(128) resynth_prepare_kernel(RParams p, int64_t
 // Inner loops shared by the two render kernels.  A thread owns RS consecutive samples qs..qs+RS
 // of block b and adds the staged partial bodies items[c], c = g, g+G, ... < nbody, to acc[].
 // Fast path (no knot inside the chunk -- practically always): the phase polynomial is evaluated
-// once in fp64 at the chunk centre, reduced to [-0.5, 0.5] cycles and advanced over the RS samples
-// as an fp32 quadratic in radians (|increment| < RS/2 * pi); one MUFU cosine + 5 FMA-pipe
+// once in fp64 at the chunk centre, reduced to an angle in [0, 2 pi) (frac_angle) and advanced over
+// the RS samples as an fp32 quadratic in radians (|increment| < RS/2 * pi, so the MUFU cosine sees
+// arguments in (-RS/2 * pi, 2 pi + RS/2 * pi), about +-30 rad at RS = 16); one MUFU cosine + 5 FMA-pipe
 // instructions per partial-sample.  Slow path (knot inside the chunk): fp64 phase per sample.
 template <int RS>
 __device__ __forceinline__ void render_bodies(const RParams &p, const BodyItem *items, int nbody, int g, int G,
