@@ -7,8 +7,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# PVK_LIB: load an experimental build variant of the same library (tuning runs only)
-LIB_PATH = os.environ.get("PVK_LIB") or os.path.join(_HERE, "libpvk.so")
+LIB_PATH = os.path.join(_HERE, "libpvk.so")
 
 _p = C.c_void_p
 _i64 = C.c_int64

@@ -29,18 +29,10 @@ def needs_build():
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force=False, verbose=False, defines=(), out=None):
-    """defines / out: build an experimental variant (e.g. defines=("PVK_TSHIFT=1",)) elsewhere."""
-    if out is None:
-        out = OUT
-        if not force and not needs_build():
-            return OUT
-    return _build(verbose, defines, out)
-
-
-def _build(verbose, defines, OUT):
+def build(force=False, verbose=False):
+    if not force and not needs_build():
+        return OUT
     cmd = [_nvcc()] + NVCC_FLAGS + ["-I", os.path.join(ROOT, "include"), "-I", CSRC]
-    cmd += ["-D" + d for d in defines]
     if verbose:
         cmd += ["-Xptxas", "-v"]
     cmd += [os.path.join(CSRC, s) for s in SOURCES] + ["-o", OUT]
@@ -54,6 +46,4 @@ def _build(verbose, defines, OUT):
 
 
 if __name__ == "__main__":
-    defs = [a[2:] for a in sys.argv[1:] if a.startswith("-D")]
-    outs = [a[3:] for a in sys.argv[1:] if a.startswith("-o=")]
-    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv, defines=defs, out=outs[0] if outs else None))
+    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))

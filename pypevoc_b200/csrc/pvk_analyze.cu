@@ -47,29 +47,10 @@ struct AParams {
   double *fine_pos, *fine_val;   // optional PeakFinder.refine outputs (PeakFinder.py:331-372)
 };
 
-// tuning knobs (compile time): PVK_TSHIFT = log2 of extra threads per frame for nfft >= 1024,
-// PVK_TWREG = 1 keeps the inter-pass twiddles of a thread in registers across the frame loop
-#ifndef PVK_TSHIFT
-#define PVK_TSHIFT 0
-#endif
-#ifndef PVK_TWREG
-#define PVK_TWREG 0
-#endif
-// PVK_CKEY = 1 keeps a compact copy of the candidate keys in shared memory; 0 (default) looks
-// the key up in |fx|^2 through the candidate's bin (4 KB less shared memory at nfft 2048: one
-// more resident CTA per SM)
-#ifndef PVK_CKEY
-#define PVK_CKEY 0
-#endif
-// PVK_MINB(T): minimum resident CTAs per SM the analysis kernel is compiled for (register budget)
-#ifndef PVK_MINB
-#define PVK_MINB(T) (512 / (T))
-#endif
-
 template <int LOGM> struct Plan {
   static constexpr int M = 1 << LOGM;
   // (at most 512 threads = 16 warps per CTA: the per-warp reduction slots of Smem are sized for that)
-  static constexpr int LOGT = LOGM <= 8 ? 5 : (LOGM <= 9 ? 6 : (LOGM <= 10 ? 6 : LOGM - 4) + PVK_TSHIFT);
+  static constexpr int LOGT = LOGM <= 8 ? 5 : (LOGM <= 10 ? 6 : LOGM - 4);
   static constexpr int T = 1 << LOGT;
   static constexpr int LP0 = LOGM - LOGT;
   static constexpr int LP = LP0 < 2 ? 2 : (LP0 > 4 ? 4 : LP0);
@@ -82,16 +63,6 @@ template <int LOGM> struct Plan {
     return o;
   }
   static constexpr int TW_TOTAL = tw_off(NPASS);
-  // register-resident twiddles: NB_q * (R_q - 1) per pass q >= 1
-  __host__ __device__ static constexpr int twr_off(int q) {
-    int o = 0;
-    for (int i = 1; i < q; ++i) {
-      const int nbf = M >> lr(i);
-      o += ((nbf + T - 1) / T) * ((1 << lr(i)) - 1);
-    }
-    return o;
-  }
-  static constexpr int TWR_TOTAL = twr_off(NPASS) > 0 ? twr_off(NPASS) : 1;
   static constexpr int MP = M + (M >> 4) + 1;
   static constexpr int NW = T / 32;
 };
@@ -146,42 +117,22 @@ template <int LOGM, int Q> struct Pass {
   static constexpr int M = P::M, T = P::T;
   static constexpr int LR = P::lr(Q), R = 1 << LR, LPQ = P::lp(Q), PP = 1 << LPQ;
   static constexpr int NBF = M >> LR, NB = (NBF + T - 1) / T;
-  static constexpr int OFF = P::tw_off(Q), OFFR = P::twr_off(Q);
+  static constexpr int OFF = P::tw_off(Q);
 
-  // twiddles of this thread for pass Q and all later passes -> treg
-  static __device__ __forceinline__ void load_tw(const float2 *__restrict__ twp, float2 *treg) {
-    const int tid = threadIdx.x;
-#pragma unroll
-    for (int b = 0; b < NB; ++b) {
-      const int i = tid + b * T;
-      if (NBF >= T || i < NBF) {
-        const int k = i & (PP - 1);
-#pragma unroll
-        for (int r = 1; r < R; ++r) treg[OFFR + b * (R - 1) + r - 1] = __ldg(twp + OFF + (r - 1) * PP + k);
-      }
-    }
-    if constexpr (Q + 1 < P::NPASS) Pass<LOGM, Q + 1>::load_tw(twp, treg);
-  }
-
-  static __device__ __forceinline__ void run(const float2 *__restrict__ twp, const float2 *treg, float2 *buf) {
+  static __device__ __forceinline__ void run(const float2 *__restrict__ twp, float2 *buf) {
     const int tid = threadIdx.x;
     float2 u[NB][R];
-#if !PVK_TWREG
     // twiddles first: their loads overlap the shared-memory reads and the barrier
-    float2 tloc[NB * (R - 1) > 0 ? NB * (R - 1) : 1];
+    float2 tw[NB * (R - 1) > 0 ? NB * (R - 1) : 1];
 #pragma unroll
     for (int b = 0; b < NB; ++b) {
       const int i = tid + b * T;
       if (NBF >= T || i < NBF) {
         const int k = i & (PP - 1);
 #pragma unroll
-        for (int r = 1; r < R; ++r) tloc[b * (R - 1) + r - 1] = __ldg(twp + OFF + (r - 1) * PP + k);
+        for (int r = 1; r < R; ++r) tw[b * (R - 1) + r - 1] = __ldg(twp + OFF + (r - 1) * PP + k);
       }
     }
-    const float2 *tw = tloc;
-#else
-    const float2 *tw = treg + OFFR;
-#endif
 #pragma unroll
     for (int b = 0; b < NB; ++b) {
       const int i = tid + b * T;
@@ -205,28 +156,14 @@ template <int LOGM, int Q> struct Pass {
       }
     }
     __syncthreads();
-    if constexpr (Q + 1 < P::NPASS) Pass<LOGM, Q + 1>::run(twp, treg, buf);
+    if constexpr (Q + 1 < P::NPASS) Pass<LOGM, Q + 1>::run(twp, buf);
   }
 };
 
-// Two consecutive signal samples.  Build knob PVK_STREAM (off: it measured neutral on B200,
-// profiles/r2_tune_analyze.txt): load past L1 (ld.global.nc.L1::no_allocate), which keeps the window
-// and twiddle tables in the small L1 left beside 8 x 26 KB of shared memory.  Requesting the samples
-// of row r + 1 one phase early (32 more live registers during the peak picking) was neutral too.
+// Two consecutive signal samples: one 64-bit load when p is 8-byte aligned (al8)
 __device__ __forceinline__ float2 ldg_stream2(const float *p, bool al8) {
-#if defined(PVK_EMU) || !defined(PVK_STREAM)
   if (al8) return __ldg(reinterpret_cast<const float2 *>(p));
   return make_float2(__ldg(p), __ldg(p + 1));
-#else
-  float2 v;
-  if (al8) {
-    asm volatile("ld.global.nc.L1::no_allocate.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "l"(p));
-  } else {
-    asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v.x) : "l"(p));
-    asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v.y) : "l"(p + 1));
-  }
-  return v;
-#endif
 }
 
 // samples of one frame -> registers: thread `tid` gets the packed points z[m] = (x[2m], x[2m+1]),
@@ -251,7 +188,7 @@ __device__ __forceinline__ void frame_load(const float *__restrict__ xf, float2 
 // natural order in buf
 template <int LOGM>
 __device__ __forceinline__ void fft_frame_regs(float2 *u, const float *__restrict__ win,
-                                               const float2 *__restrict__ twp, const float2 *treg, float2 *buf) {
+                                               const float2 *__restrict__ twp, float2 *buf) {
   using P = Plan<LOGM>;
   constexpr int M = P::M, T = P::T;
   constexpr int LR = P::lr(0), R = 1 << LR;
@@ -268,17 +205,15 @@ __device__ __forceinline__ void fft_frame_regs(float2 *u, const float *__restric
     for (int s = 0; s < R; ++s) buf[PADC(i * R + s)] = u[brev<LR>(s)];
   }
   __syncthreads();
-  if constexpr (P::NPASS > 1) Pass<LOGM, 1>::run(twp, treg, buf);
+  if constexpr (P::NPASS > 1) Pass<LOGM, 1>::run(twp, buf);
 }
 
 template <int LOGM>
-__device__ __forceinline__ void fft_frame(const float *__restrict__ xf, bool al8,
-                                          const float *__restrict__ win,
-                                          const float2 *__restrict__ twp, const float2 *treg, float2 *buf) {
-  (void)al8;
+__device__ __forceinline__ void fft_frame(const float *__restrict__ xf, const float *__restrict__ win,
+                                          const float2 *__restrict__ twp, float2 *buf) {
   float2 u[1 << Plan<LOGM>::lr(0)];
   frame_load<LOGM>(xf, u);
-  fft_frame_regs<LOGM>(u, win, twp, treg, buf);
+  fft_frame_regs<LOGM>(u, win, twp, buf);
 }
 
 // ------------------------------------------------------------------ per-peak epilogue
@@ -376,9 +311,6 @@ __device__ __forceinline__ void peak_phase_freq_fast(int k, const float2 *cur, c
   const float qr = fmaf(c.x, p.x, c.y * p.y), qi = fmaf(c.y, p.x, -(c.x * p.y));
   const float qn = fabsf(qr) + fabsf(qi);
   bool ok = qn > 1e-30f && qn < 1e30f;                        // false for NaN / inf / 0 as well
-#ifdef PVK_EPI_EXACT
-  ok = false;
-#endif
   const double PI2 = 6.283185307179586;
   const double fb = __ldg(fbin + k);
   if (ok) {
@@ -444,8 +376,7 @@ template <int LOGM> struct Smem {
   static constexpr int OFF_BUF0 = 0;
   static constexpr int OFF_BUF1 = OFF_BUF0 + P::MP * 8;
   static constexpr int OFF_FAMP = OFF_BUF1 + P::MP * 8;
-  static constexpr int OFF_CKEY = OFF_FAMP + (P::M + P::M / 4 + 4) * 4;   // candidate keys (compact, bin order)
-  static constexpr int OFF_HIST = OFF_CKEY + (PVK_CKEY ? P::M * 4 : 0);
+  static constexpr int OFF_HIST = OFF_FAMP + (P::M + P::M / 4 + 4) * 4;
   static constexpr int OFF_RED = (OFF_HIST + 3 * 128 * 4 + 7) / 8 * 8;   // doubles: one sum per warp (<= 16 warps)
   static constexpr int OFF_REDF = OFF_RED + 16 * 8;                  // floats: 16 min, 16 max
   static constexpr int OFF_REDU = OFF_REDF + 32 * 4;                 // uints: 16 cnt, 16 kmin, 16 kmax
@@ -475,7 +406,7 @@ __device__ __forceinline__ int round_pos(bool flag, int *wsum, int round, int &b
 }
 
 template <int LOGM>
-__global__ void __launch_bounds__(Plan<LOGM>::T, PVK_MINB(Plan<LOGM>::T)) analyze_kernel(AParams prm) {
+__global__ void __launch_bounds__(Plan<LOGM>::T, 512 / Plan<LOGM>::T) analyze_kernel(AParams prm) {
   using P = Plan<LOGM>;
   using S = Smem<LOGM>;
   constexpr int M = P::M, T = P::T, NW = P::NW, N = 2 * M;
@@ -487,15 +418,10 @@ __global__ void __launch_bounds__(Plan<LOGM>::T, PVK_MINB(Plan<LOGM>::T)) analyz
   constexpr int BUF_STRIDE = S::OFF_BUF1 - S::OFF_BUF0;
 #define PVK_BUF(par) reinterpret_cast<float2 *>(smem + S::OFF_BUF0 + (int)(par) * BUF_STRIDE)
   float *famp = reinterpret_cast<float *>(smem + S::OFF_FAMP);
-#if PVK_CKEY
-  unsigned *ckey = reinterpret_cast<unsigned *>(smem + S::OFF_CKEY);
-#define PVK_KEY(e) ckey[e]
-#define PVK_BIN(v) (v)
-#else
-  // candidate list entry = bin | 0x8000 for a candidate that is not a local maximum (key 0)
+  // candidate list entry = bin | 0x8000 for a candidate that is not a local maximum (key 0); the
+  // key is looked up in |fx|^2 through the bin
 #define PVK_KEY(e) ((cbin[e] & 0x8000) ? 0u : __float_as_uint(famp[FA(cbin[e])]))
 #define PVK_BIN(v) ((v) & 0x7fff)
-#endif
   unsigned *hist = reinterpret_cast<unsigned *>(smem + S::OFF_HIST);   // 3 x 128 words (256 16-bit buckets each)
   double *redd = reinterpret_cast<double *>(smem + S::OFF_RED);
   float *redf = reinterpret_cast<float *>(smem + S::OFF_REDF);
@@ -520,11 +446,6 @@ __global__ void __launch_bounds__(Plan<LOGM>::T, PVK_MINB(Plan<LOGM>::T)) analyz
   const double inv_2pidt = 1.0 / (prm.dt * 6.283185307179586), inv_dt = 1.0 / prm.dt;
   const double pi_fstep = 3.141592653589793 / prm.fstep;
 
-  float2 treg[P::TWR_TOTAL];
-#if PVK_TWREG
-  if constexpr (P::NPASS > 1) Pass<LOGM, 1>::load_tw(twp, treg);
-#endif
-
   // ---- the run starts one row early: row r0 - 1 only leaves its spectrum behind (the "previous"
   //      spectrum of row r0) and emits nothing -- same code, one copy of the FFT in the instruction
   //      cache.  Global frame 0 has the all-zero previous spectrum instead (PVAnalysis.py:121).
@@ -542,7 +463,7 @@ __global__ void __launch_bounds__(Plan<LOGM>::T, PVK_MINB(Plan<LOGM>::T)) analyz
     {
       float2 ux[1 << P::lr(0)];
       frame_load<LOGM>(xc + (prm.frame0 + r) * (int64_t)prm.hop, ux);
-      fft_frame_regs<LOGM>(ux, prm.win, twp, treg, cur);
+      fft_frame_regs<LOGM>(ux, prm.win, twp, cur);
     }
 
     // ---- untangle -> fx[0..M), |fx|, min / max / sum of squares
@@ -681,12 +602,7 @@ __global__ void __launch_bounds__(Plan<LOGM>::T, PVK_MINB(Plan<LOGM>::T)) analyz
       for (unsigned rem = cbits; rem;) {
         const int i = __ffs((int)rem) - 1;
         rem &= rem - 1u;
-#if PVK_CKEY
-        cbin[pos] = (unsigned short)(kb0 + i);
-        ckey[pos] = ((pbits >> i) & 1u) ? __float_as_uint(famp[FA(kb0 + i)]) : 0u;
-#else
         cbin[pos] = (unsigned short)((kb0 + i) | (((pbits >> i) & 1u) ? 0 : 0x8000));
-#endif
         ++pos;
       }
     }
@@ -955,7 +871,7 @@ __global__ void __launch_bounds__(Plan<LOGM>::T) harmonic_kernel(HParams prm) {
   constexpr int BUF_STRIDE = S::OFF_BUF1 - S::OFF_BUF0;
   float *famp = reinterpret_cast<float *>(smem + S::OFF_FAMP);
   double *redd = reinterpret_cast<double *>(smem + S::OFF_RED);      // 8 doubles
-  double *redc = reinterpret_cast<double *>(smem + S::OFF_CKEY);     // 8 doubles (candidate area is free here)
+  double *redc = reinterpret_cast<double *>(smem + S::OFF_HIST);     // 8 doubles (histogram area is free here)
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int64_t r0 = (int64_t)blockIdx.x * prm.run;
   const int64_t r1 = (r0 + prm.run < prm.nframes) ? r0 + prm.run : prm.nframes;
@@ -963,10 +879,6 @@ __global__ void __launch_bounds__(Plan<LOGM>::T) harmonic_kernel(HParams prm) {
   const float2 *twr = prm.tables + P::TW_TOTAL;
   const int K = prm.npks;
   const double inv_2pidt = 1.0 / (prm.dt * 6.283185307179586), inv_dt = 1.0 / prm.dt;
-  float2 treg[P::TWR_TOTAL];
-#if PVK_TWREG
-  if constexpr (P::NPASS > 1) Pass<LOGM, 1>::load_tw(twp, treg);
-#endif
   int cb = 0;                                                 // PVK_BUF(cb) = spectrum of the last processed frame
   {
     int64_t p = r0 - 1;
@@ -975,9 +887,7 @@ __global__ void __launch_bounds__(Plan<LOGM>::T) harmonic_kernel(HParams prm) {
     if (p < 0) {
       for (int i = tid; i < P::MP; i += T) pb[i] = make_float2(0.f, 0.f);   // oldfft = zeros (:121)
     } else {
-      const float *xf = prm.x + p * (int64_t)prm.hop;
-      const bool al8 = ((reinterpret_cast<uintptr_t>(xf) & 7) == 0);
-      fft_frame<LOGM>(xf, al8, prm.win, twp, treg, pb);
+      fft_frame<LOGM>(prm.x + p * (int64_t)prm.hop, prm.win, twp, pb);
       double dummy = 0.0;
       untangle_power<LOGM>(pb, famp, twr, false, dummy);
     }
@@ -993,9 +903,7 @@ __global__ void __launch_bounds__(Plan<LOGM>::T) harmonic_kernel(HParams prm) {
     }
     float2 *cur = PVK_BUF(cb ^ 1);
     const float2 *prev = PVK_BUF(cb);
-    const float *xf = prm.x + r * (int64_t)prm.hop;
-    const bool al8 = ((reinterpret_cast<uintptr_t>(xf) & 7) == 0);
-    fft_frame<LOGM>(xf, al8, prm.win, twp, treg, cur);
+    fft_frame<LOGM>(prm.x + r * (int64_t)prm.hop, prm.win, twp, cur);
     double lsum = 0.0;
     untangle_power<LOGM>(cur, famp, twr, true, lsum);
     {
@@ -1135,29 +1043,23 @@ __global__ void __launch_bounds__(Plan<LOGM>::T) bank_kernel(BParams prm) {
   float2 *buf = reinterpret_cast<float2 *>(smem + S::OFF_BUF0);
   float *pws[2] = {reinterpret_cast<float *>(smem + S::OFF_BUF1), reinterpret_cast<float *>(smem + S::OFF_BUF1) + (M + 2)};
   double *redd = reinterpret_cast<double *>(smem + S::OFF_RED);       // 8 doubles
-  double *redf = reinterpret_cast<double *>(smem + S::OFF_CKEY);      // 8 doubles
+  double *redf = reinterpret_cast<double *>(smem + S::OFF_HIST);      // 8 doubles
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int64_t r0 = (int64_t)blockIdx.x * prm.run;
   const int64_t r1 = (r0 + prm.run < prm.nframes) ? r0 + prm.run : prm.nframes;
   const float2 *twp = prm.tables;
   const float2 *twr = prm.tables + P::TW_TOTAL;
-  float2 treg[P::TWR_TOTAL];
-#if PVK_TWREG
-  if constexpr (P::NPASS > 1) Pass<LOGM, 1>::load_tw(twp, treg);
-#endif
   const bool want_flux = prm.flux != nullptr;
   int cb = 0;
   if (want_flux && r0 > 0) {                                  // spectrum of the frame before the run
-    const float *xf = prm.x + (r0 - 1) * (int64_t)prm.hop;
-    fft_frame<LOGM>(xf, (reinterpret_cast<uintptr_t>(xf) & 7) == 0, prm.win, twp, treg, buf);
+    fft_frame<LOGM>(prm.x + (r0 - 1) * (int64_t)prm.hop, prm.win, twp, buf);
     untangle_to_power<LOGM>(buf, pws[cb ^ 1], twr);
     __syncthreads();
   }
   for (int64_t r = r0; r < r1; ++r) {
     float *pw = pws[cb];
     const float *pprev = pws[cb ^ 1];
-    const float *xf = prm.x + r * (int64_t)prm.hop;
-    fft_frame<LOGM>(xf, (reinterpret_cast<uintptr_t>(xf) & 7) == 0, prm.win, twp, treg, buf);
+    fft_frame<LOGM>(prm.x + r * (int64_t)prm.hop, prm.win, twp, buf);
     untangle_to_power<LOGM>(buf, pw, twr);
     __syncthreads();
     if (prm.bank) {                                           // one warp per filter

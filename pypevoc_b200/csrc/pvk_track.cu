@@ -234,7 +234,7 @@ __global__ void track_link_kernel(const double *__restrict__ f, const double *__
   }
 }
 
-// ---- rows of up to 512 peaks: the greedy loop without ranking either row.
+// ---- rows of up to 128 peaks: the greedy loop without ranking either row.
 // The sequential loop (:903-950) hands every current peak, in descending magnitude order, its
 // nearest still-unused previous peak (if within maxpitchjmp).  Only peaks that compete for the same
 // previous peak need to know who comes first, and that is a direct magnitude comparison:
@@ -1051,10 +1051,7 @@ __global__ void resolve_fix_kernel(int32_t *__restrict__ T, int64_t n, int K, co
 // Every thread walks one column over a strip of PACK_STRIP consecutive frames and merges runs of
 // equal ids (a partial usually stays in its column for a while) before touching the per-track
 // counters: ~PACK_STRIP x fewer atomics than one per point.
-#ifndef PVK_PACK_STRIP
-#define PVK_PACK_STRIP 64
-#endif
-constexpr int PACK_STRIP = PVK_PACK_STRIP;
+constexpr int PACK_STRIP = 64;
 // Ids >= ntracks (the capacity of tstart / tlen: a speculative pack is sized by an upper bound
 // before the real count is known, pv.track_pack_device) are skipped, never written.
 __global__ void pack_count_kernel(const int32_t *__restrict__ tid, int64_t F, int K, int64_t ntracks,
@@ -1234,25 +1231,11 @@ extern "C" int pvk_track(const double *f, const double *mag, int64_t nclips, int
 
   {  // link: one warp per frame pair
     int64_t g;
-    // rows of `wide_from` or more peaks take the sequential loop kernel (PVK_LINK_GENERIC_FROM: test override)
-    static const int wide_from = []() { const char *e = getenv("PVK_LINK_GENERIC_FROM"); return e ? atoi(e) : 513; }();
-    static const int cta_from = []() { const char *e = getenv("PVK_LINK_CTA_FROM"); return e ? atoi(e) : 129; }();
-    if (K <= 512 && K < wide_from && K >= cta_from) {
-      // one CTA per row: 128 threads up to 256 columns, 256 threads up to 512
-      const int T = K <= 256 ? 128 : 256;
-      const int smem = link_cta_smem(2 * T);
-      if (smem > 48 * 1024 && PVK_SET_SMEM(track_link_cta_kernel, smem) != 0) {
-        set_error("pvk_track: cannot reserve %d bytes of shared memory", smem);
-        return PVK_ERR_CUDA;
-      }
-      g = rows < 148 * 16 ? rows : 148 * 16;
-      PVK_LAUNCH(track_link_cta_kernel, dim3((unsigned)g), dim3(T), smem, stream, f, mag, rows, nframes, K, maxpitchjmp,
-                 link, newcount);
-    } else if (K <= 512 && K < wide_from) {
-      const int S = K <= 32 ? 1 : (K <= 64 ? 2 : (K <= 128 ? 4 : (K <= 256 ? 8 : 16)));
-      const int per_warp = link_claim_smem_per_warp(S);
-      const int W = S <= 4 ? 8 : (S == 8 ? 4 : 2);
-      const int smem = W * per_warp;
+    // up to 128 peaks: one warp per row; up to 512: one CTA per row; wider rows: the sequential loop kernel
+    if (K <= 128) {
+      const int S = K <= 32 ? 1 : (K <= 64 ? 2 : 4);
+      const int W = 8;
+      const int smem = W * link_claim_smem_per_warp(S);
       g = (rows + W - 1) / W;
       if (g > 148 * 64) g = 148 * 64;
 #define PVK_LINK_CLAIM(SS)                                                                         \
@@ -1266,10 +1249,19 @@ extern "C" int pvk_track(const double *f, const double *mag, int64_t nclips, int
       } while (0)
       if (S == 1) PVK_LINK_CLAIM(1);
       else if (S == 2) PVK_LINK_CLAIM(2);
-      else if (S == 4) PVK_LINK_CLAIM(4);
-      else if (S == 8) PVK_LINK_CLAIM(8);
-      else PVK_LINK_CLAIM(16);
+      else PVK_LINK_CLAIM(4);
 #undef PVK_LINK_CLAIM
+    } else if (K <= 512) {
+      // one CTA per row: 128 threads up to 256 columns, 256 threads up to 512
+      const int T = K <= 256 ? 128 : 256;
+      const int smem = link_cta_smem(2 * T);
+      if (smem > 48 * 1024 && PVK_SET_SMEM(track_link_cta_kernel, smem) != 0) {
+        set_error("pvk_track: cannot reserve %d bytes of shared memory", smem);
+        return PVK_ERR_CUDA;
+      }
+      g = rows < 148 * 16 ? rows : 148 * 16;
+      PVK_LAUNCH(track_link_cta_kernel, dim3((unsigned)g), dim3(T), smem, stream, f, mag, rows, nframes, K, maxpitchjmp,
+                 link, newcount);
     } else {
       const int per_warp = link_generic_smem_per_warp(K);
       int W = 96 * 1024 / per_warp;                               // two CTAs per SM

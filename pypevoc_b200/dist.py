@@ -301,8 +301,7 @@ def _stitch_stream(dev):
     if key not in _STITCH_STREAMS:
         # high priority: its kernels are tiny (summary, resolve, rename + stores, barriers, the collective's
         # copy CTAs) and must not queue behind the thousands of CTAs of the rendering kernel they overlap
-        prio = -1 if os.environ.get("PVK_STITCH_PRIORITY", "1") != "0" else 0
-        _STITCH_STREAMS[key] = torch.cuda.Stream(device=dev, priority=prio)
+        _STITCH_STREAMS[key] = torch.cuda.Stream(device=dev, priority=-1)
     return _STITCH_STREAMS[key]
 
 

@@ -7,9 +7,6 @@ STEPS=${3:-5}
 OUT=gpurun_out
 mkdir -p $OUT
 python -W ignore -m pytest tests -x -q -m gpu 2>&1 | tail -8 | tee $OUT/pytest_gpu_$TAG.log
-if ls pypevoc_b200/libpvk_*.so > /dev/null 2>&1; then
-PVK_CASES=metric_10min,cfg2_10min python tools/tune_analyze.py pypevoc_b200/libpvk.so pypevoc_b200/libpvk_*.so 2>&1 | tee $OUT/tune_$TAG.txt
-fi
 python bench.py --steps $STEPS --warmup 3 --no-cpu > $OUT/bench_${TAG}_g1.json 2> $OUT/bench_${TAG}_g1.err
 tail -c 1500 $OUT/bench_${TAG}_g1.json; tail -3 $OUT/bench_${TAG}_g1.err
 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29531 \
