@@ -451,6 +451,27 @@ int pvk_nyquist_flags_curve(const double *f, const int32_t *gid, int64_t n, doub
                             const double *fcurve, int64_t fcurve_len, int npks, uint8_t *flags, int64_t nflags,
                             void *stream);
 
+/* ------------------------------------------------------------------ formant gains
+ * The magnitudes of a formant-preserving / formant-shifting resynthesis (DESIGN.md 4.3), to be passed as
+ * pmag to pvk_resynth_ex / pvk_resynth_render (and their _curve variants).  The envelope of frame row j is
+ * the piecewise-linear interpolation L_j of ln(pmag) over the frequencies of the row's points (slots with
+ * 0 <= tid < ntracks; knots sorted by frequency, ties by column; held constant beyond the first / last
+ * knot, as np.interp).  Every point (f, m) of row j is written as pmag_out[toff[v] + j - tstart[v]] =
+ * m * exp(L_j(f * q_j) - L_j(f)), and = m bit for bit where f * q_j == f.  q_j = fscale_j / formant_j, the
+ * render's frequency ratio of the row over its formant factor.
+ *   tid, ntracks, ntracks_dev, tstart, toff, pf, pmag   as pvk_resynth_ex takes them (ntracks_dev != NULL:
+ *                the partial count is read on the device, at most ntracks)
+ *   q            the ratio of every row when qcurve = NULL (finite, > 0)
+ *   qcurve       device, one ratio per frame row (qcurve_len >= nframes; values the caller's to check)
+ *   pmag_out     one double per packed point; a length below min(ntracks, nframes * npks) is rejected,
+ *                points at or beyond pmag_out_len are not written
+ * Checks its arguments before any CUDA call; allocates nothing.
+ */
+int pvk_formant_gains(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *ntracks_dev,
+                      const int32_t *tstart, const int64_t *toff, const double *pf, const double *pmag, double q,
+                      const double *qcurve, int64_t qcurve_len, double *pmag_out, int64_t pmag_out_len,
+                      void *stream);
+
 #ifdef __cplusplus
 }
 #endif

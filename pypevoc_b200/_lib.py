@@ -65,6 +65,7 @@ SIGNATURES = {
     "pvk_resynth_scan_curve": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _d, _i, _i, _i, _d, _p, _i64, _p, _i64, _p,
                                     _i64, _i64, _i64, _p, _i64, _p]),
     "pvk_nyquist_flags_curve": (_i, [_p, _p, _i64, _d, _d, _p, _i64, _i, _p, _i64, _p]),
+    "pvk_formant_gains": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _d, _p, _i64, _p, _i64, _p]),
 }
 
 

@@ -1321,3 +1321,134 @@ extern "C" int pvk_resynth_import_flags(const int32_t *tid, int64_t nframes, int
   PVK_CHECK_LAUNCH("pvk_resynth_import_flags");
   return PVK_OK;
 }
+
+// ------------------------------------------------------------------ formant gains (DESIGN.md 4.3)
+// The spectral envelope of frame row j is L_j, the piecewise-linear interpolation of ln(pmag) over the
+// frequencies of the row's points (as np.interp: clamped at both ends; knots sorted by frequency, ties
+// by column).  Point (f, m) of row j gets m' = m * exp(L_j(f * q_j) - L_j(f)), and m' = m when
+// f * q_j == f.  One CTA per row, blockDim = K rounded up to a warp (at most FORMANT_THREADS), so a row
+// of up to 32 peaks is one warp: keys in column order, a sortedness check (analysed rows are ascending),
+// a bitonic sort of (frequency, column) in shared memory otherwise, one ln per knot, one exp per point.
+namespace pvk {
+
+constexpr int FORMANT_THREADS = 256;
+
+// L(x) over the sorted knots xs[0..n), ys[0..n), n >= 1, evaluated as np.interp does
+__device__ __forceinline__ double formant_env(const double *xs, const double *ys, int n, double x) {
+  if (x < xs[0]) return ys[0];
+  if (x >= xs[n - 1]) return ys[n - 1];
+  int lo = 0, hi = n - 1;                                         // xs[lo] <= x < xs[hi]
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (xs[mid] <= x) lo = mid; else hi = mid;
+  }
+  if (xs[lo] == x) return ys[lo];                                 // lo: the last of equal knots
+  const double slope = (ys[hi] - ys[lo]) / (xs[hi] - xs[lo]);
+  return slope * (x - xs[lo]) + ys[lo];
+}
+
+// P: power of two >= K.  Shared memory: key [P], ln(pmag) of the sorted knots [P] (doubles), packed
+// point of every column [K] (int64), column of every key [P], knot count (ints)
+static int64_t formant_smem(int K, int P) { return (int64_t)P * 16 + (int64_t)K * 8 + (int64_t)P * 4 + 16; }
+
+__global__ void __launch_bounds__(FORMANT_THREADS) formant_gain_kernel(
+    const int32_t *__restrict__ tid, int64_t F, int K, int P, int64_t ntracks, const int32_t *__restrict__ ntracks_dev,
+    const int32_t *__restrict__ tstart, const int64_t *__restrict__ toff, const double *__restrict__ pf,
+    const double *__restrict__ pmag, double q, const double *__restrict__ qcurve, double *__restrict__ pmag_out,
+    int64_t pmag_out_len) {
+  PVK_SMEM(smem);
+  double *key = reinterpret_cast<double *>(smem);
+  double *ly = key + P;
+  int64_t *pt = reinterpret_cast<int64_t *>(ly + P);
+  int *col = reinterpret_cast<int *>(pt + K);
+  int *s_nk = col + P;
+  const int t = threadIdx.x, T = blockDim.x;
+  if (ntracks_dev != nullptr) { const int64_t m = *ntracks_dev; ntracks = m < ntracks ? m : ntracks; }
+  for (int64_t row = blockIdx.x; row < F; row += gridDim.x) {
+    // keys in column order: the frequency of a point, +inf for a slot without one (sorts behind every knot)
+    for (int c = t; c < P; c += T) {
+      double k = INFINITY;
+      if (c < K) {
+        const int v = tid[row * K + c];
+        int64_t i = -1;
+        if (v >= 0 && v < ntracks) {
+          i = toff[v] + (row - tstart[v]);
+          k = pf[i];
+        }
+        pt[c] = i;
+      }
+      key[c] = k;
+      col[c] = c;
+    }
+    __syncthreads();
+    int down = 0;
+    for (int c = t; c + 1 < P; c += T) down |= key[c] > key[c + 1] ? 1 : 0;
+    if (__syncthreads_count(down) != 0) {
+      // bitonic sort of (key, column), a total order: the result does not depend on T
+      for (int k2 = 2; k2 <= P; k2 <<= 1) {
+        for (int j = k2 >> 1; j > 0; j >>= 1) {
+          for (int i = t; i < P; i += T) {
+            const int ix = i ^ j;
+            if (ix > i) {
+              const double a = key[i], b = key[ix];
+              const bool gt = a > b || (a == b && col[i] > col[ix]);
+              if (gt == ((i & k2) == 0)) {
+                key[i] = b; key[ix] = a;
+                const int ci = col[i]; col[i] = col[ix]; col[ix] = ci;
+              }
+            }
+          }
+          __syncthreads();
+        }
+      }
+    }
+    // knot count: the keys below +inf lead
+    for (int c = t; c < P; c += T) {
+      const bool in = key[c] < INFINITY;
+      if (c == 0 && !in) *s_nk = 0;
+      if (in && (c + 1 == P || !(key[c + 1] < INFINITY))) *s_nk = c + 1;
+    }
+    __syncthreads();
+    const int nk = *s_nk;
+    for (int r = t; r < nk; r += T) ly[r] = log(pmag[pt[col[r]]]);
+    __syncthreads();
+    const double qr = qcurve != nullptr ? qcurve[row] : q;
+    for (int c = t; c < K; c += T) {
+      const int64_t i = pt[c];
+      if (i < 0 || i >= pmag_out_len) continue;
+      const double f = pf[i], m = pmag[i], x = f * qr;
+      pmag_out[i] = x == f ? m : m * exp(formant_env(key, ly, nk, x) - formant_env(key, ly, nk, f));
+    }
+    __syncthreads();                                              // shared memory is the next row's
+  }
+}
+
+}  // namespace pvk
+
+extern "C" int pvk_formant_gains(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks,
+                                 const int32_t *ntracks_dev, const int32_t *tstart, const int64_t *toff,
+                                 const double *pf, const double *pmag, double q, const double *qcurve,
+                                 int64_t qcurve_len, double *pmag_out, int64_t pmag_out_len, void *stream) {
+  PVK_REQUIRE(npks >= 1 && npks <= PVK_MAX_NPKS, "pvk_formant_gains: npks=%d must be in [1, %d]", npks, PVK_MAX_NPKS);
+  PVK_REQUIRE(nframes >= 0 && ntracks >= 0, "pvk_formant_gains: negative sizes");
+  if (qcurve == nullptr)
+    PVK_REQUIRE(isfinite(q) && q > 0.0, "pvk_formant_gains: q=%g must be finite and > 0", q);
+  else
+    PVK_REQUIRE(qcurve_len >= nframes, "pvk_formant_gains: qcurve_len=%lld is short (one ratio per frame row, %lld rows)",
+                (long long)qcurve_len, (long long)nframes);
+  const int64_t need = ntracks < nframes * (int64_t)npks ? ntracks : nframes * (int64_t)npks;
+  PVK_REQUIRE(pmag_out_len >= need,
+              "pvk_formant_gains: pmag_out_len=%lld is short (one double per packed point, at least %lld)",
+              (long long)pmag_out_len, (long long)need);
+  if (nframes == 0 || ntracks == 0) return PVK_OK;
+  PVK_REQUIRE(tid && tstart && toff && pf && pmag && pmag_out, "pvk_formant_gains: NULL pointer argument");
+  int P = 1;
+  while (P < npks) P <<= 1;
+  const int T = ((npks + 31) / 32) * 32 < FORMANT_THREADS ? ((npks + 31) / 32) * 32 : FORMANT_THREADS;
+  const int64_t smem = formant_smem(npks, P);
+  int64_t g = nframes < 148 * 32 ? nframes : 148 * 32;
+  PVK_LAUNCH(formant_gain_kernel, dim3((unsigned)g), dim3(T), (int)smem, stream, tid, nframes, npks, P, ntracks,
+             ntracks_dev, tstart, toff, pf, pmag, q, qcurve, pmag_out, pmag_out_len);
+  PVK_CHECK_LAUNCH("pvk_formant_gains");
+  return PVK_OK;
+}

@@ -571,20 +571,22 @@ def resynth_local(tid_local, pk_local, plan, plans, max_end, sr, hop, nfft, hop_
 
 
 def track_pack_resynth_local(tab, plan, plans, sr, hop, nfft, hop_an, edge=1.0, minframes=3, maxpitchjmp=0.5,
-                             after_link=None, after_pack=None, before_sync=None):
+                             after_link=None, after_pack=None, before_sync=None, formant=None):
     """Back half of the path for one rank's window, queued without a host round trip
     (pv.track_pack_resynth_device): link, pack and the rendering of the rank's block range.  No count
     is needed to know the range: every rank but the one owning the last frames renders its own blocks
     [j0, j1); the last one renders up to the bound its window allows (its last window row as "last
     frame") -- cut with trim_local() once the global last frame is known.  ``tab``: device tables f mag
-    ph realph [window rows, K].  Returns (tr, pk, w, b0): w holds global samples [b0*hop, ...)."""
+    ph realph [window rows, K].  ``formant``: the formant ratio q of the window rows (pv.formant_ratio(),
+    float or pv._DeviceCurve).  Returns (tr, pk, w, b0): w holds global samples [b0*hop, ...)."""
     w1 = plan["w1"]
     b0, b1, bound = render_range_local(plan, plans, (w1 - 1) if plan["nown"] > 0 else -1, hop, nfft, hop_an, edge)
     w0 = plan["w0"]
     rng = (b0 - w0, max(b1 - b0, 0), max(bound - w0 * hop, 0))
     tr, pk, w = P.track_pack_resynth_device(tab["f"], tab["mag"], tab["ph"], tab["realph"], sr, hop, nfft, hop_an, edge=edge,
                                             minframes=minframes, maxpitchjmp=maxpitchjmp, after_link=after_link,
-                                            after_pack=after_pack, block_range=rng, before_sync=before_sync)
+                                            after_pack=after_pack, block_range=rng, before_sync=before_sync,
+                                            formant=formant)
     if w is None:
         w = torch.zeros((0,), dtype=torch.float64, device=tab["f"].device)
     return tr, pk, w, b0
@@ -793,7 +795,7 @@ class ShardedSinSum(object):
         return ss
 
     def synth_local(self, sr=None, hop=None, edge=1.0, minframes=3, hostbuf=None, chunks=8, to_host=False,
-                    phase_preserve=True, fscale=1.0):
+                    phase_preserve=True, fscale=1.0, formant_shift=None):
         """Render this rank's own block range of the resynthesised signal (the last rank also renders
         the tail): global samples [b0*hop, ...).  Returns (signal, first global sample).  ``hostbuf``:
         render in ``chunks`` ranges and download each into pinned ``hostbuf['w']`` meanwhile.
@@ -803,11 +805,18 @@ class ShardedSinSum(object):
         ntracks bytes), so the concatenated own signals equal the unsharded render bit for bit.
         COLLECTIVE in that mode: every rank makes the same call.  ``fscale`` may be a curve over the
         GLOBAL frames, ``[frames_total]`` (see pv.synth_mode()); each rank uses its window's rows.  It is
-        checked on every rank before anything is launched."""
+        checked on every rank before anything is launched.  ``formant_shift`` as in SinSum.synth (a curve over
+        the global frames, too): a row's formant gains depend on that row's points only, all of which are
+        in the window, so this needs no collective of its own."""
         spv = self._spv
-        phase_preserve, fscale = P.synth_mode(phase_preserve, fscale, nframes=spv.plans[0]["frames_total"])
+        nf = spv.plans[0]["frames_total"]
+        phase_preserve, fscale = P.synth_mode(phase_preserve, fscale, nframes=nf)
+        formant = P.formant_ratio(phase_preserve, fscale, formant_shift, nframes=nf)
+        win = slice(spv.plan["w0"], spv.plan["w1"])
         if isinstance(fscale, np.ndarray):
-            fscale = P._on_device(np.ascontiguousarray(fscale[spv.plan["w0"]:spv.plan["w1"]]), spv.pv._dev)
+            fscale = P._on_device(np.ascontiguousarray(fscale[win]), spv.pv._dev)
+        if isinstance(formant, np.ndarray):
+            formant = P._on_device(np.ascontiguousarray(formant[win]), spv.pv._dev)
         sr = spv.sr if sr is None else sr
         hop = spv.hop if hop is None else int(hop)
         if (edge, minframes) != (spv.edge, spv.minframes):
@@ -819,7 +828,8 @@ class ShardedSinSum(object):
             t = self.local._tables
             tr, pk, w, b0 = track_pack_resynth_local(t, spv.plan, spv.plans, sr, hop, self.nfft, self.hop, edge, minframes,
                                                      maxpitchjmp=self.local._maxpitchjmp, after_link=self._hook,
-                                                     after_pack=lambda tr_: self._handle.join_before_render())
+                                                     after_pack=lambda tr_: self._handle.join_before_render(),
+                                                     formant=formant)
             self.local._trk = tr
             if pk is not None:
                 self.local._pk = pk
@@ -850,6 +860,9 @@ class ShardedSinSum(object):
                                    self.device_track_table, self.ntracks, sr, hop, self.nfft, self.hop, fscale, ws, pws,
                                    edge, spv.group)
             mode = dict(phase_preserve=False, fscale=fscale, phase_ws=pws, scanned=True)
+        if formant is not None:
+            mode["pmag"] = P._formant_gains(formant, tidl, int(pk["tstart"].shape[0]), None, pk["tstart"], pk["toff"],
+                                            pk["pf"], pk["pmag"], pk["pf"].numel())
         if hostbuf is None:
             w = resynth_local(tidl, pk, *args, None, sr, hop, self.nfft, self.hop, edge, minframes, ws=ws,
                               local_last=ll, **mode)

@@ -384,20 +384,59 @@ class _DeviceCurve(object):
         self.t = t
 
 
-def _curve_values(fscale):
+def _curve_values(fscale, name="fscale"):
     """float64 numpy copy of a ratio curve of any shape, every value finite and > 0."""
     if isinstance(fscale, torch.Tensor):
         if fscale.dtype == torch.bool or fscale.is_complex():
-            raise TypeError("an fscale curve must hold real numbers, not %s" % fscale.dtype)
+            raise TypeError("an %s curve must hold real numbers, not %s" % (name, fscale.dtype))
         a = fscale.detach().cpu().numpy()
     else:
         a = np.asarray(fscale)
     if a.dtype.kind not in "iuf":
-        raise TypeError("an fscale curve must hold real numbers, not %s" % a.dtype)
+        raise TypeError("an %s curve must hold real numbers, not %s" % (name, a.dtype))
     a = np.ascontiguousarray(a, dtype=np.float64)
     if not np.all(np.isfinite(a)) or np.any(a <= 0.0):
-        raise ValueError("every value of an fscale curve must be finite and > 0")
+        raise ValueError("every value of an %s curve must be finite and > 0" % name)
     return a
+
+
+def _is_curve(v):
+    return isinstance(v, (np.ndarray, torch.Tensor, list, tuple))
+
+
+def _formant_values(formant_shift):
+    """Checked formant factor: a float, or a float64 numpy curve (any shape; 1-D checked by the caller)."""
+    if _is_curve(formant_shift):
+        return _curve_values(formant_shift, "formant_shift")
+    if isinstance(formant_shift, bool) or not isinstance(formant_shift, (int, float, np.integer, np.floating)):
+        raise TypeError("formant_shift must be None, a real number or a curve, not %s" % type(formant_shift).__name__)
+    phi = float(formant_shift)
+    if not np.isfinite(phi) or phi <= 0.0:
+        raise ValueError("formant_shift=%r must be finite and > 0" % phi)
+    return phi
+
+
+def formant_ratio(phase_preserve, fscale, formant_shift, nframes=None):
+    """Per-row ratio ``q = r / formant_shift`` of the formant gains (DESIGN.md 4.3), from the checked
+    ``(phase_preserve, fscale)`` of synth_mode(): None when ``formant_shift`` is None (the render keeps
+    the analysed magnitudes), a float, or a float64 numpy curve of one ratio per frame row.  ``r`` is
+    ``fscale`` (or ``fscale[j]``), 1 with ``phase_preserve=True``.
+
+    ``formant_shift`` takes the forms of ``fscale``: a finite value > 0 or a 1-D curve of ``nframes``
+    values, one per frame row.  1.0 keeps the spectral envelope of every row where it was (formant
+    preservation), ``phi`` moves it up by ``phi``, and ``formant_shift=fscale`` is the plain shift."""
+    if formant_shift is None:
+        return None
+    phi = _formant_values(formant_shift)
+    if isinstance(phi, np.ndarray):
+        if phi.ndim != 1:
+            raise ValueError("a formant_shift curve must be 1-D (one factor per frame), not of shape %s" % (phi.shape,))
+        if nframes is not None and len(phi) != nframes:
+            raise ValueError("the formant_shift curve has %d factors for %d frames" % (len(phi), nframes))
+    r = 1.0 if phase_preserve else fscale
+    if isinstance(r, np.ndarray) or isinstance(phi, np.ndarray):
+        return np.ascontiguousarray(np.asarray(r, dtype=np.float64) / phi, dtype=np.float64)
+    return float(r) / phi
 
 
 def synth_mode(phase_preserve=True, fscale=1.0, nframes=None):
@@ -455,6 +494,26 @@ def _phase_ws(phase_preserve, npts, dev):
     return torch.empty((max(int(npts), 1),), dtype=torch.float64, device=dev)
 
 
+def _formant_gains(formant, tid, nt, nt_dev, tstart, toff, pf, pmag, npts):
+    """The magnitudes the render takes: ``pmag`` itself without formant gains (``formant`` None), else
+    pvk_formant_gains into a new scratch of ``npts`` float64 (one per packed point, or an upper bound
+    such as F * K while the count is on the device, ``nt_dev``).  ``formant``: the ratio q of
+    formant_ratio(), a float or a _DeviceCurve of one ratio per row of ``tid``."""
+    if formant is None:
+        return pmag
+    L = _lib.lib()
+    F, K = tid.shape
+    out = torch.empty((max(int(npts), 1),), dtype=torch.float64, device=tid.device)
+    if isinstance(formant, _DeviceCurve):
+        q = (1.0, _ptr(formant.t), int(formant.t.numel()))
+    else:
+        q = (float(formant), None, 0)
+    with torch.cuda.device(tid.device):
+        _lib.check(L.pvk_formant_gains(_ptr(tid), F, K, int(nt), _ptr(nt_dev), _ptr(tstart), _ptr(toff), _ptr(pf),
+                                       _ptr(pmag), *q, _ptr(out), int(out.numel()), _stream()), "pvk_formant_gains")
+    return out
+
+
 def _resynth_ex(L, tid, F, K, nt, nt_dev, tstart, tlen, toff, pf, pmag, prealph, sr, hop, nfft, hop_an, edge, minframes,
                 out, nout, block0, nblocks, ws, reuse_tracks, phase_preserve, fscale, phase_ws, scanned=False):
     # scanned: the block start phases and Nyquist flags are in place already (pvk_resynth_render)
@@ -475,7 +534,7 @@ def _resynth_ex(L, tid, F, K, nt, nt_dev, tstart, tlen, toff, pf, pmag, prealph,
 
 def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edge=1.0, minframes=3,
                               maxpitchjmp=0.5, after_link=None, after_pack=None, block_range=None, before_sync=None,
-                              phase_preserve=True, fscale=1.0):
+                              phase_preserve=True, fscale=1.0, formant=None):
     """The whole back half of the hot path of one clip -- link, id resolution, pack, resynthesis --
     queued back to back with ONE host read-back at the very end: pack and resynthesis are launched
     sized by upper bounds (capacity of the index arrays, (F + 1) * hop + edge output samples) and
@@ -486,7 +545,9 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
     uncut (segment-sharded runs: the caller knows its block range without any count and trims once the
     global last frame is known).  ``before_sync`` (optional) is called once everything is queued,
     before the host waits: work launched there runs behind the rendering instead of after the wait.
-    ``phase_preserve`` / ``fscale``: see synth_mode() (a curve has one ratio per row of ``fd``)."""
+    ``phase_preserve`` / ``fscale``: see synth_mode() (a curve has one ratio per row of ``fd``).  ``formant``:
+    the ratio q of formant_ratio() (float, or _DeviceCurve of one ratio per row; None: no formant gains),
+    whose gains are computed between pack and render, still before the one read-back."""
     phase_preserve, fscale = synth_mode(phase_preserve, fscale, nframes=fd.shape[0])
     fscale = _on_device(fscale, fd.device)
     L = _lib.lib()
@@ -513,7 +574,8 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
         ws = resynth_workspace(F, K, nt_ub, nb, dev, hop=hop)
         pws = _phase_ws(phase_preserve, F * K, dev)
         with torch.cuda.device(dev):
-            _resynth_ex(L, tr["tid"], F, K, nt_ub, tr["ntracks"], tstart, tlen, toff, packed[0], packed[1], packed[3], sr,
+            pm = _formant_gains(formant, tr["tid"], nt_ub, tr["ntracks"], tstart, toff, packed[0], packed[1], F * K)
+            _resynth_ex(L, tr["tid"], F, K, nt_ub, tr["ntracks"], tstart, tlen, toff, packed[0], pm, packed[3], sr,
                         hop, nfft, hop_an, edge, minframes, out, nout_ub, b0, nb, ws, False, phase_preserve, fscale, pws)
     if before_sync is not None:
         before_sync(tr)
@@ -524,7 +586,7 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
         return tr, None, (None if block_range is None else out.zero_())
     if nt > nt_ub:                                              # more partials than the speculative cap: redo, sized exactly
         pk = pack_device(fd, magd, phd, realphd, tr["tid"], None, nt, npts=npts)
-        mode = dict(phase_preserve=phase_preserve, fscale=fscale)
+        mode = dict(phase_preserve=phase_preserve, fscale=fscale, formant=formant)
         if block_range is None:
             return tr, pk, resynth_device(tr["tid"], pk, sr, hop, nfft, hop_an, edge=edge, minframes=minframes, max_end=last,
                                           **mode)
@@ -558,14 +620,17 @@ def synth_geometry(max_end, hop, nfft, hop_an, edge=1.0):
 
 def resynth_device(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, max_end=None, block0=0,
                    nblocks=-1, out=None, ws=None, reuse_tracks=False, nout=None, phase_preserve=True, fscale=1.0,
-                   phase_ws=None, scanned=False):
+                   phase_ws=None, scanned=False, formant=None, pmag=None):
     """pvk_resynth_ex for one clip; returns the float64 device signal (asynchronous).  ``ws``: a
     workspace tensor to (re)use; ``reuse_tracks``: ``ws`` (and ``phase_ws``) already hold the per-partial
     masks, fade parameters (and block start phases) of an earlier call with the same tracks and
     synthesis parameters.  ``phase_preserve`` / ``fscale``: see synth_mode(); ``phase_ws``: the
     integrated-phase scratch to (re)use, one float64 per packed point.  ``scanned``: ``ws`` and
     ``phase_ws`` already hold the block start phases and Nyquist flags (dist.py's hand-over), so the
-    scan is left out (pvk_resynth_render).  A ``fscale`` curve has one ratio per row of ``tid``."""
+    scan is left out (pvk_resynth_render).  A ``fscale`` curve has one ratio per row of ``tid``.
+    ``formant``: the ratio q of formant_ratio() (float, or _DeviceCurve of one ratio per row of ``tid``):
+    the formant gains are computed first and rendered in place of ``pk['pmag']``; ``pmag``: such gains
+    computed already (_formant_gains; calls rendering one signal in block ranges share them)."""
     phase_preserve, fscale = synth_mode(phase_preserve, fscale, nframes=tid.shape[0])
     fscale = _on_device(fscale, tid.device)
     if scanned and (phase_preserve or phase_ws is None):
@@ -589,7 +654,9 @@ def resynth_device(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, max_en
             raise ValueError("reuse_tracks with phase_preserve=False needs the phase_ws of the first call")
         phase_ws = _phase_ws(False, pk["pf"].numel(), dev)
     with torch.cuda.device(dev):
-        _resynth_ex(L, tid, F, K, nt, None, pk["tstart"], pk["tlen"], pk["toff"], pk["pf"], pk["pmag"], pk["prealph"], sr,
+        if pmag is None:
+            pmag = _formant_gains(formant, tid, nt, None, pk["tstart"], pk["toff"], pk["pf"], pk["pmag"], pk["pf"].numel())
+        _resynth_ex(L, tid, F, K, nt, None, pk["tstart"], pk["tlen"], pk["toff"], pk["pf"], pmag, pk["prealph"], sr,
                     hop, nfft, hop_an, edge, minframes, out, nout, block0, nblocks, ws, reuse_tracks, phase_preserve,
                     fscale, None if phase_preserve else phase_ws, scanned)
     return out
@@ -1284,13 +1351,16 @@ class SinSumBatch(object):
     def __len__(self):
         return self._pb.nclips
 
-    def synth_device(self, sr, hop, edge=1.0, minframes=3, phase_preserve=True, fscale=1.0):
+    def synth_device(self, sr, hop, edge=1.0, minframes=3, phase_preserve=True, fscale=1.0, formant_shift=None):
         """Render all clips in one pvk_resynth: float64 CUDA tensor [nclips, rows_per_clip * hop]; row c
         holds clip c's signal from its sample 0 (then the silence of the guard rows).  ``phase_preserve``
         / ``fscale`` as in SinSum.synth (one phase scan over the flattened table, a segment per partial);
-        a curve is ``[nclips, nframes]``, one ratio per clip and frame."""
+        a curve is ``[nclips, nframes]``, one ratio per clip and frame.  ``formant_shift``: as in SinSum.synth,
+        a value or a ``[nclips, nframes]`` curve."""
         pb = self._pb
-        phase_preserve, fscale = self._batch_mode(phase_preserve, fscale)
+        phase_preserve, fs = self._batch_mode(phase_preserve, fscale)
+        formant = self._batch_formant(phase_preserve, fscale, formant_shift)
+        fscale = fs
         if int(hop) != hop:
             raise TypeError("hop must be an integer number of samples")
         if edge > pb.max_edge:
@@ -1302,8 +1372,27 @@ class SinSumBatch(object):
         if tr["ntracks"] == 0 or nout == 0:
             return torch.zeros((pb.nclips, pb.rows_per_clip * hop), dtype=torch.float64, device=pb._dev)
         out = resynth_device(tr["tid"], pk, sr, hop, self.nfft, self.hop, edge=edge, minframes=minframes, nout=nout,
-                             phase_preserve=phase_preserve, fscale=fscale)
+                             phase_preserve=phase_preserve, fscale=fscale, formant=formant)
         return out.view(pb.nclips, pb.rows_per_clip * hop)
+
+    def _batch_formant(self, phase_preserve, fscale, formant_shift):
+        """formant_ratio() for a batch, from the checked ``phase_preserve`` of _batch_mode() and the caller's
+        ``fscale``: a float, or one ratio per row of the flattened table (the guard rows, where no partial
+        lives, at 1) on the device; None without ``formant_shift``."""
+        if formant_shift is None:
+            return None
+        pb = self._pb
+        phi = _formant_values(formant_shift)
+        if isinstance(phi, np.ndarray) and phi.shape != (pb.nclips, pb.nframes):
+            raise ValueError("a batch formant_shift curve must be [nclips, nframes] = [%d, %d], not of shape %s"
+                             % (pb.nclips, pb.nframes, phi.shape))
+        r = 1.0 if phase_preserve else _curve_values(fscale) if _is_curve(fscale) else float(fscale)
+        q = r / phi
+        if not isinstance(q, np.ndarray):
+            return float(q)
+        rows = np.ones((pb.nclips, pb.rows_per_clip))
+        rows[:, :pb.nframes] = q
+        return _DeviceCurve(torch.from_numpy(rows.reshape(-1)).to(pb._dev))
 
     def _batch_mode(self, phase_preserve, fscale):
         """synth_mode() for a batch: a ``[nclips, nframes]`` curve becomes one ratio per row of the
@@ -1329,10 +1418,11 @@ class SinSumBatch(object):
         n = np.array([synth_geometry(int(e), int(hop), self.nfft, self.hop, edge)[0] for e in last], dtype=np.int64)
         return np.where(last >= 0, n, 0)
 
-    def synth(self, sr, hop, edge=1.0, minframes=3, to_host=True, phase_preserve=True, fscale=1.0):
+    def synth(self, sr, hop, edge=1.0, minframes=3, to_host=True, phase_preserve=True, fscale=1.0, formant_shift=None):
         """SinSum.synth of every clip (PVAnalysis.py:1053-1070): list of ``nclips`` float64 signals
         (numpy, or CUDA views with ``to_host=False``), each of its own length."""
-        w = self.synth_device(sr, hop, edge, minframes, phase_preserve=phase_preserve, fscale=fscale)
+        w = self.synth_device(sr, hop, edge, minframes, phase_preserve=phase_preserve, fscale=fscale,
+                              formant_shift=formant_shift)
         n = self.clip_lengths(hop, edge)
         if to_host:
             wh = w.cpu().numpy()
@@ -1651,7 +1741,7 @@ class SinSum(object):
 
     # -- resynthesis ---------------------------------------------------------------------
     def synth(self, sr, hop, edge=1.0, minframes=3, phase_preserve=True, to_host=True, hostbuf=None, chunks=8,
-              fscale=1.0):
+              fscale=1.0, formant_shift=None):
         """Overlap-add resynthesis of all partials with >= minframes frames
         (PVAnalysis.py:1053-1070); float64 ``[(max(end)+2)*hop + edgsamp]``.
         ``phase_preserve=False``: integrated phase instead of the analysed one -- the phase of a partial
@@ -1662,17 +1752,27 @@ class SinSum(object):
         block ``b`` (glides, vibrato, intonation), e.g. ``r = ratio_of(np.arange(nframes) * hop_an /
         sr)`` with the input time of each frame row; a partial is then left out when any of its points
         has ``r[row] * f >= sr / 2`` (see synth_mode()).
+        ``formant_shift`` (default None: every partial keeps its analysed magnitudes) moves the spectral
+        envelope of each frame row -- the piecewise-linear interpolation of ln(magnitude) over the
+        frequencies of the row's peaks -- independently of the pitch: a partial moved to ``r * f`` takes
+        the envelope's value at ``r * f / formant_shift``.  ``formant_shift=1.0`` preserves the formants
+        of a pitch shift (no "chipmunk" voice), ``formant_shift=phi`` with ``phase_preserve=True`` shifts
+        the formants by ``phi`` at the analysed pitch and phases, ``formant_shift=fscale`` renders exactly
+        the plain shift.  A value, or a curve of one factor per frame row like ``fscale``; the gains
+        change the rendered magnitudes only (see formant_ratio(), DESIGN.md 4.3).
         ``to_host=False`` returns the CUDA tensor instead of a numpy array.  ``hostbuf`` (a dict,
         reused across calls): render in ``chunks`` block ranges and download each finished range
         into the pinned tensor ``hostbuf['w']`` while the next one is rendered; returns a numpy view
         of it (valid until the next call with the same ``hostbuf``)."""
         nframes = None
-        if isinstance(fscale, (np.ndarray, torch.Tensor, list, tuple)):
+        if _is_curve(fscale) or _is_curve(formant_shift):
             if self._trk is None:
                 self._ensure_tables()
             nframes = int((self._trk["tid"] if self._trk is not None else self._tables["f"]).shape[0])
         phase_preserve, fscale = synth_mode(phase_preserve, fscale, nframes)
-        mode = dict(phase_preserve=phase_preserve, fscale=_on_device(fscale, self._dev))
+        formant = formant_ratio(phase_preserve, fscale, formant_shift, nframes)
+        mode = dict(phase_preserve=phase_preserve, fscale=_on_device(fscale, self._dev),
+                    formant=_on_device(formant, self._dev))
         if int(hop) != hop:
             raise TypeError("hop must be an integer number of samples")
         if self._trk is None and hostbuf is not None:
@@ -1707,7 +1807,8 @@ class SinSum(object):
                              max_end=tr.get("max_end"), **mode)
         return out.cpu().numpy() if to_host else out
 
-    def _synth_streamed_fused(self, sr, hop, edge, minframes, hostbuf, chunks, phase_preserve=True, fscale=1.0):
+    def _synth_streamed_fused(self, sr, hop, edge, minframes, hostbuf, chunks, phase_preserve=True, fscale=1.0,
+                              formant=None):
         """synth(hostbuf=...) on fresh partials: link, pack, the chunked rendering and the downloads of
         the finished chunks are all queued before the host reads any count (sizes are upper bounds,
         pvk_track_pack_dev / pvk_resynth_dev); the signal is cut to its real length at the end.  Returns
@@ -1734,11 +1835,12 @@ class SinSum(object):
             bounds = _chunk_bounds(nblk, chunks)
             ws = resynth_workspace(F, K, nt_ub, max(b - a for a, b in zip(bounds, bounds[1:])), dev, hop=hop)
             pws = _phase_ws(phase_preserve, F * K, dev)        # the phase scan runs with the first chunk
+            pm = _formant_gains(formant, tr["tid"], nt_ub, tr["ntracks"], tstart, toff, packed[0], packed[1], F * K)
             _mark("pack queued", cur)
             for i in range(chunks):
                 b0, b1 = bounds[i], bounds[i + 1]
                 n0, n1 = b0 * hop, min(b1 * hop, nout_ub)
-                _resynth_ex(L, tr["tid"], F, K, nt_ub, tr["ntracks"], tstart, tlen, toff, packed[0], packed[1], packed[3],
+                _resynth_ex(L, tr["tid"], F, K, nt_ub, tr["ntracks"], tstart, tlen, toff, packed[0], pm, packed[3],
                             sr, hop, self.nfft, self.hop, edge, minframes, out[n0:n1], nout_ub, b0, b1 - b0, ws, i > 0,
                             phase_preserve, fscale, pws)
                 ev = torch.cuda.Event()
@@ -1763,7 +1865,8 @@ class SinSum(object):
         self._last_out = out
         return hw[:nout].numpy()
 
-    def _synth_streamed(self, pk, tr, sr, hop, edge, minframes, hostbuf, chunks, phase_preserve=True, fscale=1.0):
+    def _synth_streamed(self, pk, tr, sr, hop, edge, minframes, hostbuf, chunks, phase_preserve=True, fscale=1.0,
+                        formant=None):
         dev = self._dev
         F, K = tr["tid"].shape
         max_end = tr.get("max_end")
@@ -1782,13 +1885,15 @@ class SinSum(object):
             ws = resynth_workspace(F, K, int(pk["tstart"].shape[0]), max(b - a for a, b in zip(bounds, bounds[1:])), dev,
                                    hop=hop)
             pws = _phase_ws(phase_preserve, pk["pf"].numel(), dev)  # the phase scan runs with the first chunk
+            pm = _formant_gains(formant, tr["tid"], int(pk["tstart"].shape[0]), None, pk["tstart"], pk["toff"], pk["pf"],
+                                pk["pmag"], pk["pf"].numel())
             _mark("pack done", cur)
             for i in range(chunks):
                 b0, b1 = bounds[i], bounds[i + 1]
                 n0, n1 = b0 * hop, min(b1 * hop, nout)
                 resynth_device(tr["tid"], pk, sr, hop, self.nfft, self.hop, edge=edge, minframes=minframes,
                                max_end=max_end, block0=b0, nblocks=b1 - b0, out=out[n0:n1], ws=ws, reuse_tracks=i > 0,
-                               phase_preserve=phase_preserve, fscale=fscale, phase_ws=pws)
+                               phase_preserve=phase_preserve, fscale=fscale, phase_ws=pws, pmag=pm)
                 ev = torch.cuda.Event()
                 ev.record(cur)
                 _mark("resynth %d" % i, cur)

@@ -10,8 +10,11 @@ nfft 2048 / hop 512 / npks 50 and tracked once; then, alternating in every round
   free_stretch  phase_preserve=False, synthesis hop 1024   (2x time stretch)
   free_curve    phase_preserve=False, a per-frame fscale curve: +-1 semitone vibrato at 5 Hz
                 (uploaded once before the timed passes; the upload is not part of the stage)
+  formant       free_shift with formant_shift=1.0: the formant gain kernel runs inside the timed stage
+  formant_curve free_curve with formant_shift=1.0 (a per-row ratio curve for the gain kernel)
 
-The phase scan alone (its three kernels) is timed from a torch.profiler capture of its own.  A
+The phase scan alone (its three kernels) is timed from a torch.profiler capture of the free mode, the
+formant gain kernel from one capture per formant mode.  A
 second leg does the same at the cfg4 length (one 8-hour signal, nfft 2048 / hop 256 / npks 100),
 where single partials span hundreds of thousands of frames.
 
@@ -98,8 +101,11 @@ def run_leg(c, dev, rounds, label):
     F, K = tid.shape
     modes = [("preserve", hop_an, True, 1.0), ("free", hop_an, False, 1.0),
              ("free_shift", hop_an, False, 2 ** (7 / 12.)), ("free_stretch", 2 * hop_an, False, 1.0),
-             ("free_curve", hop_an, False, vibrato_curve(F, hop_an, sr))]
-    dcurve = P._on_device(modes[-1][3], dev)
+             ("free_curve", hop_an, False, vibrato_curve(F, hop_an, sr)),
+             ("formant", hop_an, False, 2 ** (7 / 12.)), ("formant_curve", hop_an, False, vibrato_curve(F, hop_an, sr))]
+    dcurve = P._on_device(modes[4][3], dev)
+    # formant_shift=1.0 (formant preservation) at the shift / vibrato: the gain kernel runs inside the timed render
+    formant = {"formant": P.formant_ratio(False, modes[5][3], 1.0), "formant_curve": dcurve}
     bufs = {}
     for name, hop, pp, fs in modes:
         nout, _ = P.synth_geometry(max_end, hop, nfft, hop_an)
@@ -112,7 +118,8 @@ def run_leg(c, dev, rounds, label):
     def render(name, hop, pp, fs):
         b = bufs[name]
         P.resynth_device(tid, pk, sr, hop, nfft, hop_an, max_end=max_end, out=b["out"], ws=b["ws"],
-                         phase_preserve=pp, fscale=dcurve if name == "free_curve" else fs, phase_ws=b["pws"])
+                         phase_preserve=pp, fscale=dcurve if name in ("free_curve", "formant_curve") else fs,
+                         phase_ws=b["pws"], formant=formant.get(name))
 
     for m in modes:                                          # warm-up: module load, every shape once
         render(*m)
@@ -143,6 +150,22 @@ def run_leg(c, dev, rounds, label):
             kern[evt.key] = round(t / rounds, 2)
             if any(k in evt.key for k in SCAN_KERNELS):
                 scan_us += t / rounds
+    # the formant gain kernel alone: a capture of its own per formant mode (the scan of the free capture
+    # above stays the only one counted in scan_only_ms)
+    gain_us = {}
+    for m in (modes[5], modes[6]):
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            for _ in range(rounds):
+                flush.fill_(1)
+                render(*m)
+            torch.cuda.synchronize()
+        gain_us[m[0]] = 0.0
+        for evt in prof.key_averages():
+            if "formant_gain_kernel" in evt.key:
+                t = getattr(evt, "device_time_total", None)
+                if t is None:
+                    t = evt.cuda_time_total
+                gain_us[m[0]] += t / rounds
     res = dict(leg=label, workload=dict((k, c[k]) for k in ("sr", "seconds", "nfft", "hop", "npks")),
                frames=int(F), partials=int(tr["ntracks"]), points=int(pk["pf"].numel()),
                longest_partial_frames=int(pk["tlen"].max().item()), setup_s=round(prep_s, 1), rounds=rounds,
@@ -160,8 +183,13 @@ def run_leg(c, dev, rounds, label):
     res["scan_only_ms"] = round(scan_us / 1e3, 4)
     res["scan_share_of_free"] = round(scan_us / 1e3 / res["modes"]["free"]["median_ms"], 3)
     res["free_curve_vs_free"] = round(res["modes"]["free_curve"]["median_ms"] / res["modes"]["free"]["median_ms"], 3)
+    res["formant_vs_free_shift"] = round(res["modes"]["formant"]["median_ms"] / res["modes"]["free_shift"]["median_ms"], 3)
+    res["formant_curve_vs_free_curve"] = round(res["modes"]["formant_curve"]["median_ms"] /
+                                               res["modes"]["free_curve"]["median_ms"], 3)
+    res["formant_gain_kernel_us"] = {k: round(v, 2) for k, v in gain_us.items()}
+    res["formant_gain_share"] = {k: round(v / 1e3 / res["modes"][k]["median_ms"], 4) for k, v in gain_us.items()}
     res["profiled_kernels_us_per_pass"] = kern
-    del bufs, flush, tr, pk, dcurve
+    del bufs, flush, tr, pk, dcurve, formant
     torch.cuda.empty_cache()
     return res
 
