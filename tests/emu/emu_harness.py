@@ -201,7 +201,9 @@ def track_pack(f, mag, ph, realph, tid, link, ntracks):   # link unused (kept fo
 
 def resynth(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, block0=0, nblocks=-1, nout=None,
             ws_blocks=None):
-    """pvk_resynth for one clip: tid [F, K], pk = dict from track_pack."""
+    """pvk_resynth for one clip: tid [F, K], pk = dict from track_pack; ``ws_blocks``: see
+    resynth_emu.workspace."""
+    import resynth_emu              # tests/resynth_emu.py imports this module
     L = lib()
     tid = np.ascontiguousarray(tid, dtype=np.int32)
     F, K = tid.shape
@@ -216,46 +218,22 @@ def resynth(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, block0=0, nbl
     out = np.full(min(nb * hop, nout - block0 * hop), np.nan)
     ts = np.ascontiguousarray(pk["tstart"], dtype=np.int32)
     tl = np.ascontiguousarray(pk["tlen"], dtype=np.int32)
-    wsb = int(L.pvk_resynth_workspace_bytes(F, K, nt, max(nb, 0)))
-    if ws_blocks is not None:       # force chunked rendering: room for ws_blocks blocks only
-        wsb = int(L.pvk_resynth_workspace_bytes(F, K, nt, 0)) + (ws_blocks - 1) * (K * 80 + 4)
-    ws = np.zeros(max(wsb, 8), dtype=np.uint8)
+    ws = resynth_emu.workspace(F, K, nt, nb, ws_blocks)
     check(L.pvk_resynth(ptr(tid), F, K, nt, ptr(ts), ptr(tl), ptr(pk["toff"]), ptr(pk["pf"]), ptr(pk["pmag"]),
                         ptr(pk["prealph"]), float(sr), int(hop), int(nfft), int(hop_an), float(edge),
-                        int(minframes), ptr(out), nout, block0, nblocks, ptr(ws), wsb, 0, None))
+                        int(minframes), ptr(out), nout, block0, nblocks, ptr(ws), ws.size, 0, None))
     return out
 
 
-def segment_stitch(tids, plans):
-    """pvk_segment_summary -> (concatenate = all_gather) -> pvk_segment_resolve -> pvk_segment_rename for
-    every segment; tids[r]: local ids int32 [rows, K] of segment r.  Returns (list of global id arrays of
-    the own rows, total partials, last frame with a point)."""
-    L = lib()
-    world = len(plans)
-    K = tids[0].shape[1]
-    summ = np.zeros((world, 2 * K + 4), dtype=np.int32)
-    tids = [np.ascontiguousarray(t, dtype=np.int32) for t in tids]
-    for r, p in enumerate(plans):
-        check(L.pvk_segment_summary(ptr(tids[r]), K, p["own0"], p["nown"], p["j0"], ptr(summ[r]), None))
-    out, ntot, max_end = [], None, None
-    for r, p in enumerate(plans):
-        cap = max(max(q["own0"] for q in plans) * K, 1)      # scratch holds any segment's back-halo ids
-        scratch = np.zeros(cap, dtype=np.int32)
-        gidlow = np.zeros(cap, dtype=np.int32)
-        params = np.zeros(8, dtype=np.int32)
-        check(L.pvk_segment_resolve(ptr(summ), world, K, r, ptr(scratch), cap, ptr(gidlow), ptr(params), None))
-        own = np.ascontiguousarray(tids[r][p["own0"]:p["own0"] + p["nown"]])
-        res = np.empty_like(own)
-        check(L.pvk_segment_rename(ptr(own), own.size, ptr(gidlow), ptr(params), ptr(res), None))
-        out.append(res)
-        ntot, max_end = int(params[3]), int(params[4])
-    return out, ntot, max_end
-
-
-def segment_stitch_push(tids, plans):
-    """The fused variant: every segment's pvk_segment_rename_push stores its renamed own rows into the
-    tables of ALL ranks (here: `world` numpy arrays standing in for local + peer memory).  Returns the
-    list of tables (each must be the complete global table)."""
+def segment_stitch(tids, plans, store="rename"):
+    """pvk_segment_summary -> (concatenate = all_gather) -> pvk_segment_resolve -> the renaming store of
+    every segment; tids[r]: local ids int32 [rows, K] of segment r.  ``store``: "rename"
+    (pvk_segment_rename) writes each segment's renamed own rows to an array of their own; "push"
+    (pvk_segment_rename_push) stores them into the tables of ALL ranks (here: `world` numpy arrays
+    standing in for local + peer memory); "mcast" (pvk_segment_rename_mcast) stores them once, to one
+    table standing in for the multicast address of all ranks' tables.  Returns (the arrays written: the
+    own rows of every segment, or the tables, each of which must be the complete global table; total
+    partials; last frame with a point)."""
     L = lib()
     world = len(plans)
     K = tids[0].shape[1]
@@ -264,18 +242,25 @@ def segment_stitch_push(tids, plans):
     tids = [np.ascontiguousarray(t, dtype=np.int32) for t in tids]
     for r, p in enumerate(plans):
         check(L.pvk_segment_summary(ptr(tids[r]), K, p["own0"], p["nown"], p["j0"], ptr(summ[r]), None))
-    tables = [np.full((F, K), -7, dtype=np.int32) for _ in range(world)]
-    dst = np.array([t.ctypes.data for t in tables], dtype=np.uint64)
+    out = [np.full((F, K), -7, dtype=np.int32) for _ in range({"rename": 0, "push": world, "mcast": 1}[store])]
+    dst = np.array([t.ctypes.data for t in out], dtype=np.uint64)
+    cap = max(max(q["own0"] for q in plans) * K, 1)          # scratch holds any segment's back-halo ids
     for r, p in enumerate(plans):
-        cap = max(max(q["own0"] for q in plans) * K, 1)
         scratch = np.zeros(cap, dtype=np.int32)
         gidlow = np.zeros(cap, dtype=np.int32)
         params = np.zeros(8, dtype=np.int32)
         check(L.pvk_segment_resolve(ptr(summ), world, K, r, ptr(scratch), cap, ptr(gidlow), ptr(params), None))
         own = np.ascontiguousarray(tids[r][p["own0"]:p["own0"] + p["nown"]])
-        check(L.pvk_segment_rename_push(ptr(own), own.size, ptr(gidlow), ptr(params), ptr(dst), world,
-                                        p["j0"] * K, None))
-    return tables
+        if store == "rename":
+            out.append(np.empty_like(own))
+            check(L.pvk_segment_rename(ptr(own), own.size, ptr(gidlow), ptr(params), ptr(out[-1]), None))
+        elif store == "push":
+            check(L.pvk_segment_rename_push(ptr(own), own.size, ptr(gidlow), ptr(params), ptr(dst), world,
+                                            p["j0"] * K, None))
+        else:
+            check(L.pvk_segment_rename_mcast(ptr(own), own.size, ptr(gidlow), ptr(params), ptr(out[0]), p["j0"] * K,
+                                             None))
+    return out, int(params[3]), int(params[4])
 
 
 def stft_bank(x, win, nfft, hop, nframes, fb_folded=None, fb_lo=None, fb_hi=None, flux_bins=None, inv_wsum2=None,

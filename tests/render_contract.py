@@ -32,6 +32,13 @@ import synth_modes_oracle as smo
 
 pi2 = 2.0 * np.pi
 CHUNK_BLOCKS = 32768          # blocks per prepare + render chunk of the staged kernels (full workspace)
+BODY_ITEM_BYTES = 80          # sizeof(BodyItem) in pvk_resynth.cu: one staged partial body
+
+
+def row_ws_bytes(K):
+    """Workspace bytes of one staged block of a table K peaks wide: K BodyItems and a 4-byte count
+    (``resynth_row_ws`` in pvk_resynth.cu)."""
+    return K * BODY_ITEM_BYTES + 4
 
 
 # ------------------------------------------------------------------ dispatch
@@ -61,7 +68,7 @@ def render_branch(hop, npks, nfft, hop_an, edge, nblocks=None, chunk_blocks=CHUN
         nch = -(-hop // RS)
         bd = 128 if nch >= 32 else 64
         nchp = min(nch, bd)
-        smem = npks * 80 + RS * (bd + 32 // RS) * 4 > 48 * 1024
+        smem = npks * BODY_ITEM_BYTES + RS * (bd + 32 // RS) * 4 > 48 * 1024
         chunks = 1 if nblocks is None else -(-nblocks // chunk_blocks)
         br = dict(kernel="resynth<%d>" % RS, RS=RS, nchp=nchp, G=min(bd // nchp, npks), tpb=None,
                   windowed=nch > bd, smem=smem, chunks=chunks)

@@ -156,7 +156,7 @@ def test_emu_segment_numbering_kernels(world):
     assert np.array_equal(np.concatenate(rows), g["tid"])
     assert ntot == len(g["st"]) and max_end == int(np.max(g["end"]))
     # the fused variant: every segment stores its renamed rows into the tables of all ranks
-    for table in eh.segment_stitch_push(tids, plans):
+    for table in eh.segment_stitch(tids, plans, store="push")[0]:
         assert np.array_equal(table, g["tid"])
 
 
@@ -325,18 +325,8 @@ def test_emu_segment_rename_mcast_equals_push():
     plans = D.plan_segments(512 + (F - 1) * 128 + 1, 512, 128, world)
     assert plans[-1]["frames_total"] == F
     tids = [np.ascontiguousarray(eh.track(f[p["w0"]:p["w1"]], mag[p["w0"]:p["w1"]])["tid"][0]) for p in plans]
-    tables = eh.segment_stitch_push(tids, plans)
-    L = eh.lib()
-    summ = np.zeros((world, 2 * K + 4), dtype=np.int32)
-    for r, p in enumerate(plans):
-        eh.check(L.pvk_segment_summary(eh.ptr(tids[r]), K, p["own0"], p["nown"], p["j0"], eh.ptr(summ[r]), None))
-    mc = np.full((F, K), -7, dtype=np.int32)
-    for r, p in enumerate(plans):
-        cap = max(max(q["own0"] for q in plans) * K, 1)
-        scratch = np.zeros(cap, dtype=np.int32); gidlow = np.zeros(cap, dtype=np.int32); params = np.zeros(8, dtype=np.int32)
-        eh.check(L.pvk_segment_resolve(eh.ptr(summ), world, K, r, eh.ptr(scratch), cap, eh.ptr(gidlow), eh.ptr(params), None))
-        own = np.ascontiguousarray(tids[r][p["own0"]:p["own0"] + p["nown"]])
-        eh.check(L.pvk_segment_rename_mcast(eh.ptr(own), own.size, eh.ptr(gidlow), eh.ptr(params), eh.ptr(mc), p["j0"] * K, None))
+    tables = eh.segment_stitch(tids, plans, store="push")[0]
+    (mc,), _, _ = eh.segment_stitch(tids, plans, store="mcast")
     full = eh.track(f, mag)["tid"][0]
     assert np.array_equal(mc, full)
     for t in tables:

@@ -14,13 +14,12 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "emu
 
 import formant_oracle as fo
 import render_contract as rc
-import sharded_emu_util as su
-from golden_util import case_golden, case_signal, pv_kwargs
+import resynth_emu as rem
+from golden_util import case_golden, case_signal
 from oracle import pv_oracle as orc
-from pypevoc_b200 import dist as D
 from pypevoc_b200 import pv as P
 
-eh = su.eh
+eh = rem.eh
 
 SEMITONES7 = 2 ** (7 / 12.)
 
@@ -81,7 +80,7 @@ def point_table(F, K, seed):
     if F > 4 and K > 2:
         mag[4, K // 3] = 0.0                                      # a gap inside the row
     tid = np.where(mag > 0, np.arange(F * K).reshape(F, K), -1).astype(np.int32)
-    return su.pack(tid, f, mag, t["realph"]) + (f, mag, t["realph"])
+    return rem.pack(tid, f, mag, t["realph"]) + (f, mag, t["realph"])
 
 
 @pytest.mark.parametrize("K", [1, 3, 50, 400, 1024])
@@ -98,7 +97,7 @@ def test_kernel_matches_oracle_synthetic(K):
 def test_kernel_matches_oracle_goldens(name):
     g = case_golden(name)
     tr = eh.track(g["f"], g["mag"])
-    tid, pk = su.pack(np.ascontiguousarray(tr["tid"][0]), g["f"], g["mag"], g["realph"])
+    tid, pk = rem.pack(np.ascontiguousarray(tr["tid"][0]), g["f"], g["mag"], g["realph"])
     F = tid.shape[0]
     sr = float(g["sr"]) if "sr" in g.files else case_signal(name)[1]
     vib = rc.vibrato(F, int(g["hop"]), sr)
@@ -129,40 +128,14 @@ def test_equal_ratio_keeps_magnitudes_bit_for_bit():
     check_close(got, fo.gained_packed(tid, pk, q))
 
 
-def _preserve_render(tid, pk, pmag, sr, hop, nfft, hop_an, edge, minframes, nout, block0=0, nblocks=-1):
-    L = eh.lib()
-    F, K = tid.shape
-    nt = len(pk["tstart"])
-    nb = -(-nout // hop) - block0 if nblocks < 0 else nblocks
-    out = np.full(min(nb * hop, nout - block0 * hop), np.nan)
-    ws = su._ws(F, K, nt, nb)
-    eh.check(L.pvk_resynth_ex(eh.ptr(tid), F, K, nt, None, eh.ptr(pk["tstart"]), eh.ptr(pk["tlen"]), eh.ptr(pk["toff"]),
-                              eh.ptr(pk["pf"]), eh.ptr(pmag), eh.ptr(pk["prealph"]), float(sr), hop, nfft, hop_an,
-                              float(edge), minframes, eh.ptr(out), nout, block0, nb, eh.ptr(ws), ws.size, 0, 1, 1.0, None,
-                              0, None))
-    return out
-
-
-def _golden_tracked(name):
-    g = case_golden(name)
-    _, sr = case_signal(name)
-    tr = eh.track(g["f"], g["mag"])
-    tid, pk = su.pack(np.ascontiguousarray(tr["tid"][0]), g["f"], g["mag"], g["realph"])
-    return g, sr, pv_kwargs(name)["nfft"], int(g["hop"]), tid, pk
-
-
-def _max_end(tid):
-    return int(np.nonzero((tid >= 0).any(axis=1))[0].max())
-
-
 @pytest.mark.parametrize("world", [2, 3, 5])
 @pytest.mark.parametrize("mode", ["preserve", "free"])
 @pytest.mark.parametrize("curve", [False, True])
 def test_sharded_equals_unsharded(world, mode, curve):
     """Each rank computes the gains of its window rows from its window tables alone: they equal the
     unsharded gains bit for bit at every point, and the concatenated own signals equal the unsharded
-    render bit for bit (integrated phase through tests/sharded_emu_util.py)."""
-    g, sr, nfft, hop_an, tid, pk = _golden_tracked("cfg3_clip")
+    render bit for bit (simulated ranks of tests/resynth_emu.py)."""
+    g, sr, nfft, hop_an, tid, pk = rem.golden_tracked("cfg3_clip")
     F, K = tid.shape
     fscale = 1.0 if mode == "preserve" else SEMITONES7
     phi = 1.0 / (1.0 + 0.2 * np.sin(np.arange(F) / 7.0)) if curve else 1.25
@@ -172,35 +145,22 @@ def test_sharded_equals_unsharded(world, mode, curve):
     rows, cols = np.nonzero(tid >= 0)
     v = tid[rows, cols].astype(np.int64)
     gmag[rows, cols] = gains[pk["toff"][v] + rows - pk["tstart"][v]]
-    plans = su.plans_for(F, nfft, hop_an, world, 1.0, 3)
+    plans = rem.plans_for(F, nfft, hop_an, world, 1.0, 3)
     for p in plans:
         w0, w1 = p["w0"], p["w1"]
         if w1 <= w0:
             continue
-        tl, pl = su.pack(tid[w0:w1], g["f"][w0:w1], g["mag"][w0:w1], g["realph"][w0:w1])
+        tl, pl = rem.pack(tid[w0:w1], g["f"][w0:w1], g["mag"][w0:w1], g["realph"][w0:w1])
         ql = q[w0:w1] if np.ndim(q) else q
         gl = emu_gains(tl, pl, ql)
         r_, c_ = np.nonzero(tl >= 0)
         vl = tl[r_, c_].astype(np.int64)
         assert np.array_equal(gl[pl["toff"][vl] + r_ - pl["tstart"][vl]], gmag[w0:w1][r_, c_])
-    max_end = _max_end(tid)
     hop = 2 * hop_an
-    pkg = dict(pk, pmag=gains)
-    if mode == "free":
-        ref = su.unsharded(tid, pkg, sr, hop, nfft, hop_an, 1.0, 3, fscale, max_end)
-        sig, _ = su.sharded(tid, g["f"], gmag, g["realph"], sr, hop, nfft, hop_an, 1.0, 3, fscale, world, plans=plans)
-    else:
-        nout, _ = P.synth_geometry(max_end, hop, nfft, hop_an, 1.0)
-        ref = _preserve_render(tid, pk, gains, sr, hop, nfft, hop_an, 1.0, 3, nout)
-        sig = np.zeros(nout)
-        for p in plans:
-            b0, b1, _ = D.render_range(p, plans, max_end, hop, nfft, hop_an, 1.0)
-            if b1 <= b0:
-                continue
-            w0, w1 = p["w0"], p["w1"]
-            tl, pl = su.pack(tid[w0:w1], g["f"][w0:w1], gmag[w0:w1], g["realph"][w0:w1])
-            out = _preserve_render(tl, pl, pl["pmag"], sr, hop, nfft, hop_an, 1.0, 3, nout - w0 * hop, b0 - w0, b1 - b0)
-            sig[b0 * hop:b0 * hop + len(out)] = out
+    pp = mode == "preserve"
+    ref = rem.render(tid, pk, sr, hop, nfft, hop_an, 1.0, 3, pp, fscale, pmag=gains)
+    sig, _ = rem.sharded(tid, g["f"], gmag, g["realph"], sr, hop, nfft, hop_an, 1.0, 3, fscale, world, plans=plans,
+                         phase_preserve=pp)
     assert not np.array_equal(gains, pk["pmag"])
     assert sig.shape == ref.shape
     assert np.array_equal(sig, ref), np.max(np.abs(sig - ref))
@@ -219,7 +179,7 @@ def test_batch_equals_clips_one_at_a_time():
     for c, (tid, pk, f, mag, _) in enumerate(clips):
         ff[c, :F], mm[c, :F] = f, mag
     flat_tid = np.where(mm > 0, np.arange(mm.size).reshape(mm.shape), -1).reshape(-1, K).astype(np.int32)
-    tidb, pkb = su.pack(flat_tid, ff.reshape(-1, K), mm.reshape(-1, K), np.zeros((3 * (F + G), K)))
+    tidb, pkb = rem.pack(flat_tid, ff.reshape(-1, K), mm.reshape(-1, K), np.zeros((3 * (F + G), K)))
     rows = np.ones((3, F + G))
     rows[:, :F] = q
     gb = emu_gains(tidb, pkb, rows.reshape(-1))
@@ -289,21 +249,6 @@ def envelope(f):
     return 0.02 + sum(a / (1.0 + ((f - fc) / 120.0) ** 2) for fc, a in RES)
 
 
-def _render_free(tid, pk, pmag, fscale, hop):
-    L = eh.lib()
-    F, K = tid.shape
-    nt = len(pk["tstart"])
-    nout, _ = P.synth_geometry(_max_end(tid), hop, NFFT_B, HOP_B, 1.0)
-    nb = -(-nout // hop)
-    out = np.full(nout, np.nan)
-    ws, pws = su._ws(F, K, nt, nb), su._pws(pk)
-    eh.check(L.pvk_resynth_ex(eh.ptr(tid), F, K, nt, None, eh.ptr(pk["tstart"]), eh.ptr(pk["tlen"]), eh.ptr(pk["toff"]),
-                              eh.ptr(pk["pf"]), eh.ptr(pmag), eh.ptr(pk["prealph"]), SR_B, hop, NFFT_B, HOP_B, 1.0, 3,
-                              eh.ptr(out), nout, 0, nb, eh.ptr(ws), ws.size, 0, 0, float(fscale), eh.ptr(pws), pws.size,
-                              None))
-    return out
-
-
 def _envelope_misfit(x):
     """Worst |ln| ratio of the harmonic peaks of the middle frames of ``x`` to ``envelope`` (after the
     best common scale factor), over peaks from 50 Hz to 2.7 kHz: the test signal's top harmonic, above
@@ -334,10 +279,10 @@ def test_formant_preservation_follows_the_envelope():
     assert _envelope_misfit(x) < FORMANT_MARGIN / 2                 # the analysis sees the envelope
     a = orc.analyze(x, SR_B, nfft=NFFT_B, hop=HOP_B, npks=40)
     tr = eh.track(a["f"], a["mag"])
-    tid, pk = su.pack(np.ascontiguousarray(tr["tid"][0]), a["f"], a["mag"], a["realph"])
+    tid, pk = rem.pack(np.ascontiguousarray(tr["tid"][0]), a["f"], a["mag"], a["realph"])
     gains = emu_gains(tid, pk, P.formant_ratio(False, 1.5, 1.0))
-    kept = _envelope_misfit(_render_free(tid, pk, gains, 1.5, HOP_B))
-    plain = _envelope_misfit(_render_free(tid, pk, pk["pmag"], 1.5, HOP_B))
+    kept = _envelope_misfit(rem.render(tid, pk, SR_B, HOP_B, NFFT_B, HOP_B, fscale=1.5, pmag=gains))
+    plain = _envelope_misfit(rem.render(tid, pk, SR_B, HOP_B, NFFT_B, HOP_B, fscale=1.5))
     print("envelope misfit: formant_shift=1.0 %.3f, none %.3f" % (kept, plain))
     assert kept < FORMANT_MARGIN
     assert plain > 3 * FORMANT_MARGIN

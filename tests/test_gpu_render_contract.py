@@ -73,7 +73,7 @@ def gpu_render(P, t, case, mode, r):
     ws = None
     if ws_blocks is not None:
         from pypevoc_b200 import _lib
-        wsb = int(_lib.lib().pvk_resynth_workspace_bytes(F, K, nt, 0)) + (ws_blocks - 1) * (K * 80 + 4)
+        wsb = int(_lib.lib().pvk_resynth_workspace_bytes(F, K, nt, 0)) + (ws_blocks - 1) * rc.row_ws_bytes(K)
         ws = torch.zeros(wsb, dtype=torch.uint8, device=dev)
     w = P.resynth_device(tr["tid"], pk, SR, hop, nfft, hop_an, edge, minframes, ws=ws,
                          phase_preserve=mode == "preserve", fscale=r).cpu().numpy()

@@ -15,6 +15,7 @@ import pytest
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "emu"))
 
 import render_contract as rc
+import resynth_emu as rem
 import synth_modes_oracle as smo
 
 eh = pytest.importorskip("emu_harness")
@@ -45,38 +46,11 @@ def tracked(name):
     return _TABLES[name]
 
 
-def render(tid, pk, sr, hop, nfft, hop_an, edge, minframes, mode, r=1.0, ws_blocks=None):
-    """pvk_resynth_ex (pvk_resynth_ex_curve for a curve ``r``) through the emulator."""
-    L = eh.lib()
-    F, K = tid.shape
-    nt = len(pk["tstart"])
-    max_end = int((pk["tstart"] + pk["tlen"] - 1).max())
-    dfr = 1.0 / (hop_an / float(nfft)) / 2.0
-    nout = (max_end + 2) * hop + int(dfr * hop * edge)
-    nb = -(-nout // hop)
-    out = np.full(nout, np.nan)
-    wsb = int(L.pvk_resynth_workspace_bytes(F, K, nt, nb))
-    if ws_blocks is not None:
-        wsb = int(L.pvk_resynth_workspace_bytes(F, K, nt, 0)) + (ws_blocks - 1) * (K * 80 + 4)
-    ws = np.zeros(wsb, dtype=np.uint8)
-    pws = np.full(max(len(pk["pf"]), 1), np.nan)
-    ts = np.ascontiguousarray(pk["tstart"], dtype=np.int32)
-    tl = np.ascontiguousarray(pk["tlen"], dtype=np.int32)
-    common = (eh.ptr(tid), F, K, nt, None, eh.ptr(ts), eh.ptr(tl), eh.ptr(pk["toff"]), eh.ptr(pk["pf"]),
-              eh.ptr(pk["pmag"]), eh.ptr(pk["prealph"]), float(sr), int(hop), int(nfft), int(hop_an), float(edge),
-              int(minframes), eh.ptr(out), nout, 0, -1, eh.ptr(ws), ws.size, 0, 1 if mode == "preserve" else 0)
-    if np.ndim(r) == 0:
-        eh.check(L.pvk_resynth_ex(*common, float(r), eh.ptr(pws), pws.size, None))
-    else:
-        fc = np.ascontiguousarray(r, dtype=np.float64)
-        eh.check(L.pvk_resynth_ex_curve(*common, 1.0, eh.ptr(fc), fc.size, eh.ptr(pws), pws.size, None))
-    return out
-
-
 def run_case(name, label, mode, r):
     hop, nfft, hop_an, edge, K, F, minframes, ws_blocks = rc.CASES[name]
     t, tid, pk, parts = tracked(name)
-    w = render(tid, pk, rc.SR, hop, nfft, hop_an, edge, minframes, mode, r, ws_blocks)
+    w = rem.render(tid, pk, rc.SR, hop, nfft, hop_an, edge, minframes, mode == "preserve", r, ws_blocks=ws_blocks,
+                   phase_ws=rem.phase_scratch(pk))
     ref = rc.reference(parts, rc.SR, hop, nfft, hop_an, edge, minframes, mode, r)
     scale = rc.amp_scale(parts, rc.SR, hop, nfft, hop_an, edge, minframes, None if mode == "preserve" else r)
     return rc.check_render(w, ref, scale, TAU_EMU, FLOOR, "%s %s" % (name, label), hop, rc.case_branch(rc.CASES[name]))

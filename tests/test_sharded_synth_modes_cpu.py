@@ -1,6 +1,6 @@
 """CPU: integrated-phase resynthesis of a segment-sharded signal (``ShardedSinSum.synth_local(
 phase_preserve=False, fscale=...)``), with the kernels run in the SIMT emulator (tests/emu).  Ranks
-are simulated one after another (tests/sharded_emu_util.py) and the concatenated own signals must
+are simulated one after another (tests/resynth_emu.py) and the concatenated own signals must
 equal the unsharded ``pvk_resynth_ex(phase_preserve=0)`` render bit for bit: on goldens, on synthetic
 tables that put partial starts and ends at every row around a boundary, and on degenerate plans."""
 import ctypes as C
@@ -8,11 +8,10 @@ import ctypes as C
 import numpy as np
 import pytest
 
-import sharded_emu_util as su
-from golden_util import case_golden, case_signal, pv_kwargs
+import resynth_emu as rem
 from pypevoc_b200 import dist as D
 
-eh = su.eh
+eh = rem.eh
 
 SEMITONES7 = 2 ** (7 / 12.)
 
@@ -22,22 +21,9 @@ def _build():
     eh.build()
 
 
-def golden(name):
-    g = case_golden(name)
-    _, sr = case_signal(name)
-    kw = pv_kwargs(name)
-    tr = eh.track(g["f"], g["mag"])
-    tid, pk = su.pack(np.ascontiguousarray(tr["tid"][0]), g["f"], g["mag"], g["realph"])
-    return g, sr, kw["nfft"], int(g["hop"]), tid, pk
-
-
-def max_end(tid):
-    return int(np.nonzero((tid >= 0).any(axis=1))[0].max())
-
-
 def check_equal(tid, pk, f, mag, realph, sr, hop, nfft, hop_an, fscale, world, edge=1.0, minframes=3):
-    ref = su.unsharded(tid, pk, sr, hop, nfft, hop_an, edge, minframes, fscale, max_end(tid))
-    sig, ranks = su.sharded(tid, f, mag, realph, sr, hop, nfft, hop_an, edge, minframes, fscale, world)
+    ref = rem.render(tid, pk, sr, hop, nfft, hop_an, edge, minframes, fscale=fscale)
+    sig, ranks = rem.sharded(tid, f, mag, realph, sr, hop, nfft, hop_an, edge, minframes, fscale, world)
     assert sig.shape == ref.shape
     assert np.array_equal(sig, ref), np.max(np.abs(sig - ref))
     return ref, ranks
@@ -50,16 +36,16 @@ CASES = [(name, world, hop_mult, fscale) for name in ("cfg3_clip", "metric_1s") 
 @pytest.mark.parametrize("name,world,hop_mult,fscale", CASES)
 def test_golden_sharded_equals_unsharded(name, world, hop_mult, fscale):
     """hop = the analysis hop, twice it (time stretch) and 200 (the general resynth_kernel path)."""
-    g, sr, nfft, hop_an, tid, pk = golden(name)
+    g, sr, nfft, hop_an, tid, pk = rem.golden_tracked(name)
     hop = 200 if hop_mult is None else hop_mult * hop_an
     check_equal(tid, pk, g["f"], g["mag"], g["realph"], sr, hop, nfft, hop_an, fscale, world)
 
 
 def test_golden_cases_need_the_handover():
-    g, sr, nfft, hop_an, tid, pk = golden("cfg3_clip")
-    ref = su.unsharded(tid, pk, sr, 256, nfft, hop_an, 1.0, 3, SEMITONES7, max_end(tid))
-    sig, _ = su.sharded(tid, g["f"], g["mag"], g["realph"], sr, 256, nfft, hop_an, 1.0, 3, SEMITONES7, 3,
-                        handover=False)
+    g, sr, nfft, hop_an, tid, pk = rem.golden_tracked("cfg3_clip")
+    ref = rem.render(tid, pk, sr, 256, nfft, hop_an, 1.0, 3, fscale=SEMITONES7)
+    sig, _ = rem.sharded(tid, g["f"], g["mag"], g["realph"], sr, 256, nfft, hop_an, 1.0, 3, SEMITONES7, 3,
+                         handover=False)
     assert not np.array_equal(sig, ref)
 
 
@@ -73,7 +59,7 @@ def synthetic(F=60, world=3, seed=0):
     own rows; column 2 is born in [j1, j1 + dE] of rank 0 (whose own blocks hold its fade-in head) and
     exceeds the limit only in rank 1's own rows."""
     rng = np.random.default_rng(seed)
-    plans = su.plans_for(F, NFFT, HOP_AN, world, 1.0, 3)
+    plans = rem.plans_for(F, NFFT, HOP_AN, world, 1.0, 3)
     Lb, Lf = D.halos(NFFT, HOP_AN, 1.0, 3)
     j1 = plans[0]["j1"]
     spans = [(0, F - 1, None), (min(5, F - 1), max(F - 3, min(5, F - 1)), None),
@@ -99,7 +85,7 @@ def synthetic(F=60, world=3, seed=0):
     f[:, 1] = np.where(tid[:, 1] >= 0, 3000.0, 0.0)
     for c, rows in hi.items():
         f[rows, c] = 5600.0                                       # 5600 * 2^(7/12) >= 8000 > 5600
-    tid, pk = su.pack(tid, f, mag, realph)
+    tid, pk = rem.pack(tid, f, mag, realph)
     return tid, pk, f, mag, realph, plans
 
 
@@ -116,7 +102,7 @@ def test_synthetic_nyquist_flags_cross_ranks():
     g1, g2 = tid[5, 1], tid[plans[0]["j1"] + 1, 2]
     assert [int(r["flags"][g1]) for r in ranks] == [0, 0, 1]        # the last rank alone sees it
     assert [int(r["flags"][g2]) for r in ranks] == [0, 1, 0]        # rank 1 sees it, rank 0 renders its head
-    sig, _ = su.sharded(tid, f, mag, realph, SR, 256, NFFT, HOP_AN, 1.0, 3, SEMITONES7, 3, global_flags=False)
+    sig, _ = rem.sharded(tid, f, mag, realph, SR, 256, NFFT, HOP_AN, 1.0, 3, SEMITONES7, 3, global_flags=False)
     assert not np.array_equal(sig, ref)
 
 

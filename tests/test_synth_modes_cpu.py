@@ -17,6 +17,7 @@ sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "emu
 from oracle import pv_oracle as orc
 from golden_util import case_golden, case_signal, pv_kwargs
 import parity_util as pu
+import resynth_emu as rem
 import synth_modes_oracle as smo
 
 eh = pytest.importorskip("emu_harness")
@@ -29,37 +30,6 @@ def _build():
     eh.build()
 
 
-def resynth_ex(tid, pk, sr, hop, nfft, hop_an, edge=1.0, minframes=3, phase_preserve=False, fscale=1.0,
-               block0=0, nblocks=-1, nout=None, ws_blocks=None, ws=None, phase_ws=None, reuse_tracks=0):
-    """pvk_resynth_ex for one clip through the emulator (host arrays stand in for device memory).
-    ``ws`` / ``phase_ws``: workspaces to (re)use across block-range calls."""
-    L = eh.lib()
-    tid = np.ascontiguousarray(tid, dtype=np.int32)
-    F, K = tid.shape
-    nt = len(pk["tstart"])
-    max_end = int((pk["tstart"] + pk["tlen"] - 1).max()) if nt else -1
-    dfr = 1.0 / (hop_an / float(nfft)) / 2.0
-    if nout is None:
-        nout = (max_end + 2) * hop + int(dfr * hop * edge)
-    nb = -(-nout // hop) - block0 if nblocks < 0 else nblocks
-    out = np.full(min(nb * hop, nout - block0 * hop), np.nan)
-    ts = np.ascontiguousarray(pk["tstart"], dtype=np.int32)
-    tl = np.ascontiguousarray(pk["tlen"], dtype=np.int32)
-    if ws is None:
-        wsb = int(L.pvk_resynth_workspace_bytes(F, K, nt, max(nb, 0)))
-        if ws_blocks is not None:
-            wsb = int(L.pvk_resynth_workspace_bytes(F, K, nt, 0)) + (ws_blocks - 1) * (K * 80 + 4)
-        ws = np.zeros(max(wsb, 8), dtype=np.uint8)
-    if phase_ws is None:
-        phase_ws = np.full(max(len(pk["pf"]), 1), np.nan)
-    eh.check(L.pvk_resynth_ex(eh.ptr(tid), F, K, nt, None, eh.ptr(ts), eh.ptr(tl), eh.ptr(pk["toff"]), eh.ptr(pk["pf"]),
-                              eh.ptr(pk["pmag"]), eh.ptr(pk["prealph"]), float(sr), int(hop), int(nfft), int(hop_an),
-                              float(edge), int(minframes), eh.ptr(out), nout, block0, nblocks, eh.ptr(ws), ws.size,
-                              int(reuse_tracks), 0 if not phase_preserve else 1, float(fscale), eh.ptr(phase_ws),
-                              phase_ws.size, None))
-    return out
-
-
 def golden_tracks(name):
     g = case_golden(name)
     _, sr = case_signal(name)
@@ -67,13 +37,7 @@ def golden_tracks(name):
     tr = eh.track(g["f"], g["mag"])
     nt = int(tr["ntracks"][0])
     pk = eh.track_pack(g["f"], g["mag"], g["ph"], g["realph"], tr["tid"][0], tr["link"][0], nt)
-    return g, sr, kw, tr["tid"][0], pk, parts_from_pack(pk)
-
-
-def parts_from_pack(pk):
-    o = pk["toff"]
-    return [dict(start_idx=int(pk["tstart"][v]), f=pk["pf"][o[v]:o[v + 1]], mag=pk["pmag"][o[v]:o[v + 1]],
-                 realph=pk["prealph"][o[v]:o[v + 1]]) for v in range(len(pk["tstart"]))]
+    return g, sr, kw, tr["tid"][0], pk, rem.parts(pk)
 
 
 # ------------------------------------------------------------------ the model
@@ -112,7 +76,7 @@ for _name in GOLDENS:
 def test_emu_integrated_phase_vs_oracle(name, hop, fscale, edge, minframes):
     g, sr, kw, tid, pk, parts = golden_tracks(name)
     hop_an = int(g["hop"])
-    w = resynth_ex(tid, pk, sr, hop, kw["nfft"], hop_an, edge, minframes, False, fscale)
+    w = rem.render(tid, pk, sr, hop, kw["nfft"], hop_an, edge, minframes, False, fscale)
     ref = smo.synth(parts, sr, hop, kw["nfft"], hop_an, edge, minframes, phase_preserve=False, fscale=fscale)
     assert w.shape == ref.shape
     assert pu.snr_db(w, ref) > 110.0
@@ -127,7 +91,7 @@ def test_emu_nyquist_rule(name):
     fs = 0.5 * sr / np.median(fmax)                           # about half of the partials are skipped
     skipped = [fs * m >= 0.5 * sr for m in fmax]
     assert any(skipped) and not all(skipped)
-    w = resynth_ex(tid, pk, sr, 256, kw["nfft"], hop_an, 1.0, 1, False, fs)
+    w = rem.render(tid, pk, sr, 256, kw["nfft"], hop_an, 1.0, 1, False, fs)
     ref = smo.synth(parts, sr, 256, kw["nfft"], hop_an, 1.0, 1, phase_preserve=False, fscale=fs)
     assert pu.snr_db(w, ref) > 110.0
     kept = [p for p, s in zip(parts, skipped) if not s]
@@ -152,9 +116,9 @@ def synthetic_long_partial(nfr, hop_an=256, nfft=1024, sr=16000.0, seed=0):
 def test_emu_long_partial_spans_scan_groups():
     """~3000 frames: three scan groups of 1024 points, carried through the group-sum scan."""
     tid, pk, sr, nfft, hop_an = synthetic_long_partial(3000)
-    parts = parts_from_pack(pk)
+    parts = rem.parts(pk)
     for hop, fscale in ((256, 1.0), (200, 1.25)):
-        w = resynth_ex(tid, pk, sr, hop, nfft, hop_an, 1.0, 3, False, fscale)
+        w = rem.render(tid, pk, sr, hop, nfft, hop_an, 1.0, 3, False, fscale)
         ref = smo.synth(parts, sr, hop, nfft, hop_an, 1.0, 3, phase_preserve=False, fscale=fscale)
         assert pu.snr_db(w, ref) > 110.0
 
@@ -163,7 +127,7 @@ def test_emu_batch_layout_does_not_change_a_partial():
     """The scanned phases depend on the partial's own points only: a partial placed after others in
     the packed array (shifting its group boundaries) renders to the same bits."""
     tid, pk, sr, nfft, hop_an = synthetic_long_partial(1500, seed=1)
-    w1 = resynth_ex(tid, pk, sr, 256, nfft, hop_an, 1.0, 3, False, 1.1)
+    w1 = rem.render(tid, pk, sr, 256, nfft, hop_an, 1.0, 3, False, 1.1)
     pre = 333                                                 # a short partial in front, in its own column
     F = 1500 + pre
     tid2 = np.full((F, 2), -1, dtype=np.int32)
@@ -173,7 +137,7 @@ def test_emu_batch_layout_does_not_change_a_partial():
                toff=np.array([0, pre, pre + 1500], dtype=np.int64),
                pf=np.concatenate([np.full(pre, 300.0), pk["pf"]]), pmag=np.concatenate([np.zeros(pre), pk["pmag"]]),
                prealph=np.concatenate([np.zeros(pre), pk["prealph"]]))
-    w2 = resynth_ex(tid2, pk2, sr, 256, nfft, hop_an, 1.0, 3, False, 1.1)
+    w2 = rem.render(tid2, pk2, sr, 256, nfft, hop_an, 1.0, 3, False, 1.1)
     assert np.array_equal(w2[pre * 256:], w1)
 
 
@@ -182,18 +146,16 @@ def test_emu_chunked_and_block_ranges_are_bit_identical(hop):
     g, sr, kw, tid, pk, parts = golden_tracks("cfg3_clip")
     hop_an = int(g["hop"])
     args = (tid, pk, sr, hop, kw["nfft"], hop_an, 1.0, 3, False, 0.75)
-    w = resynth_ex(*args)
-    assert np.array_equal(w, resynth_ex(*args))                              # repeatable
-    assert np.array_equal(w, resynth_ex(*args, ws_blocks=5))                 # small workspace
-    assert np.array_equal(w[3 * hop:7 * hop], resynth_ex(*args, block0=3, nblocks=4))
+    w = rem.render(*args)
+    assert np.array_equal(w, rem.render(*args))                              # repeatable
+    assert np.array_equal(w, rem.render(*args, ws_blocks=5))                 # small workspace
+    assert np.array_equal(w[3 * hop:7 * hop], rem.render(*args, block0=3, nblocks=4))
     # two block ranges, the second reusing the masks, fades and phases of the first
-    L = eh.lib()
     F, K = tid.shape
     nb = -(-len(w) // hop)
-    ws = np.zeros(int(L.pvk_resynth_workspace_bytes(F, K, len(pk["tstart"]), nb)), dtype=np.uint8)
-    pws = np.full(len(pk["pf"]), np.nan)
-    a = resynth_ex(*args, block0=0, nblocks=nb // 2, nout=len(w), ws=ws, phase_ws=pws)
-    b = resynth_ex(*args, block0=nb // 2, nblocks=nb - nb // 2, nout=len(w), ws=ws, phase_ws=pws, reuse_tracks=1)
+    ws, pws = rem.workspace(F, K, len(pk["tstart"]), nb), rem.phase_scratch(pk)
+    a = rem.render(*args, block0=0, nblocks=nb // 2, nout=len(w), ws=ws, phase_ws=pws)
+    b = rem.render(*args, block0=nb // 2, nblocks=nb - nb // 2, nout=len(w), ws=ws, phase_ws=pws, reuse_tracks=1)
     assert np.array_equal(w, np.concatenate([a, b]))
 
 
@@ -202,7 +164,7 @@ def test_emu_phase_preserve_through_ex_is_unchanged():
     hop_an = int(g["hop"])
     for hop in (512, 200):
         a = eh.resynth(tid, pk, sr, hop, kw["nfft"], hop_an)
-        b = resynth_ex(tid, pk, sr, hop, kw["nfft"], hop_an, phase_preserve=True, phase_ws=np.zeros(0))
+        b = rem.render(tid, pk, sr, hop, kw["nfft"], hop_an, phase_preserve=True, phase_ws=np.zeros(0))
         assert np.array_equal(a, b)
 
 
