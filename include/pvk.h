@@ -472,6 +472,28 @@ int pvk_formant_gains(const int32_t *tid, int64_t nframes, int npks, int64_t ntr
                       const double *qcurve, int64_t qcurve_len, double *pmag_out, int64_t pmag_out_len,
                       void *stream);
 
+/* ------------------------------------------------------------------ time map
+ * A time-varying time stretch (DESIGN.md 4.3, "Time map"): resample the partials of a packed table onto
+ * nrows_out output rows, row b read at the fractional frame tmap[b] = i + u (i = floor(tmap[b])).  For every
+ * slot c of row i holding partial v (0 <= tid[i, c] < ntracks), with k = i - tstart[v]:
+ *   tid_out[b, c]    = v (ids are kept; -1 for a slot without a point)
+ *   f_out, mag_out   = x0 + u * (x1 - x0), x0 / x1 the packed knots k / k + 1 of v (x1 = x0 past its last
+ *                      knot), every operation rounded separately (no FMA): u == 0 gives x0 exactly
+ *   realph_out       = prealph of knot k
+ * Slots without a point get zeros.  The outputs are [nrows_out, npks] frame tables, to be counted with
+ * pvk_track_stats and packed with pvk_track_pack (ph = realph_out) for the integrated-phase render.  With a
+ * non-decreasing map every partial's output rows form one run, so they are a valid track table; a
+ * partial whose rows the map skips is left without points (tlen = 0 after the pack).
+ *   tid, ntracks, tstart, tlen, toff, pf, pmag, prealph   the pack of the source table [nframes, npks]
+ *   tmap         device, nrows_out float64 frames; the caller checks them (finite, in [0, nframes - 1],
+ *                non-decreasing) -- a value outside [0, nframes - 1] gives a row without points
+ * Checks sizes, npks and NULL pointers before any CUDA call; allocates nothing.
+ */
+int pvk_time_map(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                 const int32_t *tlen, const int64_t *toff, const double *pf, const double *pmag,
+                 const double *prealph, const double *tmap, int64_t nrows_out, int32_t *tid_out,
+                 double *f_out, double *mag_out, double *realph_out, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -66,6 +66,7 @@ SIGNATURES = {
                                     _i64, _i64, _i64, _p, _i64, _p]),
     "pvk_nyquist_flags_curve": (_i, [_p, _p, _i64, _d, _d, _p, _i64, _i, _p, _i64, _p]),
     "pvk_formant_gains": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _d, _p, _i64, _p, _i64, _p]),
+    "pvk_time_map": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _p]),
 }
 
 

@@ -1452,3 +1452,77 @@ extern "C" int pvk_formant_gains(const int32_t *tid, int64_t nframes, int npks, 
   PVK_CHECK_LAUNCH("pvk_formant_gains");
   return PVK_OK;
 }
+
+// ------------------------------------------------------------------ time map (DESIGN.md 4.3)
+// Output row b reads the partials at the fractional frame tau[b] = i + u (i = floor(tau[b])): slot c
+// keeps the id of tid[i, c], and a point of partial v there becomes x0 + u * (x1 - x0) for its
+// frequency and magnitude, x0 / x1 the knots k = i - tstart[v] and k + 1 (x1 = x0 past the partial's
+// last knot, as np.interp), with its realph the lower knot's.  Every operation is rounded on its own
+// (no FMA), so the result equals the numpy model bit for bit and u == 0 gives x0 exactly.  One warp
+// per output row, lanes over columns: coalesced id reads and stores, gathers of two knots per point.
+// Ids at or beyond ntracks, and rows whose tau lies outside [0, F - 1], are slots without a point.
+namespace pvk {
+
+constexpr int TMAP_THREADS = 256;
+
+__global__ void __launch_bounds__(TMAP_THREADS) time_map_kernel(
+    const int32_t *__restrict__ tid, int64_t F, int K, int64_t ntracks, const int32_t *__restrict__ tstart,
+    const int32_t *__restrict__ tlen, const int64_t *__restrict__ toff, const double *__restrict__ pf,
+    const double *__restrict__ pmag, const double *__restrict__ prealph, const double *__restrict__ tmap, int64_t B,
+    int32_t *__restrict__ tid_out, double *__restrict__ f_out, double *__restrict__ mag_out,
+    double *__restrict__ realph_out) {
+  const int lane = lane_id();
+  const int64_t nw = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t b = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; b < B; b += nw) {
+    const double tau = tmap[b];
+    const bool inside = tau >= 0.0 && tau <= (double)(F - 1);
+    const double fl = inside ? floor(tau) : 0.0;
+    const int64_t i = (int64_t)fl;
+    const double u = __dadd_rn(tau, -fl);                         // exact: fl <= tau < fl + 1
+    for (int c = lane; c < K; c += 32) {
+      const int v = inside ? tid[i * K + c] : -1;
+      int id = -1;
+      double f = 0.0, m = 0.0, ph = 0.0;
+      if (v >= 0 && v < ntracks) {
+        const int64_t k = i - tstart[v];
+        const int n = tlen[v];
+        if (k >= 0 && k < n) {
+          const int64_t o = toff[v] + k;
+          const double f0 = pf[o], m0 = pmag[o];
+          const double f1 = k + 1 < n ? pf[o + 1] : f0, m1 = k + 1 < n ? pmag[o + 1] : m0;
+          f = __dadd_rn(f0, __dmul_rn(u, __dadd_rn(f1, -f0)));
+          m = __dadd_rn(m0, __dmul_rn(u, __dadd_rn(m1, -m0)));
+          ph = prealph[o];
+          id = v;
+        }
+      }
+      const int64_t q = b * K + c;
+      tid_out[q] = id;
+      f_out[q] = f;
+      mag_out[q] = m;
+      realph_out[q] = ph;
+    }
+  }
+}
+
+}  // namespace pvk
+
+extern "C" int pvk_time_map(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, const int32_t *tstart,
+                            const int32_t *tlen, const int64_t *toff, const double *pf, const double *pmag,
+                            const double *prealph, const double *tmap, int64_t nrows_out, int32_t *tid_out,
+                            double *f_out, double *mag_out, double *realph_out, void *stream) {
+  PVK_REQUIRE(npks >= 1 && npks <= PVK_MAX_NPKS, "pvk_time_map: npks=%d must be in [1, %d]", npks, PVK_MAX_NPKS);
+  PVK_REQUIRE(nframes >= 0 && ntracks >= 0 && nrows_out >= 0, "pvk_time_map: negative sizes");
+  if (nrows_out == 0) return PVK_OK;
+  PVK_REQUIRE(nframes >= 1, "pvk_time_map: a time map needs a table with at least one frame row");
+  PVK_REQUIRE(tid && tmap && tid_out && f_out && mag_out && realph_out &&
+                  (ntracks == 0 || (tstart && tlen && toff && pf && pmag && prealph)),
+              "pvk_time_map: NULL pointer argument");
+  const int64_t rows_per_cta = TMAP_THREADS / 32;
+  const int64_t g = (nrows_out + rows_per_cta - 1) / rows_per_cta < 148 * 16 ? (nrows_out + rows_per_cta - 1) / rows_per_cta
+                                                                               : 148 * 16;
+  PVK_LAUNCH(time_map_kernel, dim3((unsigned)g), dim3(TMAP_THREADS), 0, stream, tid, nframes, npks, ntracks, tstart,
+             tlen, toff, pf, pmag, prealph, tmap, nrows_out, tid_out, f_out, mag_out, realph_out);
+  PVK_CHECK_LAUNCH("pvk_time_map");
+  return PVK_OK;
+}

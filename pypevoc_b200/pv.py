@@ -598,6 +598,59 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
     return tr, _pack_sliced(raw, nt, npts), out[:nout]
 
 
+def time_map_values(time_map, nframes):
+    """Checked time map of a table of ``nframes`` frame rows: a float64 numpy copy of a 1-D array,
+    sequence or torch tensor of at least one real value, every value finite, in ``[0, nframes - 1]``,
+    and non-decreasing (equal neighbours hold the sound: a freeze).  Output block ``b`` renders the
+    partials as they are at the fractional analysis frame ``time_map[b]`` (DESIGN.md 4.3, "Time map")."""
+    if isinstance(time_map, torch.Tensor):
+        if time_map.dtype == torch.bool or time_map.is_complex():
+            raise TypeError("a time_map must hold real numbers, not %s" % time_map.dtype)
+        a = time_map.detach().cpu().numpy()
+    elif isinstance(time_map, (np.ndarray, list, tuple)):
+        a = np.asarray(time_map)
+    else:
+        raise TypeError("time_map must be a 1-D array of frame positions, not %s" % type(time_map).__name__)
+    if a.dtype.kind not in "iuf":
+        raise TypeError("a time_map must hold real numbers, not %s" % a.dtype)
+    a = np.ascontiguousarray(a, dtype=np.float64)
+    if a.ndim != 1 or a.size == 0:
+        raise ValueError("a time_map must be 1-D with at least one frame position, not of shape %s" % (a.shape,))
+    if not np.all(np.isfinite(a)):
+        raise ValueError("every value of a time_map must be finite")
+    if a[0] < 0.0 or a.max() > nframes - 1:
+        raise ValueError("the values of a time_map must lie in [0, %d] (the frame rows of the partials)"
+                         % (nframes - 1))
+    if np.any(np.diff(a) < 0.0):
+        raise ValueError("a time_map must be non-decreasing (a partial may only be read forwards)")
+    return a
+
+
+def time_map_device(tid, pk, tmap_dev):
+    """pvk_time_map of the partials ``tid`` ``[F, K]`` / ``pk`` (pack_device()) at the fractional frames
+    ``tmap_dev`` (float64 CUDA tensor, checked by time_map_values()), then pvk_track_stats and the pack
+    of the mapped tables, with ONE 24-byte read-back in between: ``(tid', pk', max_end')``, ``tid'``
+    ``[len(tmap_dev), K]`` with the partial ids kept (a partial the map skips packs with tlen 0) and
+    ``max_end'`` the last output row holding a point (-1: none)."""
+    L = _lib.lib()
+    dev = tid.device
+    F, K = tid.shape
+    B = int(tmap_dev.numel())
+    nt = int(pk["tstart"].shape[0])
+    tid_m = torch.empty((B, K), dtype=torch.int32, device=dev)
+    f_m, mag_m, realph_m = (torch.empty((B, K), dtype=torch.float64, device=dev) for _ in range(3))
+    stats = torch.empty((3, 1), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(L.pvk_time_map(_ptr(tid), F, K, nt, _ptr(pk["tstart"]), _ptr(pk["tlen"]), _ptr(pk["toff"]),
+                                  _ptr(pk["pf"]), _ptr(pk["pmag"]), _ptr(pk["prealph"]), _ptr(tmap_dev), B,
+                                  _ptr(tid_m), _ptr(f_m), _ptr(mag_m), _ptr(realph_m), _stream()), "pvk_time_map")
+        ntd = torch.full((1,), nt, dtype=torch.int32, device=dev)
+        _lib.check(L.pvk_track_stats(_ptr(tid_m), _ptr(ntd), 1, B, K, _ptr(stats), _stream()), "pvk_track_stats")
+    _, npts, last = track_counts(dict(stats=stats))
+    pk_m = pack_device(f_m, mag_m, realph_m, realph_m, tid_m, None, nt, npts=npts)
+    return tid_m, pk_m, last
+
+
 def spans_device(tid, ntracks):
     """pvk_track_spans: first frame / length of every partial of an id table ``[F, K]`` (device)."""
     L = _lib.lib()
@@ -1741,7 +1794,7 @@ class SinSum(object):
 
     # -- resynthesis ---------------------------------------------------------------------
     def synth(self, sr, hop, edge=1.0, minframes=3, phase_preserve=True, to_host=True, hostbuf=None, chunks=8,
-              fscale=1.0, formant_shift=None):
+              fscale=1.0, formant_shift=None, time_map=None):
         """Overlap-add resynthesis of all partials with >= minframes frames
         (PVAnalysis.py:1053-1070); float64 ``[(max(end)+2)*hop + edgsamp]``.
         ``phase_preserve=False``: integrated phase instead of the analysed one -- the phase of a partial
@@ -1760,21 +1813,40 @@ class SinSum(object):
         the formants by ``phi`` at the analysed pitch and phases, ``formant_shift=fscale`` renders exactly
         the plain shift.  A value, or a curve of one factor per frame row like ``fscale``; the gains
         change the rendered magnitudes only (see formant_ratio(), DESIGN.md 4.3).
+        ``time_map`` (default None: output block ``b`` renders frame row ``b``) stretches time by a
+        different amount at every point: a 1-D, non-decreasing array of ``B`` fractional analysis frames
+        in ``[0, nframes - 1]``, output block ``b`` rendering the partials as they are at ``time_map[b]``
+        (frequency and magnitude interpolated between neighbouring frames; see time_map_values()).  The
+        local stretch at block ``b`` is ``hop / (hop_an * (time_map[b + 1] - time_map[b]))``; repeated
+        values freeze the sound.  A speed curve (analysis frames per output block) becomes a map as
+        ``tau = np.concatenate([[0.], np.cumsum(speed)]); tau = tau[tau <= nframes - 1]``.  A map needs
+        ``phase_preserve=False``; ``fscale`` and ``formant_shift`` curves then have one value per output
+        block (``B``), and ``minframes`` counts output blocks.  ``time_map=np.arange(nframes)`` renders
+        exactly what no map renders.  On the first use of the partials, link and pack run and are read
+        back before the map (the first use without a map queues everything behind one read-back).
         ``to_host=False`` returns the CUDA tensor instead of a numpy array.  ``hostbuf`` (a dict,
         reused across calls): render in ``chunks`` block ranges and download each finished range
         into the pinned tensor ``hostbuf['w']`` while the next one is rendered; returns a numpy view
         of it (valid until the next call with the same ``hostbuf``)."""
-        nframes = None
-        if _is_curve(fscale) or _is_curve(formant_shift):
+        nframes = tau = None
+        if _is_curve(fscale) or _is_curve(formant_shift) or time_map is not None:
             if self._trk is None:
                 self._ensure_tables()
             nframes = int((self._trk["tid"] if self._trk is not None else self._tables["f"]).shape[0])
+        if time_map is not None:
+            tau = time_map_values(time_map, nframes)
+            if phase_preserve:
+                raise ValueError("a time_map needs phase_preserve=False: analysed phases at fractional frames "
+                                 "mean nothing")
+            nframes = len(tau)                                  # curves: one value per output block
         phase_preserve, fscale = synth_mode(phase_preserve, fscale, nframes)
         formant = formant_ratio(phase_preserve, fscale, formant_shift, nframes)
         mode = dict(phase_preserve=phase_preserve, fscale=_on_device(fscale, self._dev),
                     formant=_on_device(formant, self._dev))
         if int(hop) != hop:
             raise TypeError("hop must be an integer number of samples")
+        if tau is not None:
+            return self._synth_mapped(tau, sr, int(hop), edge, minframes, to_host, hostbuf, int(chunks), **mode)
         if self._trk is None and hostbuf is not None:
             self._ensure_tables()
             if self._tables["f"].shape[0] * self._tables["f"].shape[1] > 0:
@@ -1805,6 +1877,32 @@ class SinSum(object):
             return self._synth_streamed(pk, tr, sr, int(hop), edge, minframes, hostbuf, int(chunks), **mode)
         out = resynth_device(tr["tid"], pk, sr, int(hop), self.nfft, self.hop, edge=edge, minframes=minframes,
                              max_end=tr.get("max_end"), **mode)
+        return out.cpu().numpy() if to_host else out
+
+    def _synth_mapped(self, tau, sr, hop, edge, minframes, to_host, hostbuf, chunks, phase_preserve=False, fscale=1.0,
+                      formant=None):
+        """synth(time_map=tau): the partials (linked and packed first if need be) resampled onto the output
+        rows by time_map_device(), then rendered by the staged or the streamed path as they render a
+        table.  The partials of this SinSum stay as they are."""
+        pk = self._ensure_packed()
+        tr = self._trk
+        if tr["ntracks"] == 0:
+            raise ValueError("max() arg is an empty sequence")     # what the reference raises (:1059)
+        tid_m, pk_m, last = time_map_device(tr["tid"], pk, torch.from_numpy(tau).to(self._dev))
+        if last < 0:                                            # the map reads only rows without points
+            nout, _ = synth_geometry(last, hop, self.nfft, self.hop, edge)
+            if hostbuf is not None:
+                hw = _pinned(hostbuf, "w", (nout,), torch.float64)[:nout]
+                hw.zero_()
+                return hw.numpy()
+            out = torch.zeros((nout,), dtype=torch.float64, device=self._dev)
+            return out.cpu().numpy() if to_host else out
+        mode = dict(phase_preserve=phase_preserve, fscale=fscale, formant=formant)
+        trm = dict(tid=tid_m, ntracks=tr["ntracks"], max_end=last)
+        if hostbuf is not None:
+            return self._synth_streamed(pk_m, trm, sr, hop, edge, minframes, hostbuf, chunks, **mode)
+        out = resynth_device(tid_m, pk_m, sr, hop, self.nfft, self.hop, edge=edge, minframes=minframes, max_end=last,
+                             **mode)
         return out.cpu().numpy() if to_host else out
 
     def _synth_streamed_fused(self, sr, hop, edge, minframes, hostbuf, chunks, phase_preserve=True, fscale=1.0,

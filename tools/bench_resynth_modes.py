@@ -12,6 +12,10 @@ nfft 2048 / hop 512 / npks 50 and tracked once; then, alternating in every round
                 (uploaded once before the timed passes; the upload is not part of the stage)
   formant       free_shift with formant_shift=1.0: the formant gain kernel runs inside the timed stage
   formant_curve free_curve with formant_shift=1.0 (a per-row ratio curve for the gain kernel)
+  time_map      phase_preserve=False, time_map: a stretch curve between 0.8x and 1.25x over the whole
+                signal.  Timed twice: the map stage alone (pvk_time_map, pvk_track_stats and its 24-byte
+                read-back, pvk_track_pack of the mapped tables) and the whole stage (map stage + render
+                of the mapped partials, allocations included, as SinSum.synth(time_map=...) runs it)
 
 The phase scan alone (its three kernels) is timed from a torch.profiler capture of the free mode, the
 formant gain kernel from one capture per formant mode.  A
@@ -90,6 +94,48 @@ def partial_samples(pk, hop, nfft, hop_an, sr, fscale=None, edge=1.0, minframes=
         keep &= fscale * fmax < 0.5 * sr
     E = int(nfft / hop_an / 2. * hop * edge)
     return int((tl[keep] * hop + 2 * E).sum().item())
+
+
+def stretch_map(F, period=700.0):
+    """A time map over the whole table whose local stretch moves between 0.8x and 1.25x (speed 1.25 ..
+    0.8 analysis frames per output block, a sine of ``period`` output blocks)."""
+    b = np.arange(2 * F)
+    tau = np.concatenate([[0.0], np.cumsum(1.025 + 0.225 * np.sin(2 * np.pi * b / period))])
+    return tau[tau <= F - 1]
+
+
+def time_leg_map(tid, pk, sr, nfft, hop_an, dev, rounds, flush):
+    """Median / min / max ms of the map stage and of the whole time-map stage (stretch_map)."""
+    F = tid.shape[0]
+    tau = stretch_map(F)
+    td = torch.from_numpy(tau).to(dev)
+
+    def whole():
+        tm, pkm, last = P.time_map_device(tid, pk, td)
+        P.resynth_device(tm, pkm, sr, hop_an, nfft, hop_an, max_end=last, phase_preserve=False)
+        return pkm
+
+    pkm = whole()                                            # warm-up
+    torch.cuda.synchronize()
+    ps = partial_samples(pkm, hop_an, nfft, hop_an, sr, 1.0)
+    del pkm
+    times = dict(map=[], whole=[])
+    for _ in range(rounds):
+        for name, fn in (("map", lambda: P.time_map_device(tid, pk, td)), ("whole", whole)):
+            flush.fill_(1)
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+            fn()
+            e1.record()
+            e1.synchronize()
+            times[name].append(e0.elapsed_time(e1))
+    t = {k: np.array(v) for k, v in times.items()}
+    return dict(output_blocks=int(len(tau)), stretch="0.8x .. 1.25x (speed sine, 700-block period)",
+                temp_table_bytes=int(len(tau) * tid.shape[1] * 28),
+                median_ms=round(float(np.median(t["whole"])), 4), min_ms=round(float(t["whole"].min()), 4),
+                max_ms=round(float(t["whole"].max()), 4), map_stage_median_ms=round(float(np.median(t["map"])), 4),
+                map_stage_min_ms=round(float(t["map"].min()), 4), partial_samples=ps,
+                partial_samples_per_s=float("%.4g" % (ps / (np.median(t["whole"]) * 1e-3))))
 
 
 def run_leg(c, dev, rounds, label):
@@ -189,6 +235,10 @@ def run_leg(c, dev, rounds, label):
     res["formant_gain_kernel_us"] = {k: round(v, 2) for k, v in gain_us.items()}
     res["formant_gain_share"] = {k: round(v / 1e3 / res["modes"][k]["median_ms"], 4) for k, v in gain_us.items()}
     res["profiled_kernels_us_per_pass"] = kern
+    tmr = time_leg_map(tid, pk, sr, nfft, hop_an, dev, rounds, flush)
+    res["modes"]["time_map"] = dict(hop=hop_an, phase_preserve=False, fscale=1.0, **tmr)
+    res["time_map_vs_free"] = round(tmr["median_ms"] / res["modes"]["free"]["median_ms"], 3)
+    res["time_map_stage_share"] = round(tmr["map_stage_median_ms"] / tmr["median_ms"], 3)
     del bufs, flush, tr, pk, dcurve, formant
     torch.cuda.empty_cache()
     return res
