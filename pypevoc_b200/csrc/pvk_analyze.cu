@@ -1,6 +1,8 @@
 // pvk_analyze.cu -- fused phase-vocoder analysis kernel for sm_100a.
 //
-// One CTA walks a run of consecutive STFT frames of one signal.  Per frame, without ever
+// One CTA walks a run of consecutive STFT frames of one signal (analyze_kernel: one frame at a
+// time; analyze_warp_kernel, nfft 1024 / 2048: one warp per frame, AW frames at a time, same
+// results bit for bit).  Per frame, without ever
 // leaving shared memory / registers:
 //   1. framing + windowing: the hop-strided frame is read straight from the signal with
 //      coalesced 64-bit loads (re-reads of the nfft-hop overlap hit L1/L2, HBM sees each
@@ -333,18 +335,33 @@ __device__ __forceinline__ void peak_phase_freq_fast(int k, const float2 *cur, c
   }
 }
 
+// |fx[k]|^2 in fp32 without FMA contraction (bit-identical to numpy float32 re*re + im*im)
+__device__ __forceinline__ float bin_power(float2 c) { return __fadd_rn(__fmul_rn(c.x, c.x), __fmul_rn(c.y, c.y)); }
+
+// Where the per-bin powers come from: analyze_kernel stores them (famp), analyze_warp_kernel
+// recomputes them from the untangled spectrum with bin_power -- the same bits either way.
+struct FampPow {
+  const float *famp;
+  __device__ __forceinline__ float operator()(int k) const { return famp[FA(k)]; }
+};
+struct SpecPow {
+  const float2 *spec;
+  __device__ __forceinline__ float operator()(int k) const { return bin_power(spec[PADC(k)]); }
+};
+
 // PVAnalysis.py:188-207 for the peak at bin k (1 <= k <= M-2)
+template <class Pow>
 __device__ __forceinline__ bool peak_epilogue(int k, int M, const float2 *cur, const float2 *prev,
-                                              const float *famp, const double *__restrict__ fbin,
+                                              const Pow &famp, const double *__restrict__ fbin,
                                               const double *__restrict__ wfbin, double dt, double inv,
                                               double step, double pi_fstep, PeakVals &o) {
   double thisph, bf, bdf;
   peak_phase_freq_fast(k, cur, prev, fbin, wfbin, dt, inv, step, thisph, bf, bdf);
   // mag = sqrt(sum(famp[max(nbin-1,1) : min(nbin+1,len)+1]**2)), left to right :197-199; famp holds
   // the fp32 powers |fx|^2, summed and rooted in fp32 (relative error ~2e-7, tolerance 1e-4)
-  float s = famp[FA(k)];
-  if (k - 1 >= 1) s = famp[FA(k - 1)] + s;
-  if (k + 1 <= M - 1) s = s + famp[FA(k + 1)];
+  float s = famp(k);
+  if (k - 1 >= 1) s = famp(k - 1) + s;
+  if (k + 1 <= M - 1) s = s + famp(k + 1);
   o.f = bf;
   o.mag = (double)sqrtf(s);
   o.ph = thisph;
@@ -355,8 +372,8 @@ __device__ __forceinline__ bool peak_epilogue(int k, int M, const float2 *cur, c
 // PeakFinder.refine (PeakFinder.py:331-372, fun=None, x = arange): parabola through
 // famp[k-1], famp[k], famp[k+1] (famp = sqrt of the stored power) -> fine position and value;
 // a bin that is not a local maximum keeps (k, famp[k]).  1 <= k <= M-2.
-__device__ __forceinline__ void refine_peak(int k, const float *famp, double &fpos, double &fval) {
-  const double s0 = sqrt((double)famp[FA(k - 1)]), s1 = sqrt((double)famp[FA(k)]), s2 = sqrt((double)famp[FA(k + 1)]);
+template <class Pow> __device__ __forceinline__ void refine_peak(int k, const Pow &famp, double &fpos, double &fval) {
+  const double s0 = sqrt((double)famp(k - 1)), s1 = sqrt((double)famp(k)), s2 = sqrt((double)famp(k + 1));
   if (s1 > s0 && s1 >= s2) {                                 // :354
     const double c = s1;
     const double b = __ddiv_rn(__dsub_rn(s2, s0), 2.0);
@@ -767,7 +784,7 @@ __global__ void __launch_bounds__(Plan<LOGM>::T, 512 / Plan<LOGM>::T) analyze_ke
       int k = 0;
       if (p < nk) {
         k = pk[p];
-        valid = peak_epilogue(k, M, cur, prev, famp, prm.fbin, prm.wfbin, prm.dt, inv_2pidt, inv_dt, pi_fstep, v);
+        valid = peak_epilogue(k, M, cur, prev, FampPow{famp}, prm.fbin, prm.wfbin, prm.dt, inv_2pidt, inv_dt, pi_fstep, v);
       }
       const int64_t pos = ob + round_pos<NW>(valid, wsB, round, outbase);
       if (valid) {
@@ -775,7 +792,7 @@ __global__ void __launch_bounds__(Plan<LOGM>::T, 512 / Plan<LOGM>::T) analyze_ke
         prm.realph[pos] = v.realph; prm.binno[pos] = (double)k;
         if (prm.fine_pos) {
           double fp, fv;
-          refine_peak(k, famp, fp, fv);
+          refine_peak(k, FampPow{famp}, fp, fv);
           prm.fine_pos[pos] = fp; prm.fine_val[pos] = fv;
         }
       }
@@ -792,6 +809,475 @@ __global__ void __launch_bounds__(Plan<LOGM>::T, 512 / Plan<LOGM>::T) analyze_ke
     __syncthreads();   // prev buffer is overwritten by the next frame's FFT
   }
   (void)N;
+}
+
+// ------------------------------------------------------------------ one warp per frame (LOGM 9, 10)
+// analyze_warp_kernel: a CTA of W warps walks a run of frames W at a time, warp w taking local frame
+// t = g W + w of group g (t = 0 is the warm-up row r0 - 1).  A frame never leaves its warp: the FFT
+// exchanges, the reductions, the select and the compactions use __syncwarp, shuffles and ballots.
+// The spectra live in a ring of W + 1 slots, frame t in slot t mod (W + 1); the only data shared
+// between warps is the previous frame's untangled spectrum that a frame's epilogue reads.  Two
+// block barriers per group: A, after the group's untangles and selects (frame t's epilogue reads
+// slot t - 1, which warp w - 1 wrote), and B, after the group's epilogues (each of them reads its
+// own slot and the one before, and the next group overwrites every slot but the last one written).
+// Every value is computed as analyze_kernel<LOGM> computes it, so the outputs are bit-identical:
+//   - the FFT runs Plan<LOGM>'s passes, twiddles and butterflies; lane l takes the butterflies
+//     i = l, l + 32, ... of each pass (two of the 64-thread plan's threads per lane);
+//   - the untangle keeps the 64-thread partition of the bins (virtual thread v = l + 32 h, h = 0, 1)
+//     because totalmag sums the fp32 partial sums of those threads per warp in fp64, then adds the
+//     two warp sums;
+//   - the powers are not stored: every reader recomputes them from the spectrum (bin_power);
+//   - candidates, radix select, tie rule, salience and epilogue decide exactly as there.
+// analyze_kernel's FFT and untangle are written with plain fp32 products and sums, and the compiler
+// fuses products into FFMA at its own discretion, site by site and depending on the kernel around
+// them.  The warp kernel spells out the roundings analyze_kernel<9/10> was compiled to (read off its
+// SASS), so that its spectrum has the same bits:
+//   - twiddle products of the exchange passes: re = a.x w.x (exact) - rn(a.y w.y), im = a.y w.x
+//     (exact) + rn(a.x w.y); of the untangle: re = o.x w.x - rn(o.y w.y), im = o.x w.y + rn(o.y w.x);
+//   - mul_w16 cases 1, 3, 5, 7: the first product exact, the second rounded; case 6 rounded; the
+//     case-2 products (d.x + d.y) C8 and (d.y - d.x) C8 stay exact into both sums of the next stage;
+//   - first pass: the windowed upper half of each first-stage butterfly is rounded, the lower half exact.
+// The fused multiply-add of those roundings.  The emulator build (g++ -ffp-contract=off) fuses no
+// product anywhere, so there it is unfused too: the emulator's analysis spectra then stay those of
+// its analyze_kernel, bank_kernel and harmonic_kernel builds.
+__device__ __forceinline__ float wfma(float a, float b, float c) {
+#ifdef PVK_EMU
+  return __fadd_rn(__fmul_rn(a, b), c);
+#else
+  return fmaf(a, b, c);
+#endif
+}
+__device__ __forceinline__ float2 wcmul_pass(float2 a, float2 w) {
+  return make_float2(wfma(a.x, w.x, -__fmul_rn(a.y, w.y)), wfma(a.y, w.x, __fmul_rn(a.x, w.y)));
+}
+__device__ __forceinline__ float2 wcmul_untangle(float2 o, float2 w) {
+  return make_float2(wfma(o.x, w.x, -__fmul_rn(o.y, w.y)), wfma(o.x, w.y, __fmul_rn(o.y, w.x)));
+}
+__device__ __forceinline__ float wsub(float a, float b) { return __fadd_rn(a, -b); }
+
+// dft_dif<LR> with those roundings.  WIN: u holds raw samples, w the window (first pass).
+template <int LR, bool WIN> __device__ __forceinline__ void wdft_dif(float2 *u, const float2 *w) {
+  constexpr int R = 1 << LR;
+  const float C8 = 0.70710678118654752440f, C1 = 0.92387953251128675613f, S1 = 0.38268343236508977173f;
+  unsigned pend = 0;                                         // u[i] holds s with value s * C8, unrounded
+#pragma unroll
+  for (int h = R / 2; h >= 1; h >>= 1) {
+    unsigned npend = 0;
+#pragma unroll
+    for (int g = 0; g < R; g += 2 * h) {
+#pragma unroll
+      for (int j = 0; j < h; ++j) {
+        const int ia = g + j, ib = g + j + h;
+        const float2 a = u[ia], b = u[ib];
+        float2 sm, d;
+        if (WIN && h == R / 2) {
+          const float2 pb = make_float2(__fmul_rn(b.x, w[ib].x), __fmul_rn(b.y, w[ib].y));
+          sm = make_float2(wfma(a.x, w[ia].x, pb.x), wfma(a.y, w[ia].y, pb.y));
+          d = make_float2(wfma(a.x, w[ia].x, -pb.x), wfma(a.y, w[ia].y, -pb.y));
+        } else if ((pend >> ia) & 1u) {
+          sm = make_float2(wfma(a.x, C8, b.x), wfma(a.y, C8, b.y));
+          d = make_float2(wfma(a.x, C8, -b.x), wfma(a.y, C8, -b.y));
+        } else if ((pend >> ib) & 1u) {
+          sm = make_float2(wfma(b.x, C8, a.x), wfma(b.y, C8, a.y));
+          d = make_float2(wfma(-b.x, C8, a.x), wfma(-b.y, C8, a.y));
+        } else {
+          sm = make_float2(__fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y));
+          d = make_float2(wsub(a.x, b.x), wsub(a.y, b.y));
+        }
+        u[ia] = sm;
+        switch (j * (8 / h)) {
+          case 0: u[ib] = d; break;
+          case 4: u[ib] = make_float2(d.y, -d.x); break;
+          case 2: u[ib] = make_float2(__fadd_rn(d.x, d.y), wsub(d.y, d.x)); npend |= 1u << ib; break;
+          case 6: u[ib] = make_float2(__fmul_rn(wsub(d.y, d.x), C8), -__fmul_rn(__fadd_rn(d.x, d.y), C8)); break;
+          case 1: u[ib] = make_float2(wfma(d.x, C1, __fmul_rn(d.y, S1)), wfma(d.y, C1, -__fmul_rn(d.x, S1))); break;
+          case 3: u[ib] = make_float2(wfma(d.x, S1, __fmul_rn(d.y, C1)), wfma(d.y, S1, -__fmul_rn(d.x, C1))); break;
+          case 5: u[ib] = make_float2(wfma(d.y, C1, -__fmul_rn(d.x, S1)), wfma(-d.y, S1, -__fmul_rn(d.x, C1))); break;
+          default: u[ib] = make_float2(wfma(d.y, S1, -__fmul_rn(d.x, C1)), wfma(-d.y, C1, -__fmul_rn(d.x, S1))); break;
+        }
+      }
+    }
+    pend = npend;
+  }
+}
+
+template <int LOGM, int Q> struct WPass {
+  using P = Plan<LOGM>;
+  static constexpr int M = P::M;
+  static constexpr int LR = P::lr(Q), R = 1 << LR, PP = 1 << P::lp(Q);
+  static constexpr int NBF = M >> LR, NBL = NBF / 32;        // butterflies per lane
+  static constexpr int OFF = P::tw_off(Q);
+  static_assert(NBF % 32 == 0, "whole butterflies per lane");
+
+  static __device__ __forceinline__ void run(const float2 *__restrict__ twp, float2 *buf) {
+    const int lane = lane_id();
+    // in place: every input of the lane's butterflies is read before any output lands.  Each
+    // butterfly is twiddled and transformed as soon as it is read, so that no twiddle stays live
+    // beside the 2 x 16 points of a radix-16 pass.
+    float2 u[NBL][R];
+#pragma unroll
+    for (int b = 0; b < NBL; ++b) {
+      const int i = lane + 32 * b;
+      const int k = i & (PP - 1);
+      u[b][0] = buf[PADC(i)];
+#pragma unroll
+      for (int r = 1; r < R; ++r) u[b][r] = wcmul_pass(buf[PADC(i + r * NBF)], __ldg(twp + OFF + (r - 1) * PP + k));
+      wdft_dif<LR, false>(u[b], nullptr);
+    }
+    __syncwarp();
+#pragma unroll
+    for (int b = 0; b < NBL; ++b) {
+      const int i = lane + 32 * b;
+      const int k = i & (PP - 1);
+      const int j = ((i - k) << LR) + k;
+#pragma unroll
+      for (int s = 0; s < R; ++s) buf[PADC(j + s * PP)] = u[b][brev<LR>(s)];
+    }
+    __syncwarp();
+    if constexpr (Q + 1 < P::NPASS) WPass<LOGM, Q + 1>::run(twp, buf);
+  }
+};
+
+// framing + window + first pass straight from the signal, then the exchange passes; natural order in buf
+template <int LOGM>
+__device__ __forceinline__ void wfft_frame(const float *__restrict__ xf, const float *__restrict__ win,
+                                           const float2 *__restrict__ twp, float2 *buf) {
+  using P = Plan<LOGM>;
+  constexpr int M = P::M, LR = P::lr(0), R = 1 << LR, NBF = M >> LR;
+  static_assert(NBF % 32 == 0, "whole butterflies per lane");
+  const int lane = lane_id();
+  const bool al8 = ((reinterpret_cast<uintptr_t>(xf) & 7) == 0);
+#pragma unroll
+  for (int b = 0; b < NBF / 32; ++b) {
+    const int i = lane + 32 * b;
+    float2 u[R], wv[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) u[r] = ldg_stream2(xf + 2 * (i + r * NBF), al8);
+#pragma unroll
+    for (int r = 0; r < R; ++r) wv[r] = __ldg(reinterpret_cast<const float2 *>(win) + i + r * NBF);
+    wdft_dif<LR, true>(u, wv);
+#pragma unroll
+    for (int s = 0; s < R; ++s) buf[PADC(i * R + s)] = u[brev<LR>(s)];
+  }
+  __syncwarp();
+  if constexpr (P::NPASS > 1) WPass<LOGM, 1>::run(twp, buf);
+}
+
+// Warps per CTA.  W + 1 spectrum slots plus W scratch areas: 98.9 KB at LOGM 10 (two CTAs = 16
+// warps per SM, as many as 128 registers per thread allow), 51.5 KB at LOGM 9.
+constexpr int AW = 8;
+
+template <int LOGM> struct WSmem {
+  using P = Plan<LOGM>;
+  static constexpr int SLOT = P::MP * 8;                     // one padded spectrum
+  static constexpr int OFF_SCR = (AW + 1) * SLOT;
+  // per warp: the candidate list (uint16), compacted in place into the selection and then into the
+  // salience survivors (a compaction never moves an entry up), and one 256-bucket histogram
+  static constexpr int SCR = P::M * 2 + 128 * 4;
+  static constexpr int BYTES = OFF_SCR + AW * SCR;
+};
+
+// Peak picking of one frame by one warp on its untangled spectrum `cur` (PeakFinder.__init__
+// :57-70, findpos, salience :113-134): the same decisions as analyze_kernel, with warp scans and
+// ballots instead of block barriers.  Leaves the surviving bins, ascending, in pk[0, return value).
+template <int LOGM>
+__device__ __forceinline__ int warp_peaks(const float2 *cur, float miny, float ymax, double pkthresh, int K,
+                                          unsigned short *pk, unsigned *hist) {
+  constexpr int M = Plan<LOGM>::M;
+  constexpr int CB = M / 32;                                 // contiguous bins per lane in the candidate scan
+  constexpr unsigned CB_MASK = CB == 32 ? 0xffffffffu : (1u << CB) - 1u;
+  const SpecPow pw{cur};
+  const int lane = lane_id();
+  unsigned short *cbin = pk;
+  // candidate list entry = bin | 0x8000 for a candidate that is not a local maximum (key 0)
+#define PVK_WKEY(v) (((v) & 0x8000) ? 0u : __float_as_uint(pw(v)))
+  const double miny_d = sqrt((double)miny);
+  double minamp = sqrt((double)ymax) * pkthresh;
+  if (minamp == 0.0) minamp = miny_d;
+  const double th = minamp - miny_d;
+
+  // ---- candidates: interior local maxima above threshold (or everything when th < 0), compacted in
+  //      bin order.  Lane l scans bins [l CB, (l + 1) CB); the guard band as in analyze_kernel.
+  int C;
+  unsigned lo, hi;
+  {
+    const int kb0 = lane * CB;
+    const bool allc = th < 0.0;
+    float thr_hi = -1.f, thr_lo = -1.f;                      // th < 0: every local maximum passes
+    if (!allc) {
+      const float mf = (float)(minamp * minamp);
+      thr_hi = mf * (1.f + 7.6293945e-6f); thr_lo = mf * (1.f - 7.6293945e-6f);
+    }
+    unsigned interior = CB_MASK;                             // bins 1 .. M-2
+    if (lane == 0) interior &= ~1u;
+    if (lane == 31) interior &= ~(1u << (CB - 1));
+    unsigned pbits = 0;                                      // local maxima not below the band
+    float yl = kb0 > 0 ? pw(kb0 - 1) : 0.f, yv = pw(kb0);
+#pragma unroll
+    for (int i = 0; i < CB; ++i) {
+      const float yr = (i + 1 < CB || kb0 + CB < M) ? pw(kb0 + i + 1) : 0.f;
+      if ((yl < yv) && (yv >= yr) && !(yv < thr_lo)) pbits |= 1u << i;
+      yl = yv; yv = yr;
+    }
+    pbits &= interior;
+    unsigned kmin = 0xffffffffu, kmax = 0u;
+    for (unsigned rem = pbits; rem;) {                       // few per lane: settle the band, key range
+      const int i = __ffs((int)rem) - 1;
+      rem &= rem - 1u;
+      const float y = pw(kb0 + i);
+      bool c = y > thr_hi;
+      if (!c) c = (sqrt((double)y) - miny_d) > th;
+      if (c) {
+        const unsigned key = __float_as_uint(y);
+        kmin = key < kmin ? key : kmin; kmax = key > kmax ? key : kmax;
+      } else {
+        pbits &= ~(1u << i);
+      }
+    }
+    unsigned cbits = pbits;
+    if (allc) {                                              // non-maxima are candidates too, key 0
+      cbits = interior;
+      if (interior & ~pbits) kmin = 0u;
+    }
+    const int cnt = __popc(cbits);
+    const int incl = warp_scan_incl(cnt);
+    C = __shfl_sync(FULL, incl, 31);
+    lo = warp_umin(kmin);
+    hi = warp_umax(kmax);
+    int pos = incl - cnt;
+    for (unsigned rem = cbits; rem;) {
+      const int i = __ffs((int)rem) - 1;
+      rem &= rem - 1u;
+      cbin[pos++] = (unsigned short)((kb0 + i) | (((pbits >> i) & 1u) ? 0 : 0x8000));
+    }
+    __syncwarp();
+  }
+
+  // ---- top-K by (key desc, bin asc): exact radix select of the K-th largest key, 8 bits per level,
+  //      as in analyze_kernel; every lane clears the histogram words it reads
+  int rr = K;
+  bool exact_ties = false;
+  const bool need_sel = C > K;
+  if (need_sel) {
+    for (int level = 0; level < 4; ++level) {
+      const unsigned range = hi - lo;
+      const int bl = 32 - __clz((int)range);
+      const int sh = bl > 8 ? bl - 8 : 0;
+      for (int e = lane; e < C; e += 32) {
+        const unsigned key = PVK_WKEY(cbin[e]);
+        if (key >= lo && key <= hi) {
+          const unsigned b = (key - lo) >> sh;
+          atomicAdd(&hist[b >> 1], 1u << ((b & 1u) * 16u));
+        }
+      }
+      __syncwarp();
+      // lane l owns buckets 255 - 8 l - q, q = 0 .. 7 (descending keys) = words 127 - 4 l - j, high half first
+      int c[8], sum = 0;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const unsigned w = hist[127 - 4 * lane - j];
+        hist[127 - 4 * lane - j] = 0u;
+        c[2 * j] = (int)(w >> 16); c[2 * j + 1] = (int)(w & 0xffffu);
+        sum += c[2 * j] + c[2 * j + 1];
+      }
+      __syncwarp();
+      const int incl = warp_scan_incl(sum);
+      int above = incl - sum;
+      const bool mine = above < rr && rr <= incl;               // exactly one lane
+      int bq = 0, ab = 0, cq = 0;
+      if (mine) {
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+          if (above < rr && rr <= above + c[q]) { bq = 255 - 8 * lane - q; ab = above; cq = c[q]; }
+          above += c[q];
+        }
+      }
+      const int src = __ffs((int)__ballot_sync(FULL, mine)) - 1;
+      const int b = __shfl_sync(FULL, bq, src), nabove = __shfl_sync(FULL, ab, src), cb = __shfl_sync(FULL, cq, src);
+      lo = lo + ((unsigned)b << sh);
+      const unsigned hi2 = lo + ((1u << sh) - 1u);
+      hi = hi2 < hi ? hi2 : hi;
+      rr -= nabove;
+      if (cb == rr) break;
+      if (sh == 0) { exact_ties = true; break; }
+    }
+
+    // ---- selected entries, compacted in place in bin order.  Selected = key above the boundary
+    //      bucket, or inside it (only its first rr entries in bin order when the bucket is a run of
+    //      exactly equal keys).  An entry's position is at most its index, and the entries of a
+    //      round are read before its ballot, so no entry is overwritten before it is read.
+    int sbase = 0, tbase = 0;
+    for (int e0 = 0; e0 < C; e0 += 32) {
+      const int e = e0 + lane;
+      const unsigned v = e < C ? cbin[e] : 0u;
+      const unsigned key = e < C ? PVK_WKEY(v) : 0u;
+      const bool inA = e < C && key > hi;
+      const bool inB = e < C && key >= lo && key <= hi;
+      bool s = inA || inB;
+      if (exact_ties) {                                          // rare: the first rr ties in bin order join
+        const unsigned mt = __ballot_sync(FULL, inB);
+        s = inA || (inB && tbase + __popc(mt & lanemask_lt()) < rr);
+        tbase += __popc(mt);
+      }
+      const unsigned ms = __ballot_sync(FULL, s);
+      if (s) cbin[sbase + __popc(ms & lanemask_lt())] = (unsigned short)(v & 0x7fff);
+      sbase += __popc(ms);
+    }
+    __syncwarp();
+  }
+  const int ns = need_sel ? K : C;
+
+  // ---- salience filter, rad = 5 (PeakFinder.py:113-134 as called at PVAnalysis.py:177), one lane
+  //      per selected peak; survivors compacted in place in bin order
+  int nk = 0;
+  for (int e0 = 0; e0 < ns; e0 += 32) {
+    const int e = e0 + lane;
+    bool keep = false;
+    int k = 0;
+    if (e < ns) {
+      k = cbin[e] & 0x7fff;
+      const float y = pw(k);
+      const int a = k - 5 > 1 ? k - 5 : 1, b = k + 5 < M - 1 ? k + 5 : M - 1;
+      keep = true;
+      for (int m = a; m <= b; ++m) keep = keep && !(pw(m) > y);
+    }
+    const unsigned mk = __ballot_sync(FULL, keep);
+    if (keep) cbin[nk + __popc(mk & lanemask_lt())] = (unsigned short)k;
+    nk += __popc(mk);
+  }
+  __syncwarp();
+#undef PVK_WKEY
+  return nk;
+}
+
+template <int LOGM>
+__global__ void __launch_bounds__(AW * 32, 16 / AW) analyze_warp_kernel(AParams prm) {
+  using P = Plan<LOGM>;
+  using S = WSmem<LOGM>;
+  constexpr int M = P::M, VT = P::T, W = AW;
+  static_assert(VT == 64, "totalmag follows the 64-thread partition of analyze_kernel<LOGM>");
+  PVK_SMEM(smem);
+#define PVK_SLOT(s) reinterpret_cast<float2 *>(smem + (int)(s) * S::SLOT)
+  const int lane = lane_id(), warp = warp_id();
+  unsigned short *cbin = reinterpret_cast<unsigned short *>(smem + S::OFF_SCR + warp * S::SCR);
+  unsigned *hist = reinterpret_cast<unsigned *>(cbin + M);  // 128 words (256 16-bit buckets)
+
+  const int64_t clip = blockIdx.x / prm.nruns;
+  const int64_t run = blockIdx.x % prm.nruns;
+  const int64_t r0 = run * prm.run;
+  const int64_t r1 = (r0 + prm.run < prm.nframes) ? r0 + prm.run : prm.nframes;
+  const int K = prm.npks;
+  const bool zero_start = (r0 == 0 && prm.prev_zero);
+  // local frame t = r - (r0 - 1): t = 0 only leaves its spectrum behind (the warm-up row, or the
+  // all-zero previous spectrum of global frame 0, PVAnalysis.py:121)
+  const float *x0 = prm.x + clip * prm.clip_stride + (prm.frame0 + r0 - 1) * (int64_t)prm.hop;   // frame t = 0
+  const int64_t row0 = clip * prm.out_rows + r0 - 1;
+  const int nloc = (int)(r1 - r0) + 1;
+
+  // every level of the select reads its histogram and clears it: zero once, zero after every frame
+#pragma unroll
+  for (int j = 0; j < 4; ++j) hist[lane + 32 * j] = 0u;
+  __syncwarp();
+
+  int slot = warp;                                           // t mod (W + 1)
+  for (int g0 = 0; g0 < nloc; g0 += W, slot = slot == 0 ? W : slot - 1) {
+    const int t = g0 + warp;
+    const bool act = t < nloc, emit = act && t > 0;
+    const int64_t row = row0 + t;
+    float2 *cur = PVK_SLOT(slot);
+    const float2 *prev = PVK_SLOT(slot == 0 ? W : slot - 1);
+    double sumsq = 0.0;
+    int nk = 0;
+    if (act && t == 0 && zero_start) {
+      for (int i = lane; i < P::MP; i += 32) cur[i] = make_float2(0.f, 0.f);
+    } else if (act) {
+      wfft_frame<LOGM>(x0 + t * (int64_t)prm.hop, prm.win, prm.tables, cur);
+
+      // ---- untangle -> fx[0..M), min / max / sum of the powers (bins of virtual thread v = lane + 32 h)
+      float lmin = 3.402823466e+38f, lmax = 0.f, lsum[2] = {0.f, 0.f};
+      float2 *so = (prm.spec_out && emit) ? prm.spec_out + row * M : nullptr;
+      constexpr int UI = (M / 2) / VT;
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+#pragma unroll
+        for (int it = 0; it < UI; ++it) {
+          const int k = lane + 32 * h + it * VT;
+          float2 xa, xb;
+          if (h == 0 && it == 0 && k == 0) {
+            const float2 z0 = cur[PADC(0)], zh = cur[PADC(M / 2)];
+            xa = make_float2(z0.x + z0.y, 0.f);
+            xb = make_float2(zh.x, -zh.y);
+          } else {
+            const float2 a = cur[PADC(k)], bq = cur[PADC(M - k)];
+            // (the products by 0.5 are exact: fused or not, the same bits)
+            const float2 e = make_float2(__fmul_rn(0.5f, __fadd_rn(a.x, bq.x)), __fmul_rn(0.5f, wsub(a.y, bq.y)));
+            const float2 o = make_float2(__fmul_rn(0.5f, __fadd_rn(a.y, bq.y)), __fmul_rn(-0.5f, wsub(a.x, bq.x)));
+            const float2 wo = wcmul_untangle(o, __ldg(prm.tables + P::TW_TOTAL + k));
+            xa = make_float2(__fadd_rn(e.x, wo.x), __fadd_rn(e.y, wo.y));
+            xb = make_float2(wsub(e.x, wo.x), -wsub(e.y, wo.y));
+          }
+          const int kb = (k == 0) ? M / 2 : M - k;
+          cur[PADC(k)] = xa;
+          cur[PADC(kb)] = xb;
+          const float pa = bin_power(xa), pb = bin_power(xb);
+          if (so) { so[k] = xa; so[kb] = xb; }
+          lmin = fminf(lmin, fminf(pa, pb));
+          lmax = fmaxf(lmax, fmaxf(pa, pb));
+          lsum[h] += pa + pb;
+        }
+      }
+      // powers are >= 0: their bit patterns order like the values, so one REDUX each
+      const float miny = __uint_as_float(warp_umin(__float_as_uint(lmin)));
+      const float ymax = __uint_as_float(warp_umax(__float_as_uint(lmax)));
+      sumsq = warp_sum((double)lsum[0]);
+      sumsq += warp_sum((double)lsum[1]);
+      __syncwarp();                                          // the untangled spectrum, for every lane
+      if (emit) nk = warp_peaks<LOGM>(cur, miny, ymax, prm.pkthresh, K, cbin, hist);
+    }
+    __syncthreads();                                         // A: slot t - 1 holds frame t - 1's spectrum
+
+    // ---- per-peak epilogue, freq > 0 filter, ordered write of the zero padded row
+    if (emit) {
+      const SpecPow pw{cur};
+      const double inv_2pidt = 1.0 / (prm.dt * 6.283185307179586), inv_dt = 1.0 / prm.dt;
+      const double pi_fstep = 3.141592653589793 / prm.fstep;
+      const int64_t ob = row * K;
+      int outbase = 0;
+      for (int p0 = 0; p0 < nk; p0 += 32) {
+        const int p = p0 + lane;
+        PeakVals v;
+        bool valid = false;
+        int k = 0;
+        if (p < nk) {
+          k = cbin[p];
+          valid = peak_epilogue(k, M, cur, prev, pw, prm.fbin, prm.wfbin, prm.dt, inv_2pidt, inv_dt, pi_fstep, v);
+        }
+        const unsigned m = __ballot_sync(FULL, valid);
+        const int64_t pos = ob + outbase + __popc(m & lanemask_lt());
+        outbase += __popc(m);
+        if (valid) {
+          prm.f[pos] = v.f; prm.mag[pos] = v.mag; prm.ph[pos] = v.ph;
+          prm.realph[pos] = v.realph; prm.binno[pos] = (double)k;
+          if (prm.fine_pos) {
+            double fp, fv;
+            refine_peak(k, pw, fp, fv);
+            prm.fine_pos[pos] = fp; prm.fine_val[pos] = fv;
+          }
+        }
+      }
+      for (int p = outbase + lane; p < K; p += 32) {
+        prm.f[ob + p] = 0.0; prm.mag[ob + p] = 0.0; prm.ph[ob + p] = 0.0;
+        prm.realph[ob + p] = 0.0; prm.binno[ob + p] = 0.0;
+        if (prm.fine_pos) { prm.fine_pos[ob + p] = 0.0; prm.fine_val[ob + p] = 0.0; }
+      }
+      if (lane == 0) {
+        prm.npk[row] = outbase;
+        prm.totalmag[row] = sqrt(sumsq);                     // PVAnalysis.py:210
+      }
+    }
+    __syncthreads();                                         // B: the next group overwrites this group's slots
+  }
+#undef PVK_SLOT
 }
 
 // ------------------------------------------------------------------ f0-guided analysis
@@ -1242,17 +1728,16 @@ template <int LOGM> static int launch_tables(void *tables, void *stream) {
   return PVK_OK;
 }
 
-// CTAs of analyze_kernel<LOGM> the current device holds at once (occupancy x SM count)
-template <int LOGM> static int64_t resident_ctas(int smem) {
+// CTAs of `kernel` (block of `threads`, `smem` bytes) the current device holds at once (occupancy x SM count)
+template <class Kernel> static int64_t resident_ctas(Kernel kernel, int threads, int smem) {
 #ifdef PVK_EMU
-  (void)smem;
+  (void)kernel; (void)threads; (void)smem;
   return 148 * 7;
 #else
   int dev = 0, sms = 148, occ = 1;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, analyze_kernel<LOGM>, Plan<LOGM>::T, (size_t)smem) != cudaSuccess ||
-      occ < 1) {
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, (size_t)smem) != cudaSuccess || occ < 1) {
     cudaGetLastError();
     occ = 1;
   }
@@ -1260,24 +1745,33 @@ template <int LOGM> static int64_t resident_ctas(int smem) {
 #endif
 }
 
+// nfft 1024 / 2048 run analyze_warp_kernel (one warp per frame, AW frames per CTA), every other size
+// analyze_kernel (one CTA per frame)
 template <int LOGM> static int launch_analyze(AParams prm, int64_t nclips, int run_frames, void *stream) {
-  using P = Plan<LOGM>;
-  const int smem = Smem<LOGM>::bytes(prm.npks);
+  constexpr bool warp_kernel = LOGM == 9 || LOGM == 10;
+  auto kernel = [] {
+    if constexpr (warp_kernel) return analyze_warp_kernel<LOGM>;
+    else return analyze_kernel<LOGM>;
+  }();
+  constexpr int threads = warp_kernel ? AW * 32 : Plan<LOGM>::T;
+  int smem;
+  if constexpr (warp_kernel) smem = WSmem<LOGM>::BYTES;
+  else smem = Smem<LOGM>::bytes(prm.npks);
   if (smem > 48 * 1024) {
-    if (PVK_SET_SMEM(analyze_kernel<LOGM>, smem) != 0) {
+    if (PVK_SET_SMEM(kernel, smem) != 0) {
       set_error("pvk_analyze: cannot reserve %d bytes of shared memory", smem);
       return PVK_ERR_CUDA;
     }
   }
   int64_t run = run_frames;
   if (run <= 0) {
-    // The kernel is latency bound (one CTA = one chain of dependent frames), so what matters is
-    // that every resident CTA slot is busy for the same time: size the runs so that the grid is a
-    // whole number of waves, as few as possible (every run pays one warm-up frame), with runs of
-    // 4..256 frames.
+    // The kernel is latency bound (one CTA = one chain of dependent frames, or of groups of AW
+    // frames), so what matters is that every resident CTA slot is busy for the same time: size the
+    // runs so that the grid is a whole number of waves, as few as possible (every run pays one
+    // warm-up frame), with runs of 4..256 frames.
     // Clip batches: every clip is cut into the same number of equally long runs, as many as keep the
     // grid within those waves (a clip's last run is not a short straggler that opens another wave).
-    const int64_t slots = resident_ctas<LOGM>(smem);
+    const int64_t slots = resident_ctas(kernel, threads, smem);
     const int64_t total = nclips * prm.nframes;
     const int64_t waves = (total + slots * 256 - 1) / (slots * 256);
     int64_t per_clip = slots * waves / nclips;                 // runs per clip
@@ -1291,7 +1785,7 @@ template <int LOGM> static int launch_analyze(AParams prm, int64_t nclips, int r
   prm.nruns = (prm.nframes + run - 1) / run;
   const int64_t nblk = nclips * prm.nruns;
   PVK_REQUIRE(nblk < (int64_t)2147483647, "pvk_analyze: grid too large (%lld CTAs)", (long long)nblk);
-  PVK_LAUNCH(analyze_kernel<LOGM>, dim3((unsigned)nblk), dim3(P::T), smem, stream, prm);
+  PVK_LAUNCH(kernel, dim3((unsigned)nblk), dim3(threads), smem, stream, prm);
   PVK_CHECK_LAUNCH("pvk_analyze");
   return PVK_OK;
 }
