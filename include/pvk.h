@@ -110,6 +110,10 @@ int pvk_analyze_ex(const float *x, int64_t nclips, int64_t clip_stride, int64_t 
  * partial at a clip boundary, so ONE pvk_track / pvk_track_pack / pvk_resynth over the flattened
  * [nclips * out_rows_per_clip, npks] tables links, packs and renders all clips at once, each
  * exactly like a PV of its own (ids are numbered clip after clip).
+ * fine_pos / fine_val (optional) follow the same layout, float64 [nclips, out_rows_per_clip,
+ * npks]; the kernel writes only the nframes rows of each clip, so the caller zeroes their guard
+ * rows as those of the other tables.  spec_out must be NULL unless out_rows_per_clip == nframes
+ * (PVK_ERR_ARG otherwise): the spectrum has no guard rows.
  */
 int pvk_analyze_batch(const float *x, int64_t nclips, int64_t clip_stride, int64_t nsamp,
                       const float *win_scaled, const double *fbin, const double *wfbin,

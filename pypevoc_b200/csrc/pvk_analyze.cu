@@ -1842,6 +1842,9 @@ extern "C" int pvk_analyze_batch(const float *x, int64_t nclips, int64_t clip_st
                                  double *fine_pos, double *fine_val, int64_t out_rows_per_clip, void *stream) {
   PVK_REQUIRE(out_rows_per_clip >= nframes, "pvk_analyze_batch: out_rows_per_clip=%lld < nframes=%lld",
               (long long)out_rows_per_clip, (long long)nframes);
+  PVK_REQUIRE(spec_out == nullptr || out_rows_per_clip == nframes,
+              "pvk_analyze_batch: spec_out needs out_rows_per_clip=%lld == nframes=%lld (no guard rows)",
+              (long long)out_rows_per_clip, (long long)nframes);
   const int l = log2_exact(nfft);
   PVK_REQUIRE(l >= 0 && nfft >= PVK_MIN_NFFT && nfft <= PVK_MAX_NFFT,
               "pvk_analyze: nfft=%d must be a power of two in [%d, %d]", nfft, PVK_MIN_NFFT, PVK_MAX_NFFT);

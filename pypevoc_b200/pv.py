@@ -148,9 +148,10 @@ def analyze_device(xd, sr, nfft, hop, npks, pkthresh, tb, frame0=0, nframes=None
     tensors ``f mag ph realph binno`` (float64 ``[nclips, nframes, npks]``), ``npk`` (int32),
     ``totalmag`` (float64) and optionally ``fx`` (complex64 ``[nclips, nframes, nfft/2]``);
     ``refine=True`` adds ``fine_pos`` / ``fine_val`` (PeakFinder.refine of every emitted peak,
-    PeakFinder.py:331-372).  ``out_rows`` (>= nframes; pvk_analyze_batch): the tables get
-    ``out_rows`` rows per clip, the rows beyond ``nframes`` are zero guard rows (clip batches that
-    go on to tracking / resynthesis as ONE flattened table).  Asynchronous on the current stream.
+    PeakFinder.py:331-372).  ``out_rows`` (>= nframes; pvk_analyze_batch): the tables, ``fine_pos``
+    / ``fine_val`` included, get ``out_rows`` rows per clip, the rows beyond ``nframes`` are zero
+    guard rows (clip batches that go on to tracking / resynthesis as ONE flattened table); not
+    with ``spectra``.  Asynchronous on the current stream.
     """
     L = _lib.lib()
     if xd.dim() == 1:
@@ -172,7 +173,8 @@ def analyze_device(xd, sr, nfft, hop, npks, pkthresh, tb, frame0=0, nframes=None
     assert rows >= nframes and not (spectra and rows != nframes)
     if out is None:
         out = {}
-        for k in ("f", "mag", "ph", "realph", "binno"):
+        # fine_pos / fine_val have the rows of the tables, guard rows included (pvk.h)
+        for k in ("f", "mag", "ph", "realph", "binno") + (("fine_pos", "fine_val") if refine else ()):
             out[k] = torch.empty((nclips, rows, npks), dtype=torch.float64, device=dev)
         out["npk"] = torch.empty((nclips, rows), dtype=torch.int32, device=dev)
         out["totalmag"] = torch.empty((nclips, rows), dtype=torch.float64, device=dev)
@@ -181,8 +183,8 @@ def analyze_device(xd, sr, nfft, hop, npks, pkthresh, tb, frame0=0, nframes=None
                 v[:, nframes:].zero_()
     spec = torch.empty((nclips, nframes, nfft // 2), dtype=torch.complex64, device=dev) if spectra else None
     if refine and "fine_pos" not in out:
-        out["fine_pos"] = torch.empty((nclips, nframes, npks), dtype=torch.float64, device=dev)
-        out["fine_val"] = torch.empty((nclips, nframes, npks), dtype=torch.float64, device=dev)
+        out["fine_pos"] = torch.zeros((nclips, rows, npks), dtype=torch.float64, device=dev)
+        out["fine_val"] = torch.zeros((nclips, rows, npks), dtype=torch.float64, device=dev)
     with torch.cuda.device(dev):
         _lib.check(L.pvk_analyze_batch(
             _ptr(xd), nclips, xd.stride(0), nsamp, _ptr(dtb["win"]), _ptr(dtb["fbin"]), _ptr(dtb["wfbin"]),

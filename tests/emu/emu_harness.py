@@ -58,8 +58,8 @@ def host_tables(sr, nfft, hop, wind=np.hanning):
 
 def analyze(x, sr, nfft, hop, npks, pkthresh=0.005, nclips=1, frame0=0, nframes=None,
             prev_zero=1, run_frames=0, spectra=False, wind=np.hanning, refine=False, out_rows=None):
-    """``out_rows`` (>= nframes): pvk_analyze_batch -- tables [nclips, out_rows, npks] whose rows beyond
-    nframes are zero guard rows."""
+    """``out_rows`` (>= nframes): pvk_analyze_batch -- tables [nclips, out_rows, npks] (fine_pos /
+    fine_val with ``refine``) whose rows beyond nframes are zero guard rows."""
     L = lib()
     x = np.ascontiguousarray(x, dtype=np.float32)
     if x.ndim == 1:
@@ -80,9 +80,10 @@ def analyze(x, sr, nfft, hop, npks, pkthresh=0.005, nclips=1, frame0=0, nframes=
     totalmag = np.full((nclips, nframes), np.nan)
     spec = np.zeros((nclips, nframes, nfft // 2, 2), dtype=np.float32) if spectra else None
     if out_rows is not None:
-        assert not spectra and not refine and out_rows >= nframes
+        assert not spectra and out_rows >= nframes
         shp = (nclips, out_rows, npks)
-        out = {k: np.full(shp, np.nan) for k in ("f", "mag", "ph", "realph", "binno")}
+        names = ("f", "mag", "ph", "realph", "binno") + (("fine_pos", "fine_val") if refine else ())
+        out = {k: np.full(shp, np.nan) for k in names}
         for v in out.values():
             v[:, nframes:] = 0.0
         npk = np.zeros((nclips, out_rows), dtype=np.int32)
@@ -91,7 +92,7 @@ def analyze(x, sr, nfft, hop, npks, pkthresh=0.005, nclips=1, frame0=0, nframes=
                                   ptr(tb["wfbin"]), ptr(tables), nfft, hop, npks, pkthresh, tb["dt"], tb["fstep"],
                                   frame0, nframes, prev_zero, run_frames, ptr(out["f"]), ptr(out["mag"]),
                                   ptr(out["ph"]), ptr(out["realph"]), ptr(out["binno"]), ptr(npk), ptr(totalmag),
-                                  None, None, None, out_rows, None))
+                                  None, ptr(out.get("fine_pos")), ptr(out.get("fine_val")), out_rows, None))
     elif refine:
         out["fine_pos"], out["fine_val"] = np.full(shp, np.nan), np.full(shp, np.nan)
         check(L.pvk_analyze_ex(ptr(x), nclips, x.strides[0] // 4, nsamp, ptr(tb["win_scaled"]), ptr(tb["fbin"]),

@@ -58,6 +58,21 @@ def test_argument_validation_without_gpu(libpath):
     assert st == 1 and b"npks" in lib.pvk_last_error()
 
 
+def test_analyze_batch_rejects_spectra_with_guard_rows(libpath):
+    """spec_out has no guard rows: with out_rows_per_clip > nframes the batch call refuses it before
+    any CUDA call; without spec_out the same arguments pass that check."""
+    from pypevoc_b200 import _lib
+    lib = _lib.declare(ctypes.CDLL(libpath))
+    spec = np.zeros((2, 10, 512, 2), dtype=np.float32)
+    p = spec.ctypes.data_as(ctypes.c_void_p)
+    st = lib.pvk_analyze_batch(None, 2, 20000, 20000, None, None, None, None, 1024, 256, 20, 0.005, 0.0, 0.0, 0, 10,
+                               1, 0, None, None, None, None, None, None, None, p, None, None, 13, None)
+    assert st == 1 and b"spec_out" in lib.pvk_last_error() and b"out_rows_per_clip=13" in lib.pvk_last_error()
+    st = lib.pvk_analyze_batch(None, 2, 20000, 20000, None, None, None, None, 1024, 256, 20, 0.005, 0.0, 0.0, 0, 10,
+                               1, 0, None, None, None, None, None, None, None, None, None, None, 13, None)
+    assert st == 1 and b"NULL pointer" in lib.pvk_last_error()
+
+
 def test_product_fails_loudly_without_gpu_or_library(monkeypatch):
     import torch
     import pypevoc_b200
