@@ -256,6 +256,29 @@ int pvk_track_pack_dev(const double *f, const double *mag, const double *ph, con
                        double *pf, double *pmag, double *pph, double *prealph, void *workspace,
                        int64_t workspace_bytes, void *stream);
 
+/* Renumber a table remapped by any map, in any order (DESIGN.md 4.3, "Remap"): tid_map [nrows_out, npks]
+ * holds the SOURCE ids of pvk_time_map's tid_out under the map tmap (nrows_out float64 frames in
+ * [0, nframes - 1]), and a source partial read backwards or across a jump covers several runs of
+ * consecutive output rows.  Slot (b, c) holding source partial v continues v's run when b > 0 and
+ * tstart[v] <= floor(tmap[b - 1]) <= tstart[v] + tlen[v] - 1; otherwise it starts a new run.  Every run
+ * becomes one partial, numbered in ascending order of (first output row, source id):
+ *   link_out  int32 [nrows_out, npks], pvk_track's encoding: the column of the slot in row b - 1 (>= 0),
+ *             -1 = not a point, <= -2 = new run of rank -2 - link among the row's new runs by source id
+ *   tid_out   int32 [nrows_out, npks]: run id per slot, -1 = not a point
+ *   ntracks_out  int32 [1]: number of runs
+ * The result is a valid track table: pvk_track_stats counts it and pvk_track_pack packs it with the
+ * tables of pvk_time_map.  With a non-decreasing map it is the time map's table with the partials it
+ * skips removed and the ids compacted in order.
+ *   tid_src, nframes, ntracks_src, tstart, tlen, toff   the source table [nframes, npks] and its pack
+ *   workspace    pvk_track_relink_workspace_bytes(nframes, npks, nrows_out) bytes
+ * Checks sizes, npks, pointers and nrows_out * npks < 2^31 before any CUDA call; allocates nothing. */
+int64_t pvk_track_relink_workspace_bytes(int64_t nframes, int npks, int64_t nrows_out);
+
+int pvk_track_relink(const int32_t *tid_src, int64_t nframes, int npks, int64_t ntracks_src,
+                     const int32_t *tstart, const int32_t *tlen, const int64_t *toff, const int32_t *tid_map,
+                     const double *tmap, int64_t nrows_out, int32_t *tid_out, int32_t *link_out,
+                     int32_t *ntracks_out, void *workspace, int64_t workspace_bytes, void *stream);
+
 /* ------------------------------------------------------------------ segment sharding
  * A long signal split into per-GPU frame ranges is linked per segment (pvk_track on the
  * segment's window of rows: `own0` halo rows, then `nown` own rows, then more halo rows); these

@@ -39,7 +39,9 @@ SIGNATURES = {
     "pvk_track_pack_workspace_bytes": (_i64, [_i64]),
     "pvk_track_pack": (_i, [_p, _p, _p, _p, _p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p]),
     "pvk_track_pack_dev": (_i, [_p, _p, _p, _p, _p, _i64, _i, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _p]),
-    "pvk_segment_summary": (_i, [_p, _i, _i64, _i64, _i64, _p, _p]),
+    "pvk_track_relink_workspace_bytes": (_i64, [_i64, _i, _i64]),
+    "pvk_track_relink": (_i, [_p, _i64, _i, _i64, _p, _p, _p, _p, _p, _i64, _p, _p, _p, _p, _i64, _p]),
+    "pvk_segment_summary":(_i, [_p, _i, _i64, _i64, _i64, _p, _p]),
     "pvk_segment_resolve": (_i, [_p, _i, _i, _i, _p, _i64, _p, _p, _p]),
     "pvk_segment_rename": (_i, [_p, _i64, _p, _p, _p, _p]),
     "pvk_segment_rename_push": (_i, [_p, _i64, _p, _p, _p, _i, _i64, _p]),

@@ -1177,6 +1177,88 @@ __global__ void clip_spans_kernel(const int32_t *__restrict__ tstart, const int3
   }
 }
 
+// ------------------------------------------------------------------ relink (DESIGN.md 4.3, "Remap")
+// A table remapped onto output rows by any map tau (pvk_time_map) holds source ids, and a source partial
+// read backwards or across a jump covers several runs of consecutive output rows.  The relink gives every
+// run its own id, in pvk_track's link encoding, and the scan and resolve of pvk_track number the runs.
+//
+// col[p] = column of packed point p of the source table: with it, the column of partial v in output row
+// b - 1 (= source row floor(tau[b - 1])) is one gather instead of a search of that row.
+__global__ void relink_cols_kernel(const int32_t *__restrict__ tid, int64_t n, int K, int64_t ntracks,
+                                   const int32_t *__restrict__ tstart, const int32_t *__restrict__ tlen,
+                                   const int64_t *__restrict__ toff, int32_t *__restrict__ col) {
+  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
+    const int v = tid[e];
+    if (v < 0 || v >= ntracks) continue;
+    const int64_t i = e / K;
+    const int64_t k = i - tstart[v];
+    if (k >= 0 && k < tlen[v]) col[toff[v] + k] = (int32_t)(e - i * K);
+  }
+}
+
+// One warp per output row b, lanes over columns.  Slot (b, c) holding source partial v continues v's
+// run when output row b - 1 holds v, i.e. tstart[v] <= floor(tau[b - 1]) <= end[v]: link = v's column
+// there.  Otherwise it starts a run: link = -2 - rank, rank = number of the row's new runs with a smaller
+// source id (ids are distinct within a row), so the scan numbers runs by (first output row, source id).
+// Shared memory per warp: the row's source ids [K] | one bit per column of a new run [32 words].  Cost per
+// row: K coalesced id reads, three gathers and one `col` gather per point, and nnew^2 / 32 shared reads per
+// lane for the ranks (nnew = new runs in the row: all points in row 0 and after a jump, few elsewhere).
+// The launch bound's 4 CTAs per SM (44 registers) keeps ptxas from holding the kernel at 32 and spilling.
+constexpr int RELINK_THREADS = 256;
+
+__host__ __device__ constexpr int relink_smem_per_warp(int K) { return (K + 32) * 4; }
+
+__global__ void __launch_bounds__(RELINK_THREADS, 4) track_relink_kernel(
+    const int32_t *__restrict__ tid_map, const double *__restrict__ tmap, int64_t B, int64_t F, int K, int64_t ntracks,
+    const int32_t *__restrict__ tstart, const int32_t *__restrict__ tlen, const int64_t *__restrict__ toff,
+    const int32_t *__restrict__ col, int32_t *__restrict__ link, int32_t *__restrict__ newcount) {
+  PVK_SMEM(smem);
+  const int lane = lane_id(), warp = warp_id();
+  int *ids = reinterpret_cast<int *>(smem) + (size_t)warp * (K + 32);
+  unsigned *bits = reinterpret_cast<unsigned *>(ids + K);
+  const int nw = (int)(gridDim.x * (blockDim.x >> 5));              // warps in the grid (<= 148 * 16 * 8)
+  for (int64_t b = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp; b < B; b += nw) {
+    const double tp = b > 0 ? tmap[b - 1] : -1.0;
+    const int64_t ip = tp >= 0.0 && tp <= (double)(F - 1) ? (int64_t)floor(tp) : -1;   // -1: no row before
+    int32_t *lrow = link + b * K;
+    int nnew = 0;
+    for (int c0 = 0; c0 < K; c0 += 32) {
+      const int c = c0 + lane;
+      bool fresh = false;
+      if (c < K) {
+        int v = tid_map[b * K + c];
+        int lk = LINK_NONE;
+        if (v >= 0 && v < ntracks) {
+          const int64_t k = ip - tstart[v];
+          if (ip >= 0 && k >= 0 && k < tlen[v]) lk = col[toff[v] + k];
+          else fresh = true;
+        } else {
+          v = -1;
+        }
+        ids[c] = v;
+        if (!fresh) lrow[c] = lk;
+      }
+      const unsigned m = __ballot_sync(FULL, fresh);
+      if (lane == 0) bits[c0 >> 5] = m;
+      nnew += __popc(m);
+    }
+    __syncwarp();
+    if (nnew > 0) {
+      const int nword = (K + 31) >> 5;
+      for (int c = lane; c < K; c += 32) {
+        if (!((bits[c >> 5] >> (c & 31)) & 1u)) continue;
+        const int v = ids[c];
+        int rank = 0;
+        for (int w = 0; w < nword; ++w)
+          for (unsigned rem = bits[w]; rem; rem &= rem - 1u) rank += ids[32 * w + __ffs((int)rem) - 1] < v ? 1 : 0;
+        lrow[c] = -2 - rank;
+      }
+    }
+    if (lane == 0) newcount[b] = nnew;
+    __syncwarp();
+  }
+}
+
 static inline int grid_for(int64_t n, int block) {
   int64_t g = (n + block - 1) / block;
   const int64_t cap = 148 * 16;
@@ -1203,6 +1285,93 @@ extern "C" int64_t pvk_track_workspace_bytes(int64_t nclips, int64_t nframes, in
   return align_up(rows * 4, 256) * 2 + resolve_levels_bytes(rows, npks) +
          align_up(nclips * scan_tiles(nframes) * 8, 256) + 256;
 }
+
+// The numbering half of pvk_track, shared with pvk_track_relink: the per-clip exclusive scan of the
+// rows' new-partial counts (newcount -> base, ntracks), then the chain resolution that turns link + base
+// into ids (tid).  `name` is the export's name for error messages.
+#define PVK_CHECK_STAGE(stage)                                                                      \
+  do {                                                                                              \
+    char _what[64];                                                                                 \
+    snprintf(_what, sizeof _what, "%s(" stage ")", name);                                          \
+    PVK_CHECK_LAUNCH(_what);                                                                        \
+  } while (0)
+
+static int track_number(const int32_t *link, int32_t *newcount, int32_t *base, unsigned char *levels, long long *tsum,
+                        int64_t nclips, int64_t nframes, int K, int32_t *tid, int32_t *ntracks, void *stream,
+                        const char *name) {
+  const int64_t rows = nclips * nframes;
+  {
+    const int64_t nt = scan_tiles(nframes);
+    PVK_REQUIRE(nclips <= 65535, "%s: at most 65535 clips per call (got %lld)", name, (long long)nclips);
+    PVK_LAUNCH(scan_tile_sums_kernel, dim3((unsigned)nt, (unsigned)nclips), dim3(SCAN_BD), SCAN_SMEM, stream, newcount, nframes,
+               nframes, (const int32_t *)nullptr, nt, tsum);
+    PVK_LAUNCH(scan_tile_apply_kernel<int32_t>, dim3((unsigned)nt, (unsigned)nclips), dim3(SCAN_BD), SCAN_SMEM, stream, newcount,
+               nframes, nframes, (const int32_t *)nullptr, nt, tsum, base, nframes, ntracks, 0);
+    PVK_CHECK_STAGE("scan");
+  }
+  {
+    // ---- chain resolution: level 1 turns link + base into ids chunk by chunk, the chunks' last rows
+    //      form the next level, ... the last level is resolved by one CTA, then the references left in
+    //      every level are replaced top-down.  The first row of every clip holds no reference.
+    const int RT = track_tile_rows(K);
+    const size_t per_warp = (size_t)resolve_tile_ints(K, RT) * 4;
+    int W = (int)((64 * 1024) / per_warp);
+    if (W > 4) W = 4;
+    if (W < 1) W = 1;
+    const size_t csm = per_warp * W;
+    if (csm > 48 * 1024 && (PVK_SET_SMEM(resolve_chunk_kernel<true>, (int)csm) != 0 ||
+                            PVK_SET_SMEM(resolve_chunk_kernel<false>, (int)csm) != 0)) {
+      set_error("%s: cannot reserve %d bytes of shared memory", name, (int)csm);
+      return PVK_ERR_CUDA;
+    }
+    int32_t *tab[16];
+    int64_t len[16];
+    int nl = 0;
+    tab[0] = tid; len[0] = rows;
+    unsigned char *lp = levels;
+    {
+      const int64_t nch = (rows + RES_CHUNK - 1) / RES_CHUNK;
+      tab[1] = reinterpret_cast<int32_t *>(lp); len[1] = nch;
+      lp += align_up(nch * K * 4, 256);
+      PVK_LAUNCH(resolve_chunk_kernel<true>, dim3((unsigned)((nch + W - 1) / W)), dim3(W * 32), csm, stream, link, base,
+                 tid, rows, K, RT, tab[1]);
+      PVK_CHECK_STAGE("chunk");
+      nl = 1;
+    }
+    if (len[1] > 1) {
+      while (len[nl] > RES_MID) {
+        const int64_t nch = (len[nl] + RES_CHUNK - 1) / RES_CHUNK;
+        tab[nl + 1] = reinterpret_cast<int32_t *>(lp); len[nl + 1] = nch;
+        lp += align_up(nch * K * 4, 256);
+        PVK_LAUNCH(resolve_chunk_kernel<false>, dim3((unsigned)((nch + W - 1) / W)), dim3(W * 32), csm, stream,
+                   (const int32_t *)nullptr, (const int32_t *)nullptr, tab[nl], len[nl], K, RT, tab[nl + 1]);
+        PVK_CHECK_STAGE("chunk");
+        ++nl;
+      }
+      {
+        int NW = K > 512 ? 8 : 16;
+        int RTm = RT;
+        while (RTm > 1 && ((size_t)NW * K + 4 + (size_t)NW * resolve_tile_ints(K, RTm)) * 4 > 160 * 1024) RTm >>= 1;
+        const size_t msm = ((((size_t)NW * K + 3) & ~(size_t)3) + (size_t)NW * resolve_tile_ints(K, RTm)) * 4;
+        if (msm > 48 * 1024 && PVK_SET_SMEM(resolve_mid_kernel, (int)msm) != 0) {
+          set_error("%s: cannot reserve %d bytes of shared memory", name, (int)msm);
+          return PVK_ERR_CUDA;
+        }
+        PVK_LAUNCH(resolve_mid_kernel, dim3(1), dim3(NW * 32), msm, stream, tab[nl], len[nl], K, RTm);
+        PVK_CHECK_STAGE("mid");
+      }
+      for (int l = nl - 1; l >= 0; --l) {
+        int64_t g = (len[l] + RES_CHUNK - 1) / RES_CHUNK - 1;
+        if (g < 1) continue;
+        if (g > 148 * 32) g = 148 * 32;
+        PVK_LAUNCH(resolve_fix_kernel, dim3((unsigned)g), dim3(128), 0, stream, tab[l], len[l], K, tab[l + 1]);
+        PVK_CHECK_STAGE("fix");
+      }
+    }
+  }
+  return PVK_OK;
+}
+#undef PVK_CHECK_STAGE
 
 extern "C" int pvk_track(const double *f, const double *mag, int64_t nclips, int64_t nframes, int npks,
                          double maxpitchjmp, int32_t *tid, int32_t *link, int32_t *ntracks,
@@ -1281,76 +1450,58 @@ extern "C" int pvk_track(const double *f, const double *mag, int64_t nclips, int
     }
     PVK_CHECK_LAUNCH("pvk_track(link)");
   }
-  {
-    const int64_t nt = scan_tiles(nframes);
-    PVK_REQUIRE(nclips <= 65535, "pvk_track: at most 65535 clips per call (got %lld)", (long long)nclips);
-    PVK_LAUNCH(scan_tile_sums_kernel, dim3((unsigned)nt, (unsigned)nclips), dim3(SCAN_BD), SCAN_SMEM, stream, newcount, nframes,
-               nframes, (const int32_t *)nullptr, nt, tsum);
-    PVK_LAUNCH(scan_tile_apply_kernel<int32_t>, dim3((unsigned)nt, (unsigned)nclips), dim3(SCAN_BD), SCAN_SMEM, stream, newcount,
-               nframes, nframes, (const int32_t *)nullptr, nt, tsum, base, nframes, ntracks, 0);
-    PVK_CHECK_LAUNCH("pvk_track(scan)");
+  return track_number(link, newcount, base, levels, tsum, nclips, nframes, K, tid, ntracks, stream, "pvk_track");
+}
+
+// pvk_track's workspace for one clip of nrows_out rows, then the source column of every packed point
+extern "C" int64_t pvk_track_relink_workspace_bytes(int64_t nframes, int npks, int64_t nrows_out) {
+  if (nframes < 0 || npks < 1 || nrows_out < 0) return -1;
+  return pvk_track_workspace_bytes(1, nrows_out, npks) + align_up(nframes * npks * 4, 256);
+}
+
+extern "C" int pvk_track_relink(const int32_t *tid_src, int64_t nframes, int npks, int64_t ntracks_src,
+                                const int32_t *tstart, const int32_t *tlen, const int64_t *toff, const int32_t *tid_map,
+                                const double *tmap, int64_t nrows_out, int32_t *tid_out, int32_t *link_out,
+                                int32_t *ntracks_out, void *workspace, int64_t workspace_bytes, void *stream) {
+  PVK_REQUIRE(npks >= 1 && npks <= PVK_MAX_NPKS, "pvk_track_relink: npks=%d must be in [1, %d]", npks, PVK_MAX_NPKS);
+  PVK_REQUIRE(nframes >= 0 && ntracks_src >= 0 && nrows_out >= 0, "pvk_track_relink: negative sizes");
+  PVK_REQUIRE(ntracks_out != nullptr, "pvk_track_relink: ntracks_out is NULL");
+  PVK_REQUIRE(nrows_out * (int64_t)npks < (int64_t)2147483647 && nframes * (int64_t)npks < (int64_t)2147483647,
+              "pvk_track_relink: nrows_out*npks and nframes*npks must be < 2^31");
+  if (nrows_out == 0) {
+    cudaMemsetAsync(ntracks_out, 0, 4, (cudaStream_t)stream);
+    return PVK_OK;
+  }
+  PVK_REQUIRE(nframes >= 1, "pvk_track_relink: a remap needs a source table with at least one frame row");
+  PVK_REQUIRE(tid_src && tid_map && tmap && tid_out && link_out && workspace &&
+                  (ntracks_src == 0 || (tstart && tlen && toff)),
+              "pvk_track_relink: NULL pointer argument");
+  const int64_t need = pvk_track_relink_workspace_bytes(nframes, npks, nrows_out);
+  PVK_REQUIRE(workspace_bytes >= need, "pvk_track_relink: workspace too small (%lld < %lld bytes)",
+              (long long)workspace_bytes, (long long)need);
+  const int K = npks;
+  const int64_t B = nrows_out;
+  unsigned char *ws = reinterpret_cast<unsigned char *>(workspace);
+  int32_t *newcount = reinterpret_cast<int32_t *>(ws);
+  int32_t *base = reinterpret_cast<int32_t *>(ws + align_up(B * 4, 256));
+  unsigned char *levels = ws + 2 * align_up(B * 4, 256);
+  long long *tsum = reinterpret_cast<long long *>(levels + resolve_levels_bytes(B, npks));
+  int32_t *col = reinterpret_cast<int32_t *>(ws + pvk_track_workspace_bytes(1, B, npks));
+  if (ntracks_src > 0) {
+    PVK_LAUNCH(relink_cols_kernel, dim3(grid_for(nframes * K, 256)), dim3(256), 0, stream, tid_src, nframes * K, K,
+               ntracks_src, tstart, tlen, toff, col);
+    PVK_CHECK_LAUNCH("pvk_track_relink(cols)");
   }
   {
-    // ---- chain resolution: level 1 turns link + base into ids chunk by chunk, the chunks' last rows
-    //      form the next level, ... the last level is resolved by one CTA, then the references left in
-    //      every level are replaced top-down.  The first row of every clip holds no reference.
-    const int RT = track_tile_rows(K);
-    const size_t per_warp = (size_t)resolve_tile_ints(K, RT) * 4;
-    int W = (int)((64 * 1024) / per_warp);
-    if (W > 4) W = 4;
-    if (W < 1) W = 1;
-    const size_t csm = per_warp * W;
-    if (csm > 48 * 1024 && (PVK_SET_SMEM(resolve_chunk_kernel<true>, (int)csm) != 0 ||
-                            PVK_SET_SMEM(resolve_chunk_kernel<false>, (int)csm) != 0)) {
-      set_error("pvk_track: cannot reserve %d bytes of shared memory", (int)csm);
-      return PVK_ERR_CUDA;
-    }
-    int32_t *tab[16];
-    int64_t len[16];
-    int nl = 0;
-    tab[0] = tid; len[0] = rows;
-    unsigned char *lp = levels;
-    {
-      const int64_t nch = (rows + RES_CHUNK - 1) / RES_CHUNK;
-      tab[1] = reinterpret_cast<int32_t *>(lp); len[1] = nch;
-      lp += align_up(nch * K * 4, 256);
-      PVK_LAUNCH(resolve_chunk_kernel<true>, dim3((unsigned)((nch + W - 1) / W)), dim3(W * 32), csm, stream, link, base,
-                 tid, rows, K, RT, tab[1]);
-      PVK_CHECK_LAUNCH("pvk_track(chunk)");
-      nl = 1;
-    }
-    if (len[1] > 1) {
-      while (len[nl] > RES_MID) {
-        const int64_t nch = (len[nl] + RES_CHUNK - 1) / RES_CHUNK;
-        tab[nl + 1] = reinterpret_cast<int32_t *>(lp); len[nl + 1] = nch;
-        lp += align_up(nch * K * 4, 256);
-        PVK_LAUNCH(resolve_chunk_kernel<false>, dim3((unsigned)((nch + W - 1) / W)), dim3(W * 32), csm, stream,
-                   (const int32_t *)nullptr, (const int32_t *)nullptr, tab[nl], len[nl], K, RT, tab[nl + 1]);
-        PVK_CHECK_LAUNCH("pvk_track(chunk)");
-        ++nl;
-      }
-      {
-        int NW = K > 512 ? 8 : 16;
-        int RTm = RT;
-        while (RTm > 1 && ((size_t)NW * K + 4 + (size_t)NW * resolve_tile_ints(K, RTm)) * 4 > 160 * 1024) RTm >>= 1;
-        const size_t msm = ((((size_t)NW * K + 3) & ~(size_t)3) + (size_t)NW * resolve_tile_ints(K, RTm)) * 4;
-        if (msm > 48 * 1024 && PVK_SET_SMEM(resolve_mid_kernel, (int)msm) != 0) {
-          set_error("pvk_track: cannot reserve %d bytes of shared memory", (int)msm);
-          return PVK_ERR_CUDA;
-        }
-        PVK_LAUNCH(resolve_mid_kernel, dim3(1), dim3(NW * 32), msm, stream, tab[nl], len[nl], K, RTm);
-        PVK_CHECK_LAUNCH("pvk_track(mid)");
-      }
-      for (int l = nl - 1; l >= 0; --l) {
-        int64_t g = (len[l] + RES_CHUNK - 1) / RES_CHUNK - 1;
-        if (g < 1) continue;
-        if (g > 148 * 32) g = 148 * 32;
-        PVK_LAUNCH(resolve_fix_kernel, dim3((unsigned)g), dim3(128), 0, stream, tab[l], len[l], K, tab[l + 1]);
-        PVK_CHECK_LAUNCH("pvk_track(fix)");
-      }
-    }
+    const int W = RELINK_THREADS / 32;
+    const int smem = W * relink_smem_per_warp(K);
+    const int64_t g = (B + W - 1) / W < 148 * 16 ? (B + W - 1) / W : 148 * 16;
+    PVK_LAUNCH(track_relink_kernel, dim3((unsigned)g), dim3(RELINK_THREADS), smem, stream, tid_map, tmap, B, nframes, K,
+               ntracks_src, tstart, tlen, toff, col, link_out, newcount);
+    PVK_CHECK_LAUNCH("pvk_track_relink(link)");
   }
-  return PVK_OK;
+  return track_number(link_out, newcount, base, levels, tsum, 1, B, K, tid_out, ntracks_out, stream,
+                      "pvk_track_relink");
 }
 
 extern "C" int pvk_track_spans(const int32_t *tid, int64_t nframes, int npks, int64_t ntracks, int32_t *tstart,

@@ -600,11 +600,12 @@ def track_pack_resynth_device(fd, magd, phd, realphd, sr, hop, nfft, hop_an, edg
     return tr, _pack_sliced(raw, nt, npts), out[:nout]
 
 
-def time_map_values(time_map, nframes):
+def time_map_values(time_map, nframes, monotone=True):
     """Checked time map of a table of ``nframes`` frame rows: a float64 numpy copy of a 1-D array,
     sequence or torch tensor of at least one real value, every value finite, in ``[0, nframes - 1]``,
     and non-decreasing (equal neighbours hold the sound: a freeze).  Output block ``b`` renders the
-    partials as they are at the fractional analysis frame ``time_map[b]`` (DESIGN.md 4.3, "Time map")."""
+    partials as they are at the fractional analysis frame ``time_map[b]`` (DESIGN.md 4.3, "Time map").
+    ``monotone=False`` skips only the non-decreasing check (SinSum.remap() takes maps in any order)."""
     if isinstance(time_map, torch.Tensor):
         if time_map.dtype == torch.bool or time_map.is_complex():
             raise TypeError("a time_map must hold real numbers, not %s" % time_map.dtype)
@@ -623,7 +624,7 @@ def time_map_values(time_map, nframes):
     if a[0] < 0.0 or a.max() > nframes - 1:
         raise ValueError("the values of a time_map must lie in [0, %d] (the frame rows of the partials)"
                          % (nframes - 1))
-    if np.any(np.diff(a) < 0.0):
+    if monotone and np.any(np.diff(a) < 0.0):
         raise ValueError("a time_map must be non-decreasing (a partial may only be read forwards)")
     return a
 
@@ -651,6 +652,41 @@ def time_map_device(tid, pk, tmap_dev):
     _, npts, last = track_counts(dict(stats=stats))
     pk_m = pack_device(f_m, mag_m, realph_m, realph_m, tid_m, None, nt, npts=npts)
     return tid_m, pk_m, last
+
+
+def remap_device(tid, pk, tmap_dev):
+    """The partials ``tid`` ``[F, K]`` / ``pk`` (pack_device()) read along ``tmap_dev`` (float64 CUDA tensor
+    of frame positions in any order, checked by time_map_values(monotone=False)): pvk_time_map, then
+    pvk_track_relink, which splits every source partial into its runs of consecutive output rows and
+    numbers the runs, then pvk_track_stats with ONE 24-byte read-back, then the pack (DESIGN.md 4.3,
+    "Remap").  Returns ``(tables, tracks, pk')``: the frame tables ``f, mag, ph, realph`` ``[B, K]`` (ph =
+    realph), the tracks ``tid, link, ntracks, ntracks_dev, npts, max_end`` and their pack."""
+    L = _lib.lib()
+    dev = tid.device
+    F, K = tid.shape
+    B = int(tmap_dev.numel())
+    nt = int(pk["tstart"].shape[0])
+    tid_m = torch.empty((B, K), dtype=torch.int32, device=dev)
+    f_m, mag_m, realph_m = (torch.empty((B, K), dtype=torch.float64, device=dev) for _ in range(3))
+    tid_r = torch.empty((B, K), dtype=torch.int32, device=dev)
+    link_r = torch.empty((B, K), dtype=torch.int32, device=dev)
+    ntd = torch.empty((1,), dtype=torch.int32, device=dev)
+    stats = torch.empty((3, 1), dtype=torch.int64, device=dev)
+    wsb = int(L.pvk_track_relink_workspace_bytes(F, K, B))
+    ws = torch.empty(max(wsb, 8), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(L.pvk_time_map(_ptr(tid), F, K, nt, _ptr(pk["tstart"]), _ptr(pk["tlen"]), _ptr(pk["toff"]),
+                                  _ptr(pk["pf"]), _ptr(pk["pmag"]), _ptr(pk["prealph"]), _ptr(tmap_dev), B,
+                                  _ptr(tid_m), _ptr(f_m), _ptr(mag_m), _ptr(realph_m), _stream()), "pvk_time_map")
+        _lib.check(L.pvk_track_relink(_ptr(tid), F, K, nt, _ptr(pk["tstart"]), _ptr(pk["tlen"]), _ptr(pk["toff"]),
+                                      _ptr(tid_m), _ptr(tmap_dev), B, _ptr(tid_r), _ptr(link_r), _ptr(ntd), _ptr(ws),
+                                      wsb, _stream()), "pvk_track_relink")
+        _lib.check(L.pvk_track_stats(_ptr(tid_r), _ptr(ntd), 1, B, K, _ptr(stats), _stream()), "pvk_track_stats")
+    nt_r, npts, last = track_counts(dict(stats=stats))
+    pk_r = pack_device(f_m, mag_m, realph_m, realph_m, tid_r, None, nt_r, npts=npts)
+    tables = dict(f=f_m, mag=mag_m, ph=realph_m, realph=realph_m)
+    tracks = dict(tid=tid_r, link=link_r, ntracks=nt_r, ntracks_dev=ntd, npts=npts, max_end=last)
+    return tables, tracks, pk_r
 
 
 def spans_device(tid, ntracks):
@@ -1667,6 +1703,8 @@ class _PartialList(object):
 
 
 class SinSum(object):
+    _remapped = False            # made by remap(): the analysed phases do not belong to its rows
+
     def __init__(self, sr, nfft=1024, hop=512, device=None):
         '''
         Sine sum object (PVAnalysis.py:797-817): a sound decomposed in a sum of quasi-sine
@@ -1829,7 +1867,11 @@ class SinSum(object):
         ``to_host=False`` returns the CUDA tensor instead of a numpy array.  ``hostbuf`` (a dict,
         reused across calls): render in ``chunks`` block ranges and download each finished range
         into the pinned tensor ``hostbuf['w']`` while the next one is rendered; returns a numpy view
-        of it (valid until the next call with the same ``hostbuf``)."""
+        of it (valid until the next call with the same ``hostbuf``).
+        A SinSum made by remap() needs ``phase_preserve=False``."""
+        if self._remapped and phase_preserve:
+            raise ValueError("a remapped SinSum needs phase_preserve=False: analysed phases read along a new path "
+                             "mean nothing")
         nframes = tau = None
         if _is_curve(fscale) or _is_curve(formant_shift) or time_map is not None:
             if self._trk is None:
@@ -1880,6 +1922,33 @@ class SinSum(object):
         out = resynth_device(tr["tid"], pk, sr, int(hop), self.nfft, self.hop, edge=edge, minframes=minframes,
                              max_end=tr.get("max_end"), **mode)
         return out.cpu().numpy() if to_host else out
+
+    def remap(self, time_map):
+        """A new SinSum whose frame row ``b`` is this one read at the fractional frame ``time_map[b]``: a 1-D
+        array of ``B >= 1`` finite frame positions in ``[0, nframes - 1]`` in ANY order, so that playback
+        may reverse (``np.arange(nframes - 1, -1, -1.)``), loop, ping-pong or scrub.  The rows are those of
+        ``synth(time_map=...)`` (frequency and magnitude interpolated between neighbouring frames, realph
+        of the lower one); a source partial read backwards or across a jump comes apart into runs of
+        consecutive rows, and every run is one partial of the result, numbered by (first row, source id).
+        A partial present on both sides of a jump stays one partial: its phase stays continuous and its
+        frequency steps.  For a non-decreasing map, ``ss.remap(tau).synth(..., phase_preserve=False)``
+        renders exactly ``ss.synth(..., phase_preserve=False, time_map=tau)``.  The result renders with
+        ``phase_preserve=False`` only; ``fscale`` / ``formant_shift`` curves then have one value per row
+        of the result (``B``).  This SinSum does not change (DESIGN.md 4.3, "Remap")."""
+        if self._trk is None:
+            self._ensure_tables()
+        nframes = int((self._trk["tid"] if self._trk is not None else self._tables["f"]).shape[0])
+        tau = time_map_values(time_map, nframes, monotone=False)
+        pk = self._ensure_packed()
+        tables, tracks, pk_r = remap_device(self._trk["tid"], pk, torch.from_numpy(tau).to(self._dev))
+        ss = SinSum(self.sr, self.nfft, self.hop, device=self._dev)
+        ss._set_device_tables(tables["f"], tables["mag"], tables["ph"], tables["realph"])
+        ss._set_device_tracks(tracks["tid"], tracks["link"], tracks["ntracks"])
+        ss._trk.update(ntracks_dev=tracks["ntracks_dev"], npts=tracks["npts"], max_end=tracks["max_end"])
+        ss._pk = pk_r
+        ss._maxpitchjmp = self._maxpitchjmp
+        ss._remapped = True
+        return ss
 
     def _synth_mapped(self, tau, sr, hop, edge, minframes, to_host, hostbuf, chunks, phase_preserve=False, fscale=1.0,
                       formant=None):

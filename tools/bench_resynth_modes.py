@@ -16,6 +16,11 @@ nfft 2048 / hop 512 / npks 50 and tracked once; then, alternating in every round
                 signal.  Timed twice: the map stage alone (pvk_time_map, pvk_track_stats and its 24-byte
                 read-back, pvk_track_pack of the mapped tables) and the whole stage (map stage + render
                 of the mapped partials, allocations included, as SinSum.synth(time_map=...) runs it)
+  remap         SinSum.remap(tau) of a ping-pong loop at 1x over the first half of the signal (forwards,
+                then backwards: as many output blocks as the time_map row),
+                rendered with phase_preserve=False.  Timed twice, alternating with the time_map passes: the
+                remap stage alone (pvk_time_map, pvk_track_relink, pvk_track_stats and its 24-byte
+                read-back, pvk_track_pack) and the whole stage (remap stage + render of the runs)
 
 The phase scan alone (its three kernels) is timed from a torch.profiler capture of the free mode, the
 formant gain kernel from one capture per formant mode.  A
@@ -104,24 +109,43 @@ def stretch_map(F, period=700.0):
     return tau[tau <= F - 1]
 
 
+def pingpong_map(F):
+    """A ping-pong loop at 1x over the first half of the table: forwards from row 0 to row F // 2, then
+    backwards to row 0 (about F output blocks, as many as stretch_map)."""
+    h = F // 2
+    return np.concatenate([np.arange(0.0, h + 1.0), np.arange(h - 1.0, -1.0, -1.0)])
+
+
 def time_leg_map(tid, pk, sr, nfft, hop_an, dev, rounds, flush):
-    """Median / min / max ms of the map stage and of the whole time-map stage (stretch_map)."""
+    """Median / min / max ms of the map stage and of the whole stage of the time map (stretch_map) and of
+    the remap (pingpong_map), the four timed passes alternating in every round."""
     F = tid.shape[0]
     tau = stretch_map(F)
     td = torch.from_numpy(tau).to(dev)
+    pp = pingpong_map(F)
+    ppd = torch.from_numpy(pp).to(dev)
 
     def whole():
         tm, pkm, last = P.time_map_device(tid, pk, td)
         P.resynth_device(tm, pkm, sr, hop_an, nfft, hop_an, max_end=last, phase_preserve=False)
         return pkm
 
+    def remap_whole():
+        _, tr, pkr = P.remap_device(tid, pk, ppd)
+        P.resynth_device(tr["tid"], pkr, sr, hop_an, nfft, hop_an, max_end=tr["max_end"], phase_preserve=False)
+        return tr, pkr
+
     pkm = whole()                                            # warm-up
+    trr, pkr = remap_whole()
     torch.cuda.synchronize()
     ps = partial_samples(pkm, hop_an, nfft, hop_an, sr, 1.0)
-    del pkm
-    times = dict(map=[], whole=[])
+    ps_r = partial_samples(pkr, hop_an, nfft, hop_an, sr, 1.0)
+    runs = dict(partials=int(trr["ntracks"]), points=int(trr["npts"]))
+    del pkm, trr, pkr
+    times = dict(map=[], whole=[], remap=[], remap_whole=[])
     for _ in range(rounds):
-        for name, fn in (("map", lambda: P.time_map_device(tid, pk, td)), ("whole", whole)):
+        for name, fn in (("map", lambda: P.time_map_device(tid, pk, td)), ("whole", whole),
+                         ("remap", lambda: P.remap_device(tid, pk, ppd)), ("remap_whole", remap_whole)):
             flush.fill_(1)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
@@ -130,12 +154,20 @@ def time_leg_map(tid, pk, sr, nfft, hop_an, dev, rounds, flush):
             e1.synchronize()
             times[name].append(e0.elapsed_time(e1))
     t = {k: np.array(v) for k, v in times.items()}
-    return dict(output_blocks=int(len(tau)), stretch="0.8x .. 1.25x (speed sine, 700-block period)",
-                temp_table_bytes=int(len(tau) * tid.shape[1] * 28),
-                median_ms=round(float(np.median(t["whole"])), 4), min_ms=round(float(t["whole"].min()), 4),
-                max_ms=round(float(t["whole"].max()), 4), map_stage_median_ms=round(float(np.median(t["map"])), 4),
-                map_stage_min_ms=round(float(t["map"].min()), 4), partial_samples=ps,
-                partial_samples_per_s=float("%.4g" % (ps / (np.median(t["whole"]) * 1e-3))))
+    tm = dict(output_blocks=int(len(tau)), stretch="0.8x .. 1.25x (speed sine, 700-block period)",
+              temp_table_bytes=int(len(tau) * tid.shape[1] * 28),
+              median_ms=round(float(np.median(t["whole"])), 4), min_ms=round(float(t["whole"].min()), 4),
+              max_ms=round(float(t["whole"].max()), 4), map_stage_median_ms=round(float(np.median(t["map"])), 4),
+              map_stage_min_ms=round(float(t["map"].min()), 4), partial_samples=ps,
+              partial_samples_per_s=float("%.4g" % (ps / (np.median(t["whole"]) * 1e-3))))
+    rm = dict(output_blocks=int(len(pp)), map="ping-pong loop at 1x over the first half of the table (forwards, then backwards)",
+              temp_table_bytes=int(len(pp) * tid.shape[1] * 36), runs=runs,
+              median_ms=round(float(np.median(t["remap_whole"])), 4), min_ms=round(float(t["remap_whole"].min()), 4),
+              max_ms=round(float(t["remap_whole"].max()), 4),
+              remap_stage_median_ms=round(float(np.median(t["remap"])), 4),
+              remap_stage_min_ms=round(float(t["remap"].min()), 4), partial_samples=ps_r,
+              partial_samples_per_s=float("%.4g" % (ps_r / (np.median(t["remap_whole"]) * 1e-3))))
+    return tm, rm
 
 
 def run_leg(c, dev, rounds, label):
@@ -235,11 +267,17 @@ def run_leg(c, dev, rounds, label):
     res["formant_gain_kernel_us"] = {k: round(v, 2) for k, v in gain_us.items()}
     res["formant_gain_share"] = {k: round(v / 1e3 / res["modes"][k]["median_ms"], 4) for k, v in gain_us.items()}
     res["profiled_kernels_us_per_pass"] = kern
-    tmr = time_leg_map(tid, pk, sr, nfft, hop_an, dev, rounds, flush)
+    del bufs                                                 # room for the mapped tables (13.6 GB at cfg4)
+    torch.cuda.empty_cache()
+    tmr, rmr = time_leg_map(tid, pk, sr, nfft, hop_an, dev, rounds, flush)
     res["modes"]["time_map"] = dict(hop=hop_an, phase_preserve=False, fscale=1.0, **tmr)
     res["time_map_vs_free"] = round(tmr["median_ms"] / res["modes"]["free"]["median_ms"], 3)
     res["time_map_stage_share"] = round(tmr["map_stage_median_ms"] / tmr["median_ms"], 3)
-    del bufs, flush, tr, pk, dcurve, formant
+    res["modes"]["remap"] = dict(hop=hop_an, phase_preserve=False, fscale=1.0, **rmr)
+    res["remap_stage_vs_time_map_stage_per_block"] = round(
+        (rmr["remap_stage_median_ms"] / rmr["output_blocks"]) / (tmr["map_stage_median_ms"] / tmr["output_blocks"]), 3)
+    res["remap_stage_share"] = round(rmr["remap_stage_median_ms"] / rmr["median_ms"], 3)
+    del flush, tr, pk, dcurve, formant
     torch.cuda.empty_cache()
     return res
 
